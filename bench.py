@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: batched predict + Grad-CAM images/s at 256x256 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of predict + Grad-CAM over one batch of synthetic images that is already resident
@@ -167,6 +167,27 @@ def synth_images(n, shape, seed):
     mean = x.mean(axis=(1, 2, 3), keepdims=True)
     std = x.std(axis=(1, 2, 3), keepdims=True)
     return ((x - mean) / std).astype(np.float32)
+
+
+DUMP_HEAT_BYTES = 32 << 20        # --dump-outputs: heat-map share of the dump (the whole dump stays under 64 MB)
+
+
+def dump_sample(n_images, pixels_per_map):
+    """Sorted indices of the images whose heat-maps --dump-outputs writes: all of them when they fit DUMP_HEAT_BYTES,
+    else a fixed seeded sample, so that two runs with the same arguments dump the same images."""
+    k = min(n_images, DUMP_HEAT_BYTES // (4 * pixels_per_map))
+    if k == n_images:
+        return np.arange(n_images)
+    return np.sort(np.random.default_rng(0).choice(n_images, k, replace=False))
+
+
+def write_dump(out_dir, arrays):
+    """--dump-outputs: every array as <out_dir>/<name>.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log(f"[bench] outputs of the last timed step: {', '.join(f'{k}{list(v.shape)}' for k, v in arrays.items())} -> {out_dir}")
 
 
 def oracle_setup():
@@ -391,6 +412,11 @@ def run_ours(args, rank, world, local_rank):
         r["launches"] = e.launch_count - l0
         r["ms_total"] = ev0.elapsed_time(ev1)
         r["out"] = out
+        if args.dump_outputs and e is eng:    # copied now: every later call rewrites heat_dev
+            cls, probs, logits, heat = out
+            rows = torch.from_numpy(dump_sample(B, INPUT_SHAPE[0] * INPUT_SHAPE[1])).to(dev)
+            r["dump"] = {"classes": cls.cpu().numpy().astype(np.float32), "probs": probs.cpu().numpy(),
+                         "logits": logits.cpu().numpy(), "heatmaps": heat.index_select(0, rows).cpu().numpy()}
         # ---- per-kernel device times (CUDA events before every kernel) taken UNDER LOAD: profiled steps run back to back
         # right behind the timed region and only the last call of each group is read
         e.set_profiling(True)
@@ -711,6 +737,8 @@ def run_ours(args, rank, world, local_rank):
             "gpu_launches": int(grade["launches"]), "clocks": grade["clocks"],
             "roofline": roofline_of(grade["prof"], {}, "fp16x3"), "roofline_tail": tail_roofline(grade["prof"], "fp16x3"),
             "kernels": kernel_table(grade["prof"]), "check": check3}
+    if args.dump_outputs:
+        write_dump(args.dump_outputs, main["dump"])
     emit(out_json)
 
 
@@ -1128,7 +1156,15 @@ def main():
     ap.add_argument("--no-fp32-grade", action="store_true", help="skip the second measurement of the workload in fp16x3 mode")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-check", action="store_true", help="skip the (untimed) oracle check of the first images")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what rank 0's last timed step returned as DIR/<name>.npy (float32): classes, probs, logits and the "
+                         "heat-maps of every image, or of a fixed seeded sample of them when all would exceed 32 MB; "
+                         "explain workload of --impl ours only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "explain"):
+        ap.error("--dump-outputs writes the outputs of the explain workload of --impl ours")
     global FLAVOUR
     FLAVOUR = args.flavour
     if args.input_shape:

@@ -1,8 +1,7 @@
-"""Load the reference's own Python modules from /root/reference -- TEST INFRASTRUCTURE.
+"""Load the reference's own Python modules from a checkout of it (``BCAD_REFERENCE_ROOT``) -- TEST INFRASTRUCTURE.
 
-Only usable in the authoring container (the GPU box has no /root/reference); used by
-``tests/golden/make_golden.py`` to generate fixtures and by the ``ref``-marked CPU tests
-that re-check the oracle against the live reference when it is present.
+Used only by ``tests/golden/make_golden.py`` to generate the fixtures; the tests read those fixtures
+and never need the reference itself.
 
 The reference has import-time side effects that must not leak (SURVEY section 5):
 ``Classes/CNNModel.py:10`` opens a log file in cwd, ``:28`` replaces ``sys.stdout``,

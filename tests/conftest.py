@@ -12,7 +12,6 @@ GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run with -m gpu on the B200 box)")
-    config.addinivalue_line("markers", "ref: needs /root/reference (authoring container only; skipped elsewhere)")
 
 
 @pytest.fixture(scope="session")

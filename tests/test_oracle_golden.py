@@ -136,27 +136,13 @@ def test_tail_known_answers():
     assert out.dtype == np.float32 and out.min() == 0 and abs(out.max() - 1) < 1e-5
 
 
-@pytest.mark.ref
-def test_oracle_against_live_reference():
-    """When /root/reference is present: a fresh random case straight through the reference."""
-    from oracle import ref_loader
-    if not ref_loader.available():
-        pytest.skip("no /root/reference on this machine")
-    ref = ref_loader.load_numpy_cnn()
-    np.random.seed(99)
-    with ref_loader.silenced():
-        m = ref.CNNModel((10, 9, 2), 2, conv_layers=[(2, 3), (3, 3)], hidden_units=[4], leaky_alpha=0.1)
-    cfg = ocnn.NetConfig.numpy_flavour((10, 9, 2), 2, [(2, 3), (3, 3)], [4], 0.1)
-    p = ocnn.Params([m.layers[0]["filters"], m.layers[2]["filters"]],
-                    [m.layers[0]["biases"], m.layers[2]["biases"]],
-                    [m.layers[4]["weights"], m.layers[5]["weights"]],
-                    [m.layers[4]["biases"], m.layers[5]["biases"]])
-    x = np.random.randn(10, 9, 2)
-    with ref_loader.silenced():
-        cls, probs = m.predict(x)
-    c, pr, _ = ocnn.predict(cfg, p, x)
-    assert int(c[0]) == int(cls)
-    np.testing.assert_allclose(pr[0], probs, rtol=0, atol=1e-12)
+@pytest.mark.parametrize("name", ["ref_numpy_small", "ref_numpy_odd", "ref_numpy_ties", "ref_numpy_k5"])
+def test_oracle_predict_against_reference_fixture(name):
+    """oracle.cnn.predict vs the reference's own ``CNNModel.predict`` (class, probs) as make_golden.py recorded it."""
+    g, cfg, p, _, _ = _numpy_case(name)
+    c, pr, _ = ocnn.predict(cfg, p, g["x"])
+    assert int(c[0]) == int(g["pred_class"])
+    np.testing.assert_allclose(pr[0], g["probs"], rtol=0, atol=1e-12)
 
 
 def test_cpu_port_matches_reference_fixture():
