@@ -139,6 +139,18 @@ BCAD_API int bcad_predict_explain_sized(bcad_model* m, const float* x_dev, int B
                                float* logits_dev, float* probs_dev, int32_t* cls_dev, int out_h, int out_w, float* heatmap_dev,
                                void* stream);
 
+/* Predict + Grad-CAM for K target classes per image from ONE forward: the deployed dual-class explanation (app.py:649-657 ->
+ * GRADCAM.py:63-64 with classes_to_test) as one batched call.  1 <= K <= BCAD_MAX_EXPLAIN_CLASSES; classes_dev: int32 [B][K] on
+ * the device (duplicates allowed), or NULL = column k explains class k (K <= num_classes).  out_h = out_w = 0: heat-maps of the
+ * model's input size, else scaled to out_h x out_w as bcad_predict_explain_sized does.  heatmap_dev: fp32 [B][K][H][W].
+ * logits / probs / cls as bcad_predict_explain (each may be NULL).  heat[:, k], logits, probs and classes are bitwise equal to
+ * bcad_predict_explain_sized on the same handle with class column k (images re-run by the refinement twin included).  Afterwards
+ * bcad_get_tensor(BCAD_T_ALPHA | BCAD_T_CAM_LOWRES) returns BCAD_ERR_STATE: those caches describe one class. */
+#define BCAD_MAX_EXPLAIN_CLASSES 8
+BCAD_API int bcad_predict_explain_classes(bcad_model* m, const float* x_dev, int B, int K, const int32_t* classes_dev, int grad_mode,
+                                          float* logits_dev, float* probs_dev, int32_t* cls_dev, int out_h, int out_w,
+                                          float* heatmap_dev, void* stream);
+
 /* compute_backprops_for_explainability (explainability.py:13-68), activation-gradient part:
  * uses the activations cached by the preceding bcad_predict of the SAME B (<= max_batch,
  * keep_all_activations=1 when gradients below the last conv block are wanted).

@@ -158,6 +158,13 @@ class CNNModel(nn.Module):
             eng.set_explain_target("conv")
         return cls.long(), logits, heat
 
+    def predict_explain_classes_batch(self, x, classes=(0, 1), grad_mode="logit"):
+        """Grad-CAM for several target classes per image from one forward (the dual-class call of app.py:649-657)
+        -> (classes [B], logits [B,nc], heatmaps fp32 [B,K,H,W]) on the GPU.  ``classes``: a length-K sequence shared by the batch,
+        a [B,K] array, or None = every class; ``heat[:, k]`` equals ``predict_explain_batch(x, classes[:, k])``'s heat-maps."""
+        cls, probs, logits, heat = self.engine.predict_explain_classes(x, classes, grad_mode)
+        return cls.long(), logits, heat
+
 
 def _pull_into_modules(model, eng):
     """Weights of the training handle -> the nn.Parameters (state_dict layout); the inference handle re-uploads on its next use."""

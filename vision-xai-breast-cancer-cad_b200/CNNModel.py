@@ -312,6 +312,15 @@ class CNNModel:
         cls, probs, _, heat = self._batch_engine().predict_explain_host(X, class_idx, grad_mode)
         return cls.astype(np.int64), probs, heat
 
+    def predict_explain_classes_batch(self, X, classes=(0, 1), grad_mode="softmax_ce"):
+        """X [B,H,W,C] -> (classes [B], probs [B,nc], Grad-CAM heatmaps float32 [B,K,H,W] in [0,1]) for K target classes per image
+        from one forward.  ``classes``: a length-K sequence shared by the batch, a [B,K] array, or None = every class."""
+        X = np.asarray(X)
+        if X.dtype == np.uint8:
+            X = X.astype(np.float32) / np.float32(255.0)
+        cls, probs, _, heat = self._batch_engine().predict_explain_classes(np.asarray(X, dtype=np.float32), classes, grad_mode)
+        return cls.cpu().numpy().astype(np.int64), probs.cpu().numpy(), heat.cpu().numpy()
+
     # ------------------------------------------------------------------ persistence (Classes/CNNModel.py:530-555)
     def save_model(self, path="trained_model/cnn_model.npz"):
         d = os.path.dirname(path)

@@ -21,6 +21,7 @@ PRECISION = {"fp32": 0, "fp16": 1, "fp16x3": 2}
 GRAD_MODE = {"logit": 0, "softmax_ce": 1}
 TARGET = {"conv": 0, "conv_act": 0, "conv_preact": 1}
 T_CONV_OUT, T_POOL_OUT, T_DENSE_Z, T_ALPHA, T_CAM_LOWRES = 0, 1, 2, 3, 4
+MAX_EXPLAIN_CLASSES = 8
 
 
 class Config(C.Structure):
@@ -54,6 +55,7 @@ _SIGNATURES = {
     "bcad_predict": (C.c_int, [_P, _P, C.c_int, _P, _P, _P, _P]),
     "bcad_predict_explain": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, _P, _P, _P, _P]),
     "bcad_predict_explain_sized": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, _P, _P, C.c_int, C.c_int, _P, _P]),
+    "bcad_predict_explain_classes": (C.c_int, [_P, _P, C.c_int, C.c_int, _P, C.c_int, _P, _P, _P, C.c_int, C.c_int, _P, _P]),
     "bcad_gradcam_overlays_host": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, _P, _P, _P, _P, _P]),
     "bcad_explain_backward": (C.c_int, [_P, C.c_int, _P, C.c_int, C.POINTER(_P), _P, _P]),
     "bcad_get_tensor": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, _P, _P]),

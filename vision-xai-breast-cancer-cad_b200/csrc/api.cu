@@ -359,6 +359,7 @@ int bcad_commit(bcad_model* mm) {
         BCAD_TRY(m->alloc((void**)&m->alpha, (size_t)mb * T.Cout * sizeof(float)));
         BCAD_TRY(m->alloc((void**)&m->cam_lo, (size_t)mb * T.Ho * T.Wo * sizeof(float)));
         BCAD_TRY(m->alloc((void**)&m->mm, (size_t)mb * m->cam_splits * 2 * sizeof(float)));
+        BCAD_TRY(m->alloc((void**)&m->class_cols, (size_t)BCAD_MAX_EXPLAIN_CLASSES * mb * sizeof(int32_t)));
         BCAD_CUDA_CHECK(cudaEventCreateWithFlags(&m->call_done, cudaEventDisableTiming));
         m->ws_ready = true;
     }
@@ -417,7 +418,17 @@ int launch_fused_head(Model* m, int n, const float* fc1_part, int splits, size_t
     a.alpha = m->cfg.alpha_dense; a.head = m->cfg.head; a.probs = m->probs; a.cls = m->cls;
     a.explain = explain ? 1 : 0; a.class_idx = class_idx; a.grad_mode = grad_mode;
     a.dz1 = dz1; a.S = S; a.C = C; a.alpha_raw = alpha_raw; a.n_dev = m->n_dev;
+    m->head_last = a;
+    m->head_n = n;
     BCAD_LAUNCH(m, "dense_head_fused", launch_dense_head(a, n, s));
+    return BCAD_OK;
+}
+
+int relaunch_fused_head(Model* m, const int32_t* class_idx, float* alpha_raw, cudaStream_t s) {
+    HeadArgs a = m->head_last;
+    a.class_idx = class_idx;
+    if (a.alpha_raw != nullptr) a.alpha_raw = alpha_raw;
+    BCAD_LAUNCH(m, "dense_head_fused", launch_dense_head(a, m->head_n, s));
     return BCAD_OK;
 }
 
@@ -513,17 +524,17 @@ int dense_backward(Model* m, int n, const int32_t* class_idx, int grad_mode, flo
     return BCAD_OK;
 }
 
-static int tail_chunk(Model* m, const void* A, int a_dtype, int n, float* heat, cudaStream_t s) {
+static int tail_chunk(Model* m, const void* A, int a_dtype, int n, float* heat, size_t heat_stride, cudaStream_t s) {
     const ConvLayer& T = m->conv.back();
     const float inv_hw = 1.0f / ((float)T.Ho * (float)T.Wo);
     const float inv_slope = (m->target == BCAD_TARGET_CONV_PREACT) ? 1.0f / m->cfg.alpha_conv : 0.f;
     BCAD_LAUNCH(m, "cam", launch_cam(A, a_dtype, m->alpha_part, m->alpha_splits, inv_hw, m->alpha, m->cam_lo, m->mm, n, T.Ho,
                               T.Wo, T.Cout, m->cam_splits, s, inv_slope));
-    BCAD_LAUNCH(m, "upsample_norm", launch_upsample_norm(m->cam_lo, m->mm, m->cam_splits, heat, n, T.Ho, T.Wo, m->heat_h, m->heat_w, s));
+    BCAD_LAUNCH(m, "upsample_norm", launch_upsample_norm(m->cam_lo, m->mm, m->cam_splits, heat, n, T.Ho, T.Wo, m->heat_h, m->heat_w, s, nullptr, heat_stride));
     return BCAD_OK;
 }
 
-static int explain_chunk_fp32(Model* m, int n, const int32_t* class_idx, int grad_mode, float* heat, cudaStream_t s) {
+static int explain_chunk_fp32(Model* m, int n, const int32_t* class_idx, int grad_mode, float* heat, size_t heat_stride, cudaStream_t s) {
     const ConvLayer& T = m->conv.back();
     if (m->fused_head) {
         // dz1 was left in dense[0].h by the fused head: only the fc1 input gradient remains
@@ -535,30 +546,40 @@ static int explain_chunk_fp32(Model* m, int n, const int32_t* class_idx, int gra
     }
     BCAD_LAUNCH(m, "alpha_from_pool_grad", launch_alpha_from_pool_grad(m->g_flat, T.y, m->alpha_part, n, T.Ho, T.Wo, T.Cout, m->cfg.pool_ties,
                                                m->alpha_splits, s, m->target == BCAD_TARGET_CONV_PREACT ? m->cfg.alpha_conv : -1.f));
-    BCAD_TRY(tail_chunk(m, T.y, 0, n, heat, s));
+    BCAD_TRY(tail_chunk(m, T.y, 0, n, heat, heat_stride, s));
     return BCAD_OK;
 }
 
+// K = 0: one target per image, class_idx [B] (NULL = the predicted class).  K >= 1 (bcad_predict_explain_classes): class_idx
+// [B][K] (NULL = column k is class k), heat [B][K][H][W]
 static int run(Model* m, const float* x, int B, const int32_t* class_idx, int grad_mode, bool explain, float* logits,
-               float* probs, int32_t* cls, float* heat, cudaStream_t s, int out_h = 0, int out_w = 0);
+               float* probs, int32_t* cls, float* heat, cudaStream_t s, int out_h = 0, int out_w = 0, int K = 0);
 
 // cfg.refine_margin: re-run the chunk's small-margin images on the fp32-grade twin and write their results over the 16-bit ones
 // (refine.cu).  Stream-ordered: the twin always runs min(cap, n) slots, the device-side count selects what is written back.
-static int refine_chunk(Model* m, const float* xc, int n, const int32_t* ci, int grad_mode, bool explain, float* heat, cudaStream_t s) {
+// K >= 1: ci holds the chunk's [n][K] class rows (or NULL) and each image has K maps, contiguous (bcad_predict_explain_classes)
+static int refine_chunk(Model* m, const float* xc, int n, const int32_t* ci, int grad_mode, bool explain, float* heat, cudaStream_t s,
+                        int K = 0) {
     Refine& R = m->refine;
     Model* t = R.twin;
-    const int nc = m->cfg.num_classes, slots = std::min(R.cap, n);
-    const size_t img = (size_t)m->cfg.in_h * m->cfg.in_w * m->cfg.in_c, hm = (size_t)m->heat_h * m->heat_w;
-    if (explain && hm > R.heat_elems) {               // first call with a larger heat-map (bcad_predict_explain_sized): grow the twin's buffer
+    const int nc = m->cfg.num_classes, slots = std::min(R.cap, n), kc = K ? K : 1;
+    const size_t img = (size_t)m->cfg.in_h * m->cfg.in_w * m->cfg.in_c, hm = (size_t)kc * m->heat_h * m->heat_w;
+    if (explain && hm > R.heat_elems) {               // first call with larger or more heat-maps (_sized / _classes): grow the twin's buffer
         BCAD_CUDA_CHECK(cudaStreamSynchronize(s));
         BCAD_TRY(m->alloc((void**)&R.heat, (size_t)R.cap * hm * sizeof(float)));
         R.heat_elems = hm;
     }
+    if (kc > R.cidx_k) {
+        BCAD_CUDA_CHECK(cudaStreamSynchronize(s));
+        BCAD_TRY(m->alloc((void**)&R.cidx, (size_t)R.cap * kc * sizeof(int32_t)));
+        BCAD_CUDA_CHECK(cudaMemset(R.cidx, 0, (size_t)R.cap * kc * sizeof(int32_t)));
+        R.cidx_k = kc;
+    }
     BCAD_LAUNCH(m, "refine_flag", launch_refine_flag(m->dense.back().z, n, nc, m->cfg.refine_margin, slots, R.idx, R.counters, s));
-    BCAD_LAUNCH(m, "refine_gather", launch_refine_gather(xc, img, ci, R.idx, R.counters, slots, R.x, R.cidx, s));
+    BCAD_LAUNCH(m, "refine_gather", launch_refine_gather(xc, img, ci, R.idx, R.counters, slots, R.x, R.cidx, s, kc));
     BCAD_TRY(m->mark("refine_twin_fp16x3", s));
     const int64_t l0 = t->launches;
-    BCAD_TRY(run(t, R.x, slots, ci ? R.cidx : nullptr, grad_mode, explain, nullptr, nullptr, nullptr, explain ? R.heat : nullptr, s, m->heat_h, m->heat_w));
+    BCAD_TRY(run(t, R.x, slots, ci ? R.cidx : nullptr, grad_mode, explain, nullptr, nullptr, nullptr, explain ? R.heat : nullptr, s, m->heat_h, m->heat_w, K));
     m->launches += t->launches - l0;
     RefineScatter a;
     memset(&a, 0, sizeof(a));
@@ -576,7 +597,7 @@ static int refine_chunk(Model* m, const float* xc, int n, const int32_t* ci, int
 }
 
 static int run(Model* m, const float* x, int B, const int32_t* class_idx, int grad_mode, bool explain, float* logits,
-               float* probs, int32_t* cls, float* heat, cudaStream_t s, int out_h, int out_w) {
+               float* probs, int32_t* cls, float* heat, cudaStream_t s, int out_h, int out_w, int K) {
     BCAD_REQUIRE(m && x, "null model or input");
     BCAD_REQUIRE(out_h >= 0 && out_w >= 0 && out_h <= 16384 && out_w <= 16384 && (out_h == 0) == (out_w == 0), "bad heat-map size %dx%d", out_h, out_w);
     BCAD_REQUIRE(B >= 1, "batch must be >= 1, got %d", B);
@@ -591,19 +612,33 @@ static int run(Model* m, const float* x, int B, const int32_t* class_idx, int gr
     const int mb = m->cfg.max_batch, nc = m->cfg.num_classes;
     m->heat_h = out_h ? out_h : m->cfg.in_h;
     m->heat_w = out_w ? out_w : m->cfg.in_w;
-    const size_t img = (size_t)m->cfg.in_h * m->cfg.in_w * m->cfg.in_c, hm = (size_t)m->heat_h * m->heat_w;
+    const int kc = K ? K : 1;                                       // maps per image
+    const size_t img = (size_t)m->cfg.in_h * m->cfg.in_w * m->cfg.in_c, hm = (size_t)m->heat_h * m->heat_w, hk = kc * hm;
     m->prof_n = 0;
+    m->multi_class_call = (K > 1);
     for (int b0 = 0; b0 < B; b0 += mb) {
         const int n = std::min(mb, B - b0);
         const float* xc = x + (size_t)b0 * img;
-        const int32_t* ci = (explain && class_idx) ? class_idx + b0 : nullptr;
-        if (m->tensor_path) BCAD_TRY(tensor_forward_chunk(*m, xc, n, explain, ci, grad_mode, s));
-        else BCAD_TRY(forward_chunk_fp32(m, xc, n, explain, ci, grad_mode, s));
-        if (explain) {
-            if (m->tensor_path) BCAD_TRY(tensor_explain_chunk(*m, n, ci, grad_mode, heat + (size_t)b0 * hm, s));
-            else BCAD_TRY(explain_chunk_fp32(m, n, ci, grad_mode, heat + (size_t)b0 * hm, s));
+        const int32_t* ci = (explain && class_idx) ? class_idx + (size_t)b0 * kc : nullptr;
+        const int32_t* col = ci;                                    // target class column 0 of the chunk
+        if (K) {
+            // K classes: every image's class row becomes K contiguous columns, so that each backward gets a per-image target vector
+            BCAD_LAUNCH(m, "class_columns", launch_class_columns(ci, K, n, m->class_cols, mb, s));
+            col = m->class_cols;
         }
-        if (m->refine.twin) BCAD_TRY(refine_chunk(m, xc, n, ci, grad_mode, explain, explain ? heat + (size_t)b0 * hm : nullptr, s));
+        if (m->tensor_path) BCAD_TRY(tensor_forward_chunk(*m, xc, n, explain, col, grad_mode, s));
+        else BCAD_TRY(forward_chunk_fp32(m, xc, n, explain, col, grad_mode, s));
+        if (explain) {
+            float* hc = heat + (size_t)b0 * hk;
+            if (m->tensor_path) BCAD_TRY(tensor_explain_chunk(*m, n, col, grad_mode, hc, s, kc, mb, hk));
+            else
+                for (int k = 0; k < kc; ++k) {
+                    const int32_t* ck = col ? col + (size_t)k * mb : nullptr;
+                    if (k > 0 && m->fused_head) BCAD_TRY(relaunch_fused_head(m, ck, nullptr, s));     // dz1 of class k
+                    BCAD_TRY(explain_chunk_fp32(m, n, ck, grad_mode, hc + (size_t)k * hm, hk, s));
+                }
+        }
+        if (m->refine.twin) BCAD_TRY(refine_chunk(m, xc, n, ci, grad_mode, explain, explain ? heat + (size_t)b0 * hk : nullptr, s, K));
         if (logits) BCAD_CUDA_CHECK(cudaMemcpyAsync(logits + (size_t)b0 * nc, m->dense.back().z, (size_t)n * nc * sizeof(float), cudaMemcpyDeviceToDevice, s));
         if (probs) BCAD_CUDA_CHECK(cudaMemcpyAsync(probs + (size_t)b0 * nc, m->probs, (size_t)n * nc * sizeof(float), cudaMemcpyDeviceToDevice, s));
         if (cls) BCAD_CUDA_CHECK(cudaMemcpyAsync(cls + b0, m->cls, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToDevice, s));
@@ -634,6 +669,16 @@ int bcad_predict_explain_sized(bcad_model* mm, const float* x, int B, const int3
                                float* probs, int32_t* cls, int out_h, int out_w, float* heat, void* stream) {
     BCAD_REQUIRE(out_h >= 1 && out_w >= 1, "predict_explain_sized: bad heat-map size %dx%d", out_h, out_w);
     return run(reinterpret_cast<Model*>(mm), x, B, class_idx, grad_mode, true, logits, probs, cls, heat, (cudaStream_t)stream, out_h, out_w);
+}
+
+int bcad_predict_explain_classes(bcad_model* mm, const float* x, int B, int K, const int32_t* classes, int grad_mode, float* logits,
+                                 float* probs, int32_t* cls, int out_h, int out_w, float* heat, void* stream) {
+    Model* m = reinterpret_cast<Model*>(mm);
+    BCAD_REQUIRE(m, "predict_explain_classes: null model");
+    BCAD_REQUIRE(K >= 1 && K <= BCAD_MAX_EXPLAIN_CLASSES, "predict_explain_classes: K=%d out of range 1..%d", K, BCAD_MAX_EXPLAIN_CLASSES);
+    BCAD_REQUIRE(classes || K <= m->cfg.num_classes, "predict_explain_classes: classes=NULL explains classes 0..K-1, but K=%d > num_classes=%d",
+                 K, m->cfg.num_classes);
+    return run(m, x, B, classes, grad_mode, true, logits, probs, cls, heat, (cudaStream_t)stream, out_h, out_w, K);
 }
 
 int bcad_explain_backward(bcad_model* mm, int B, const int32_t* class_idx, int grad_mode,
@@ -728,6 +773,10 @@ int bcad_get_tensor(bcad_model* mm, int kind, int index, int B, float* dst, void
     if (m->tensor_path && (kind == BCAD_T_CONV_OUT || kind == BCAD_T_POOL_OUT)) {
         BCAD_TRY(tensor_get_activation(*m, kind, index, B, dst, s));
         return BCAD_OK;
+    }
+    if ((kind == BCAD_T_ALPHA || kind == BCAD_T_CAM_LOWRES) && m->multi_class_call) {
+        set_error("get_tensor: the last call explained several classes (bcad_predict_explain_classes); alpha / the low-resolution cam describe one");
+        return BCAD_ERR_STATE;
     }
     const float* src = nullptr;
     switch (kind) {

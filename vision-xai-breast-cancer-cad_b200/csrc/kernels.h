@@ -31,6 +31,8 @@ int launch_splitk_reduce(const float* partials, int splits, const float* bias, f
 int launch_head(const float* logits, float* probs, int32_t* cls, int B, int nc, int head, cudaStream_t s);
 int launch_top_grad(const float* probs, const int32_t* cls, const int32_t* class_idx, float* d_top,
                     int B, int nc, int grad_mode, cudaStream_t s);
+// per-image class rows [n][K] (NULL: row b is 0, 1, .., K-1) -> K contiguous class columns of ld entries: cols[k * ld + b]
+int launch_class_columns(const int32_t* rows, int K, int n, int32_t* cols, int ld, cudaStream_t s);
 int launch_leaky_mask_mul(float* d, const float* z, float alpha, int64_t n, cudaStream_t s);
 int launch_unpool(const float* g, const float* y, float* dy, int B, int Ho, int Wo, int C, int ties,
                   cudaStream_t s);
@@ -49,7 +51,8 @@ int launch_cam(const void* A, int dtype, const float* alpha_part, int alpha_spli
                float* alpha_out, float* cam_lo, float* mm, int B, int h, int w, int C, int splits,
                cudaStream_t s, float inv_slope = 0.f);       // inv_slope > 0 (fp32 A): undo the LeakyReLU first (pre-activation target)
 int launch_upsample_norm(const float* cam_lo, const float* mm, int mm_splits, float* out, int B, int h,
-                         int w, int H, int W, cudaStream_t s, const int* n_dev = nullptr);   // n_dev: live image count on the device (refine.cu)
+                         int w, int H, int W, cudaStream_t s, const int* n_dev = nullptr,    // n_dev: live image count on the device (refine.cu)
+                         size_t out_stride = 0);                                            // floats between images' maps (0 = H * W)
 // non-overlapping mean pool, floor dims (Classes/ImageSegmentation.py:145-163)
 int launch_avg_pool(const float* x, float* out, int B, int H, int W, int C, int pool, cudaStream_t s);
 // [k][k][Cin][Cout] -> [k*k][Cin][CoutPad] (zero padded)
@@ -82,8 +85,9 @@ int launch_adam_update(float* w, const float* g, float* m1, float* m2, float lr,
 // clamped to cap, running total refined, running total overflowed}
 int launch_refine_flag(const float* logits, int n, int nc, float margin, int cap, int32_t* idx, int32_t* counters, cudaStream_t s);
 // slots [0,count): image idx[slot] (the twin's kernels read the same device-side count and skip the other slots)
+// class_idx rows of K entries per image (bcad_predict_explain_classes; 1 otherwise) go to rcidx[slot * K ..]
 int launch_refine_gather(const float* x, size_t img_elems, const int32_t* class_idx, const int32_t* idx, const int32_t* counters,
-                         int slots, float* rx, int32_t* rcidx, cudaStream_t s);
+                         int slots, float* rx, int32_t* rcidx, cudaStream_t s, int K = 1);
 struct RefineScatter {
     int n_dense;
     int sizes[8];

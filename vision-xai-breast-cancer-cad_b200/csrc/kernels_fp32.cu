@@ -730,7 +730,7 @@ __device__ __forceinline__ void block_minmax(float& vmin, float& vmax, float* s_
 
 __global__ void __launch_bounds__(UP_THREADS)
 upsample_norm_kernel(const float* __restrict__ cam_lo, const float* __restrict__ mm, int mm_splits,
-                     float* __restrict__ out, int h, int w, int H, int W, int lo_in_smem) {
+                     float* __restrict__ out, size_t out_stride, int h, int w, int H, int W, int lo_in_smem) {
     extern __shared__ float sm[];
     __shared__ float s_red[64];
     // layout: x0[W] x1[W] fx[W] y0[H] y1[H] fy[H] (ints stored as float bits) then the low-res map
@@ -791,7 +791,7 @@ upsample_norm_kernel(const float* __restrict__ cam_lo, const float* __restrict__
     }
     block_minmax(vmin, vmax, s_red);
     const float denom2 = 1e-7f + (vmax - vmin);
-    float* ob = out + (size_t)b * npix;
+    float* ob = out + (size_t)b * out_stride;
     for (int i = tid; i < npix; i += blockDim.x) ob[i] = (sample(i / W, i % W) - vmin) / denom2;
 }
 
@@ -800,7 +800,7 @@ upsample_norm_kernel(const float* __restrict__ cam_lo, const float* __restrict__
 // shared-memory reads and one lerp; both min-max passes run over that.
 __global__ void __launch_bounds__(UP_THREADS)
 upsample_norm_sep_kernel(const float* __restrict__ cam_lo, const float* __restrict__ mm, int mm_splits,
-                         float* __restrict__ out, int h, int w, int H, int W, const int* __restrict__ n_dev) {
+                         float* __restrict__ out, size_t out_stride, int h, int w, int H, int W, const int* __restrict__ n_dev) {
     if (n_dev != nullptr && (int)blockIdx.x >= *n_dev) return;
     extern __shared__ float sm[];
     __shared__ float s_red[64];
@@ -866,7 +866,7 @@ upsample_norm_sep_kernel(const float* __restrict__ cam_lo, const float* __restri
     block_minmax(vmin, vmax, s_red);
     // x / d is evaluated as x * (1/d): within 1 ulp of the reference's true division
     const float inv2 = 1.f / (1e-7f + (vmax - vmin));
-    float* ob = out + (size_t)b * H * W;
+    float* ob = out + (size_t)b * out_stride;
     for (int oy = warp; oy < H; oy += nwarps) {
         const float fy = s_fy[oy], gy = 1.f - fy;
         const float* r0 = s_hr + s_y0[oy];
@@ -878,14 +878,15 @@ upsample_norm_sep_kernel(const float* __restrict__ cam_lo, const float* __restri
 }
 
 int launch_upsample_norm(const float* cam_lo, const float* mm, int mm_splits, float* out, int B, int h, int w, int H,
-                         int W, cudaStream_t s, const int* n_dev) {
+                         int W, cudaStream_t s, const int* n_dev, size_t out_stride) {
+    if (out_stride == 0) out_stride = (size_t)H * W;
     const size_t tables = (size_t)(3 * W + 3 * H) * sizeof(float);
     const size_t lo_bytes = (size_t)h * w * sizeof(float), hr_bytes = (size_t)h * W * sizeof(float);
     if (tables + lo_bytes + hr_bytes <= 220 * 1024) {
         const size_t smem = tables + lo_bytes + hr_bytes;
         if (smem > 48 * 1024)
             BCAD_CUDA_CHECK(cudaFuncSetAttribute(upsample_norm_sep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
-        upsample_norm_sep_kernel<<<B, UP_THREADS, smem, s>>>(cam_lo, mm, mm_splits, out, h, w, H, W, n_dev);
+        upsample_norm_sep_kernel<<<B, UP_THREADS, smem, s>>>(cam_lo, mm, mm_splits, out, out_stride, h, w, H, W, n_dev);
         BCAD_CUDA_CHECK(cudaGetLastError());
         return BCAD_OK;
     }
@@ -895,7 +896,7 @@ int launch_upsample_norm(const float* cam_lo, const float* mm, int mm_splits, fl
     BCAD_REQUIRE(smem <= 200 * 1024, "upsample: output %dx%d too large for the coordinate tables", H, W);
     if (smem > 48 * 1024)
         BCAD_CUDA_CHECK(cudaFuncSetAttribute(upsample_norm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    upsample_norm_kernel<<<B, UP_THREADS, smem, s>>>(cam_lo, mm, mm_splits, out, h, w, H, W, lo_in_smem);
+    upsample_norm_kernel<<<B, UP_THREADS, smem, s>>>(cam_lo, mm, mm_splits, out, out_stride, h, w, H, W, lo_in_smem);
     BCAD_CUDA_CHECK(cudaGetLastError());
     return BCAD_OK;
 }
@@ -1364,6 +1365,20 @@ __global__ void __launch_bounds__(256) dense_head_kernel(HeadArgs a) {
             }
         }
     }
+}
+
+__global__ void __launch_bounds__(256)
+class_columns_kernel(const int32_t* __restrict__ rows, int K, int n, int32_t* __restrict__ cols, int ld) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n * K) return;
+    const int b = i / K, k = i - b * K;
+    cols[(size_t)k * ld + b] = rows != nullptr ? rows[i] : k;
+}
+
+int launch_class_columns(const int32_t* rows, int K, int n, int32_t* cols, int ld, cudaStream_t s) {
+    class_columns_kernel<<<(n * K + 255) / 256, 256, 0, s>>>(rows, K, n, cols, ld);
+    BCAD_CUDA_CHECK(cudaGetLastError());
+    return BCAD_OK;
 }
 
 int launch_dense_head(const HeadArgs& a, int B, cudaStream_t s) {

@@ -7,6 +7,7 @@
 #include <vector>
 
 #include "../../include/bcad.h"
+#include "kernels.h"
 
 namespace bcad {
 
@@ -102,9 +103,10 @@ struct Refine {                         // cfg.refine_margin > 0: small-margin i
     int32_t* idx = nullptr;             // [cap] chunk-local indices of the flagged images, in ascending order
     int32_t* counters = nullptr;        // {flagged in this chunk (clamped to cap), total refined, total overflowed}
     float* x = nullptr;                 // [cap] gathered inputs
-    int32_t* cidx = nullptr;            // [cap] gathered target classes
+    int32_t* cidx = nullptr;            // [cap][cidx_k] gathered target classes
+    int cidx_k = 1;                     // classes per image `cidx` has room for (grows on the first bcad_predict_explain_classes call)
     float* heat = nullptr;              // [cap] heat-maps of the twin (its other outputs are read from its own workspace)
-    size_t heat_elems = 0;              // per-image capacity of `heat` (grows on the first larger bcad_predict_explain_sized call)
+    size_t heat_elems = 0;              // per-image capacity of `heat` (grows on the first larger bcad_predict_explain_sized / _classes call)
 };
 
 struct Model {
@@ -136,6 +138,10 @@ struct Model {
     float* cam_lo = nullptr;
     float* mm = nullptr;
     int alpha_splits = 1, cam_splits = 1;
+    int32_t* class_cols = nullptr;      // [BCAD_MAX_EXPLAIN_CLASSES][max_batch]: target class column k of the chunk (bcad_predict_explain_classes)
+    bool multi_class_call = false;      // the last call explained several classes: alpha / cam_lo describe none of them
+    HeadArgs head_last;                 // arguments of the chunk's dense_head_kernel launch, re-launched per extra target class
+    int head_n = 0;
     cudaEvent_t call_done = nullptr;
     std::vector<cudaEvent_t> prof_pool;   // profiling marks of the last call: event i precedes kernel i
     std::vector<const char*> prof_names;
@@ -161,12 +167,19 @@ bool fused_head_ok(const Model* m);
 // everything after the fc1 GEMM in one launch (dense_head_kernel); dz1 / S / alpha_raw are optional outputs
 int launch_fused_head(Model* m, int n, const float* fc1_part, int splits, size_t ld, bool explain, const int32_t* class_idx,
                       int grad_mode, float* dz1, const float* S, int C, float* alpha_raw, cudaStream_t s);
+// the chunk's last launch_fused_head again with another target class column (alpha_raw replaces its alpha output when it had one):
+// the kernel recomputes everything from the fc1 split-K partials, which no kernel after it writes, so the forward outputs it
+// rewrites come out the same and dz1 / alpha are those of the new targets
+int relaunch_fused_head(Model* m, const int32_t* class_idx, float* alpha_raw, cudaStream_t s);
 
 // ---- tensor (tcgen05) path, tensor_path.cu
 int tensor_path_supported(const Model& m);          // BCAD_OK or BCAD_ERR_INVALID (+ message)
 int tensor_path_commit(Model& m);
 int tensor_forward_chunk(Model& m, const float* x, int n, bool explain, const int32_t* class_idx, int grad_mode, cudaStream_t s);
-int tensor_explain_chunk(Model& m, int n, const int32_t* class_idx, int grad_mode, float* heat, cudaStream_t s);
+// K target classes: class column k at class_idx + k * col_ld, the map of class k of image b at heat + b * heat_stride + k * H * W
+// (heat_stride 0 = H * W)
+int tensor_explain_chunk(Model& m, int n, const int32_t* class_idx, int grad_mode, float* heat, cudaStream_t s, int K = 1,
+                         size_t col_ld = 0, size_t heat_stride = 0);
 int tensor_get_activation(Model& m, int kind, int index, int B, float* dst, cudaStream_t s);
 void tensor_path_destroy(Model& m);
 

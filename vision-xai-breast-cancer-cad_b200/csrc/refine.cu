@@ -59,13 +59,13 @@ refine_flag_kernel(const float* __restrict__ logits, int n, int nc, float margin
 
 __global__ void __launch_bounds__(256)
 refine_gather_kernel(const float* __restrict__ x, size_t img_elems, const int32_t* __restrict__ class_idx, const int32_t* __restrict__ idx,
-                     const int32_t* __restrict__ counters, float* __restrict__ rx, int32_t* __restrict__ rcidx) {
+                     const int32_t* __restrict__ counters, float* __restrict__ rx, int32_t* __restrict__ rcidx, int K) {
     const int slot = blockIdx.x;
     if (slot >= counters[0]) return;              // the twin's kernels only touch the first counters[0] slots
     const int src = idx[slot];
     const float* in = x + (size_t)src * img_elems;
     float* out = rx + (size_t)slot * img_elems;
-    if (blockIdx.y == 0 && threadIdx.x == 0 && class_idx != nullptr) rcidx[slot] = class_idx[src];
+    if (blockIdx.y == 0 && (int)threadIdx.x < K && class_idx != nullptr) rcidx[slot * K + threadIdx.x] = class_idx[src * K + threadIdx.x];
     const size_t per = (img_elems + gridDim.y - 1) / gridDim.y;
     const size_t lo = (size_t)blockIdx.y * per, hi = lo + per < img_elems ? lo + per : img_elems;
     if (((reinterpret_cast<uintptr_t>(in) | reinterpret_cast<uintptr_t>(out)) & 15) == 0 && (lo & 3) == 0) {
@@ -110,10 +110,10 @@ static int copy_blocks(size_t elems) {
 }
 
 int launch_refine_gather(const float* x, size_t img_elems, const int32_t* class_idx, const int32_t* idx, const int32_t* counters,
-                         int slots, float* rx, int32_t* rcidx, cudaStream_t s) {
+                         int slots, float* rx, int32_t* rcidx, cudaStream_t s, int K) {
     int by = copy_blocks(img_elems);
     while (by > 1 && (((img_elems + by - 1) / by) & 3)) --by;          // keep every block's range a multiple of 4 floats (vector path)
-    refine_gather_kernel<<<dim3(slots, by), 256, 0, s>>>(x, img_elems, class_idx, idx, counters, rx, rcidx);
+    refine_gather_kernel<<<dim3(slots, by), 256, 0, s>>>(x, img_elems, class_idx, idx, counters, rx, rcidx, K);
     BCAD_CUDA_CHECK(cudaGetLastError());
     return BCAD_OK;
 }

@@ -96,8 +96,15 @@ int launch_cam_c8(const __half* A, const float* alpha_raw, float scale, float* a
                   int B, int h, int w, int C, int splits, bool x3, cudaStream_t s, const int* n_dev = nullptr);
 // fused tail (sm100_tail.cu): cam + min-max + bilinear + min-max, a 2-CTA cluster per image
 bool tail_fused_supported(int h, int w, int H, int W, int C);
+// out_stride: floats between the maps of consecutive images (0 = H * W)
 int launch_tail_fused(const __half* A, const float* alpha_raw, float scale, float* alpha_out, float* out, int B, int h, int w,
-                      int H, int W, int C, bool x3, cudaStream_t s, const int* n_dev = nullptr);
+                      int H, int W, int C, bool x3, cudaStream_t s, const int* n_dev = nullptr, size_t out_stride = 0);
+// TF_GROUP target classes in one launch, one read of A: alpha of class k at alpha_raw + k * alpha_ld ([B][C] each), the map of class k
+// of image b at out + b * out_stride + k * H * W; each bit-identical to a launch_tail_fused of that class
+constexpr int TF_GROUP = 2;
+bool tail_fused_classes_supported(int h, int w, int H, int W, int C);
+int launch_tail_fused_classes(const __half* A, const float* alpha_raw, size_t alpha_ld, float scale, float* out, size_t out_stride, int B,
+                              int h, int w, int H, int W, int C, bool x3, cudaStream_t s, const int* n_dev = nullptr);
 // tie-duplicating rule on the fp16x3 path: alpha_raw[b][k] = sum_windows g * (#maxima in the window), A = split C8-planar activations
 int launch_alpha_ties_c8(const __half* A, const float* g_pool, float* alpha_raw, int B, int h, int w, int C, cudaStream_t s);
 int launch_c8_to_nhwc(const __half* src, float* dst, int B, int h, int w, int C, bool x3, cudaStream_t s);

@@ -42,7 +42,7 @@ struct TensorPath {
     __half* act = nullptr;   // conv1 output, C8 planar
     uint8_t* fc_a = nullptr;        // pooled conv1 as fc1 A tiles
     float* fc_part = nullptr;
-    float* alpha_raw = nullptr;     // [B][Cout] = dz1 . S
+    float* alpha_raw = nullptr;     // [TF_GROUP][B][Cout] = dz1 . S
     int fc_splits = 1, kb_per_split = 1, m_pad = 128;
     bool x3 = false;                // fp16x3: hi/lo split operands everywhere (fp32-grade)
     uint8_t* d_fc_wT = nullptr;     // tie-duplicating mode: fc1 transposed as W tiles of the input-gradient GEMM [col block][k-block][hi|lo][256][128 B]
@@ -314,7 +314,7 @@ int tensor_path_commit(Model& m) {
         TP_TRY(m.alloc((void**)&t.fc_a, parts * t.m_pad * npix * 128));
         BCAD_CUDA_CHECK(cudaMemset(t.fc_a, 0, parts * t.m_pad * npix * 128));     // padding rows: finite zeros
         TP_TRY(m.alloc((void**)&t.fc_part, (size_t)t.fc_splits * t.m_pad * d0.out * 4));
-        TP_TRY(m.alloc((void**)&t.alpha_raw, (size_t)mb * c1.Cout * 4));
+        TP_TRY(m.alloc((void**)&t.alpha_raw, (size_t)TF_GROUP * mb * c1.Cout * 4));      // one [mb][C] slice per class of a tail group
     }
     return BCAD_OK;
 }
@@ -437,13 +437,15 @@ int tensor_forward_chunk(Model& m, const float* x, int n, bool explain, const in
     return BCAD_OK;
 }
 
-int tensor_explain_chunk(Model& m, int n, const int32_t* class_idx, int grad_mode, float* heat, cudaStream_t s) {
+// alpha_raw of one target class column (class_idx) into alpha_dst.  rerun_head: the chunk's dense head already ran for another class
+static int tensor_alpha(Model& m, int n, const int32_t* class_idx, int grad_mode, float* alpha_dst, bool rerun_head, cudaStream_t s) {
     TensorPath& t = *m.tp;
     const ConvLayer& T = m.conv.back();
     if (m.cfg.pool_ties != BCAD_TIES_FIRST) {
         // tie-duplicating rule (the NumPy CNN): no alpha shortcut -- dz1 -> dense pooled gradient (fp32 GEMM with the fp32 fc1
         // weights) -> alpha with per-window tie counts read from the split activations; alpha_raw then feeds the usual tail
         if (!m.fused_head) TP_TRY(dense_backward(&m, n, class_idx, grad_mode, nullptr, s));          // leaves dz1 in dense[0].h
+        else if (rerun_head) TP_TRY(relaunch_fused_head(&m, class_idx, nullptr, s));
         DenseLayer& D0 = m.dense[0];
         if (t.d_fc_wT != nullptr) {
             // g[b][col] = sum_u dz1[b][u] W1[u][col] on tcgen05: split operands, one CTA per (256-column block, 128-image tile)
@@ -456,26 +458,51 @@ int tensor_explain_chunk(Model& m, int n, const int32_t* class_idx, int grad_mod
         } else {
             TP_LAUNCH(m, "fc1_dgrad_sgemm", launch_sgemm(D0.h, D0.d_w, m.g_flat, n, D0.in, D0.out, false, 1, s));
         }
-        TP_LAUNCH(m, "alpha_ties_c8", launch_alpha_ties_c8(t.act, m.g_flat, t.alpha_raw, n, T.Ho, T.Wo, T.Cout, s));
-    } else
-    if (!m.fused_head) {
+        TP_LAUNCH(m, "alpha_ties_c8", launch_alpha_ties_c8(t.act, m.g_flat, alpha_dst, n, T.Ho, T.Wo, T.Cout, s));
+    } else if (!m.fused_head) {
         // dense backward down to dz1 (left in dense[0].h); no fc1 dgrad GEMM, no dA
         TP_TRY(dense_backward(&m, n, class_idx, grad_mode, nullptr, s));
         const float* dz1 = (m.dense.size() > 1) ? m.dense[0].h : m.d_top;
-        TP_LAUNCH(m, "alpha_shortcut_sgemm", launch_sgemm(dz1, t.d_S, t.alpha_raw, n, T.Cout, m.dense[0].out, false, 1, s));
+        TP_LAUNCH(m, "alpha_shortcut_sgemm", launch_sgemm(dz1, t.d_S, alpha_dst, n, T.Cout, m.dense[0].out, false, 1, s));
+    } else if (rerun_head) {
+        TP_TRY(relaunch_fused_head(&m, class_idx, alpha_dst, s));                 // the fused head's alpha shortcut
     }
+    return BCAD_OK;
+}
+
+int tensor_explain_chunk(Model& m, int n, const int32_t* class_idx, int grad_mode, float* heat, cudaStream_t s, int K, size_t col_ld,
+                         size_t heat_stride) {
+    TensorPath& t = *m.tp;
+    const ConvLayer& T = m.conv.back();
     const float inv_hw = 1.0f / ((float)T.Ho * (float)T.Wo);
+    const size_t hm = (size_t)m.heat_h * m.heat_w, slot = (size_t)m.cfg.max_batch * T.Cout;
     // The one-launch cluster tail needs about a CTA pair per SM to pay (one image's pair streams its 2-4 MB map at a single SM
     // pair's bandwidth: 73 us whatever the batch); handles sized for a few images (single requests, the refinement twin) take the
     // two-launch form, whose channel reduction spreads one image over 8 CTAs (16 images: 30 instead of 72 us).  A property of the
     // HANDLE, so that a given handle's results do not depend on how a batch is chunked.
     const bool small_handle = m.cfg.max_batch <= 32;
-    if (!small_handle && tail_fused_supported(T.Ho, T.Wo, m.heat_h, m.heat_w, T.Cout) && getenv("BCAD_TAIL_TWO_KERNELS") == nullptr) {
-        TP_LAUNCH(m, "tail_fused", launch_tail_fused(t.act, t.alpha_raw, inv_hw, m.alpha, heat, n, T.Ho, T.Wo, m.heat_h, m.heat_w, T.Cout, t.x3, s, m.n_dev));
-        return BCAD_OK;
+    const bool fused = !small_handle && tail_fused_supported(T.Ho, T.Wo, m.heat_h, m.heat_w, T.Cout) && getenv("BCAD_TAIL_TWO_KERNELS") == nullptr;
+    // several classes: groups of TF_GROUP share one read of A in the fused tail; the two-launch form reads A once per class
+    const int group = (fused && K > 1 && tail_fused_classes_supported(T.Ho, T.Wo, m.heat_h, m.heat_w, T.Cout)) ? TF_GROUP : 1;
+    for (int k0 = 0; k0 < K; k0 += group) {
+        const int g = std::min(group, K - k0);
+        for (int j = 0; j < g; ++j) {
+            const int k = k0 + j;
+            TP_TRY(tensor_alpha(m, n, class_idx ? class_idx + k * col_ld : nullptr, grad_mode, t.alpha_raw + j * slot, k > 0, s));
+        }
+        float* hk = heat + k0 * hm;
+        if (g > 1) {
+            TP_LAUNCH(m, "tail_fused_classes", launch_tail_fused_classes(t.act, t.alpha_raw, slot, inv_hw, hk, heat_stride, n, T.Ho, T.Wo,
+                                                                         m.heat_h, m.heat_w, T.Cout, t.x3, s, m.n_dev));
+        } else if (fused) {
+            TP_LAUNCH(m, "tail_fused", launch_tail_fused(t.act, t.alpha_raw, inv_hw, m.alpha, hk, n, T.Ho, T.Wo, m.heat_h, m.heat_w, T.Cout, t.x3, s, m.n_dev,
+                                                         heat_stride));
+        } else {
+            TP_LAUNCH(m, "cam_c8", launch_cam_c8(t.act, t.alpha_raw, inv_hw, m.alpha, m.cam_lo, m.mm, n, T.Ho, T.Wo, T.Cout, m.cam_splits, t.x3, s, m.n_dev));
+            TP_LAUNCH(m, "upsample_norm", launch_upsample_norm(m.cam_lo, m.mm, m.cam_splits, hk, n, T.Ho, T.Wo, m.heat_h, m.heat_w, s, m.n_dev,
+                                                               heat_stride));
+        }
     }
-    TP_LAUNCH(m, "cam_c8", launch_cam_c8(t.act, t.alpha_raw, inv_hw, m.alpha, m.cam_lo, m.mm, n, T.Ho, T.Wo, T.Cout, m.cam_splits, t.x3, s, m.n_dev));
-    TP_LAUNCH(m, "upsample_norm", launch_upsample_norm(m.cam_lo, m.mm, m.cam_splits, heat, n, T.Ho, T.Wo, m.heat_h, m.heat_w, s, m.n_dev));
     return BCAD_OK;
 }
 

@@ -254,6 +254,47 @@ class Engine:
                                                                _ptr(logits), _ptr(probs), _ptr(cls), h, w, _ptr(heat), self._stream()))
         return cls, probs, logits, heat
 
+    def predict_explain_classes(self, x, classes=None, grad_mode: str = "logit", out_hw: Optional[Tuple[int, int]] = None,
+                                out_heat: Optional[torch.Tensor] = None):
+        """Grad-CAM for K target classes per image from one forward (the dual-class explanation of app.py:649-657 -> GRADCAM.py:63-64)
+        -> (cls, probs, logits, heatmaps fp32 [B,K,H,W]) as CUDA tensors.  ``classes``: None = every class (K = num_classes), a
+        length-K sequence shared by the batch, or a [B,K] array; K <= 8.  ``heat[:, k]`` is bitwise what ``predict_explain`` returns
+        for class column k."""
+        self.cache_tag = None
+        x = self._as_device_input(x)
+        B, nc = x.shape[0], self.spec.num_classes
+        h, w, _ = self.spec.input_shape
+        if out_hw is not None:
+            h, w = int(out_hw[0]), int(out_hw[1])
+            if h < 1 or w < 1:
+                raise ValueError(f"out_hw must be positive, got {out_hw}")
+        if classes is None:
+            K, ci = nc, None
+        else:
+            ci = torch.as_tensor(classes, dtype=torch.int32)
+            if ci.dim() == 1:
+                ci = ci[None].expand(B, -1)
+            if ci.dim() != 2 or ci.shape[0] != B:
+                raise ValueError(f"classes must be a length-K sequence or a [{B},K] array, got shape {tuple(ci.shape)}")
+            K = ci.shape[1]
+            if K >= 1 and (int(ci.min()) < 0 or int(ci.max()) >= nc):
+                raise ValueError("classes out of range")
+        if not 1 <= K <= _lib.MAX_EXPLAIN_CLASSES:
+            raise ValueError(f"{K} target classes per image; 1..{_lib.MAX_EXPLAIN_CLASSES} are supported")
+        with torch.cuda.device(self.tdev):
+            logits = torch.empty((B, nc), device=self.tdev, dtype=torch.float32)
+            probs = torch.empty((B, nc), device=self.tdev, dtype=torch.float32)
+            cls = torch.empty((B,), device=self.tdev, dtype=torch.int32)
+            heat = out_heat if out_heat is not None else torch.empty((B, K, h, w), device=self.tdev, dtype=torch.float32)
+            if tuple(heat.shape) != (B, K, h, w) or heat.dtype != torch.float32 or not heat.is_contiguous():
+                raise ValueError(f"out_heat must be a contiguous float32 [{B},{K},{h},{w}] tensor")
+            if ci is not None:
+                ci = ci.to(self.tdev).contiguous()
+            oh, ow = (h, w) if out_hw is not None else (0, 0)
+            _lib.check(self.lib.bcad_predict_explain_classes(self._h, _ptr(x), B, K, _ptr(ci), _lib.GRAD_MODE[grad_mode],
+                                                             _ptr(logits), _ptr(probs), _ptr(cls), oh, ow, _ptr(heat), self._stream()))
+        return cls, probs, logits, heat
+
     def _class_idx(self, class_idx, B):
         if class_idx is None:
             return None
