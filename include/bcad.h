@@ -159,6 +159,25 @@ BCAD_API int bcad_predict_explain_classes(bcad_model* m, const float* x_dev, int
 BCAD_API int bcad_explain_backward(bcad_model* m, int B, const int32_t* class_idx_dev, int grad_mode,
                           float* const* conv_act_grads_dev, float* d_input_dev, void* stream);
 
+/* Input-gradient saliency (explainability.py:44-78) for K target classes per image from ONE forward.  fp32 handles with
+ * keep_all_activations = 1 and no dropout masks set.  The kernels follow bcad_set_fast_training, as bcad_predict / bcad_train_backward
+ * do: with it on, the eligible conv blocks and fc1 run their input gradients on the split-operand tensor-core kernels (~1e-4 relative).
+ * A first block of one input channel, 32 filters, 3x3 and pad 0 / 1 runs as one fused kernel (plain fp32, summation order aside the
+ * same as bcad_explain_backward's d_input).  Chunked by max_batch: one forward per chunk, then one backward per class.
+ * classes_dev int32 [B][K] or NULL (column k = class k, K <= num_classes); 1 <= K <= BCAD_MAX_EXPLAIN_CLASSES; grad_mode BCAD_GRAD_*
+ * (the reference uses SOFTMAX_CE).  saliency_dev fp32 [B][K][H][W] = (s - min s) / (max s - min s + 1e-8), s = max_c |d_input| per
+ * image and class.  d_input_dev fp32 [B][K][H][W][C] or NULL.  logits / probs / cls as bcad_predict_explain (each may be NULL).
+ * saliency[:, k] and d_input[:, k] are bitwise what a K = 1 call with class column k returns; logits / probs / cls are bitwise
+ * bcad_predict's.  Afterwards the layer caches describe the last chunk's forward, as after bcad_predict. */
+BCAD_API int bcad_predict_saliency_classes(bcad_model* m, const float* x_dev, int B, int K, const int32_t* classes_dev, int grad_mode,
+                                           float* logits_dev, float* probs_dev, int32_t* cls_dev, float* saliency_dev,
+                                           float* d_input_dev, void* stream);
+/* generate_saliency_overlay (explainability.py:74-77) for [B][K] maps: heat = JET_BGR[uint8(sal * 255)] (fp32 product, truncating),
+ * overlay = addWeighted(base, 0.5, heat, 0.5, 0) (round half to even, as OpenCV's 8-bit path does).  base_dev uint8 [B][H][W][base_c],
+ * base_c = 1 (replicated to 3) or 3, shared by an image's K maps.  overlay_dev / heat_dev uint8 [B][K][H][W][3] (BGR), either may be NULL. */
+BCAD_API int bcad_saliency_overlay(const uint8_t* base_dev, int base_c, const float* saliency_dev, int B, int K, int H, int W,
+                                   uint8_t* overlay_dev, uint8_t* heat_dev, void* stream);
+
 /* cached tensors of the most recent forward / explain (layer['output'], ['z'] ... compat) -> dst_dev */
 BCAD_API int bcad_get_tensor(bcad_model* m, int kind, int index, int B, float* dst_dev, void* stream);
 /* number of fp32 elements per image of that tensor */

@@ -51,6 +51,8 @@ class CNNModel(nn.Module):
         self._versions = None
         self._train_eng = None           # fp32 handle of the train-mode forward (dropout lives on the fp32 path)
         self._train_versions = None
+        self._sal_eng = None             # fp32 handle with every activation kept, for the saliency maps (first use)
+        self._sal_versions = None
 
     # ------------------------------------------------------------------ engine plumbing
     def _make_engine(self):
@@ -85,6 +87,24 @@ class CNNModel(nn.Module):
     @property
     def engine(self) -> Engine:
         return self.sync_weights(force=False)
+
+    @property
+    def saliency_engine(self) -> Engine:
+        """fp32 handle with every activation kept and, where the network has their shape, the tensor-core input gradients of
+        ``set_fast_training``; serves ``predict_saliency_classes_batch``."""
+        ver = self._param_versions()
+        if self._sal_eng is None:
+            self._sal_eng = Engine(self._spec, precision="fp32", max_batch=self._max_batch, keep_all_activations=True,
+                                   device=self._device_index)
+            try:
+                self._sal_eng.set_fast_training(True)
+            except ValueError:                                 # no conv block of the tensor-core shape: the fp32 kernels
+                pass
+            self._sal_versions = None
+        if ver != self._sal_versions:
+            self._sal_eng.set_weights(*self._host_weights())
+            self._sal_versions = ver
+        return self._sal_eng
 
     # ------------------------------------------------------------------ forward (ADCNNM.py:72-78)
     def forward(self, x):
@@ -164,6 +184,13 @@ class CNNModel(nn.Module):
         a [B,K] array, or None = every class; ``heat[:, k]`` equals ``predict_explain_batch(x, classes[:, k])``'s heat-maps."""
         cls, probs, logits, heat = self.engine.predict_explain_classes(x, classes, grad_mode)
         return cls.long(), logits, heat
+
+    def predict_saliency_classes_batch(self, x, classes=(0, 1), grad_mode="logit"):
+        """Input-gradient saliency maps (|d logit / d x| max over channels, min-max normalised per image and class) for several
+        target classes per image from one forward -> (classes [B], logits [B,nc], saliency fp32 [B,K,H,W]) on the GPU.
+        ``classes``: a length-K sequence shared by the batch, a [B,K] array, or None = every class."""
+        cls, probs, logits, sal, _ = self.saliency_engine.predict_saliency_classes(x, classes, grad_mode)
+        return cls.long(), logits, sal
 
 
 def _pull_into_modules(model, eng):

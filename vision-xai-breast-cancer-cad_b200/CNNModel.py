@@ -90,6 +90,8 @@ class CNNModel:
         self._weights_key = None
         self._fast = None               # fast handle (None: not created yet; the compat handle itself when the shape is not covered)
         self._fast_key = None
+        self._sal = None                # saliency handle (fp32, every activation kept, fast training where accepted); first use
+        self._sal_key = None
         self._gen = 0                   # forward() generation: the lazy layer caches and the explain backward check it
         self._last_x = None
         self._last_masks = None
@@ -160,6 +162,7 @@ class CNNModel:
             self._weights_key = key
             if force:
                 self._fast_key = None
+                self._sal_key = None
         return self._engine
 
     @property
@@ -186,6 +189,27 @@ class CNNModel:
             self._upload(self._fast)
             self._fast_key = key
         return self._fast
+
+    @property
+    def saliency_engine(self) -> Engine:
+        """The handle of the batched saliency calls: fp32 with every activation kept, and the tensor-core input gradients of
+        ``set_fast_training`` where the network has their shape.  A handle of its own, so that the compat handle keeps the
+        reference-pinned kernels."""
+        if self._dirty:
+            self._pull_weights()
+        if self._sal is None:
+            self._sal = Engine(self._spec(), precision="fp32", max_batch=self._max_batch, keep_all_activations=True,
+                               device=self._device)
+            try:
+                self._sal.set_fast_training(True)
+            except ValueError:                                 # no conv block of the tensor-core shape: the fp32 kernels
+                pass
+            self._sal_key = None
+        key = self._key()
+        if key != self._sal_key:
+            self._upload(self._sal)
+            self._sal_key = key
+        return self._sal
 
     # ------------------------------------------------------------------ forward / predict
     def forward(self, x, training=True):
@@ -320,6 +344,16 @@ class CNNModel:
             X = X.astype(np.float32) / np.float32(255.0)
         cls, probs, _, heat = self._batch_engine().predict_explain_classes(np.asarray(X, dtype=np.float32), classes, grad_mode)
         return cls.cpu().numpy().astype(np.int64), probs.cpu().numpy(), heat.cpu().numpy()
+
+    def predict_saliency_classes_batch(self, X, classes=(0, 1), grad_mode="softmax_ce"):
+        """X [B,H,W,C] -> (classes [B], probs [B,nc], input-gradient saliency maps float32 [B,K,H,W] in [0,1]) for K target classes
+        per image from one forward (explainability.py:44-73 per class).  ``classes``: a length-K sequence shared by the batch, a
+        [B,K] array, or None = every class.  Runs on ``saliency_engine``."""
+        X = np.asarray(X)
+        if X.dtype == np.uint8:
+            X = X.astype(np.float32) / np.float32(255.0)
+        cls, probs, _, sal, _ = self.saliency_engine.predict_saliency_classes(np.asarray(X, dtype=np.float32), classes, grad_mode)
+        return cls.cpu().numpy().astype(np.int64), probs.cpu().numpy(), sal.cpu().numpy()
 
     # ------------------------------------------------------------------ persistence (Classes/CNNModel.py:530-555)
     def save_model(self, path="trained_model/cnn_model.npz"):

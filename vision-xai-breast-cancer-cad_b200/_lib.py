@@ -58,6 +58,8 @@ _SIGNATURES = {
     "bcad_predict_explain_classes": (C.c_int, [_P, _P, C.c_int, C.c_int, _P, C.c_int, _P, _P, _P, C.c_int, C.c_int, _P, _P]),
     "bcad_gradcam_overlays_host": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, _P, _P, _P, _P, _P]),
     "bcad_explain_backward": (C.c_int, [_P, C.c_int, _P, C.c_int, C.POINTER(_P), _P, _P]),
+    "bcad_predict_saliency_classes": (C.c_int, [_P, _P, C.c_int, C.c_int, _P, C.c_int, _P, _P, _P, _P, _P, _P]),
+    "bcad_saliency_overlay": (C.c_int, [_P, C.c_int, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P]),
     "bcad_get_tensor": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, _P, _P]),
     "bcad_tensor_elems": (C.c_int64, [_P, C.c_int, C.c_int]),
     "bcad_predict_explain_host": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, _P, _P, _P]),

@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libbcad.so")
-SOURCES = ["api.cu", "kernels_fp32.cu", "tensor_path.cu", "sm100_selftest.cu", "sm100_kernels.cu", "sm100_wide.cu", "sm100_tail.cu", "sm100_fused.cu", "sm100_fused2.cu", "kernels_train.cu", "sm100_train.cu", "api_train.cu", "refine.cu", "sm100_unet.cu"]
+SOURCES = ["api.cu", "kernels_fp32.cu", "tensor_path.cu", "sm100_selftest.cu", "sm100_kernels.cu", "sm100_wide.cu", "sm100_tail.cu", "sm100_fused.cu", "sm100_fused2.cu", "kernels_train.cu", "sm100_train.cu", "api_train.cu", "refine.cu", "sm100_unet.cu", "saliency.cu"]
 FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
          "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr"]
 

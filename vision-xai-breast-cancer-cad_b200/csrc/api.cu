@@ -524,6 +524,43 @@ int dense_backward(Model* m, int n, const int32_t* class_idx, int grad_mode, flo
     return BCAD_OK;
 }
 
+int conv_block_dz(Model* m, int i, const float* gp, int B, bool fused, float* act_grad, bool mask, cudaStream_t s) {
+    ConvLayer& L = m->conv[i];
+    const size_t elems = (size_t)B * L.Ho * L.Wo * L.Cout;
+    if (L.dz == nullptr) BCAD_TRY(m->alloc((void**)&L.dz, (size_t)m->cfg.max_batch * L.Ho * L.Wo * L.Cout * sizeof(float)));
+    if (fused) {
+        const int first_only = (m->cfg.pool_ties == BCAD_TIES_FIRST) ? 1 : 0;
+        BCAD_LAUNCH(m, "unpool_mask", launch_unpool_mask(gp, L.y, L.dz, B, L.Ho, L.Wo, L.Cout, first_only, m->cfg.alpha_conv, s));
+        return BCAD_OK;
+    }
+    BCAD_LAUNCH(m, "unpool", launch_unpool(gp, L.y, L.dz, B, L.Ho, L.Wo, L.Cout, m->cfg.pool_ties, s));
+    if (act_grad) BCAD_CUDA_CHECK(cudaMemcpyAsync(act_grad, L.dz, elems * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    if (mask) BCAD_LAUNCH(m, "leaky_mask_mul", launch_leaky_mask_mul(L.dz, L.y, m->cfg.alpha_conv, (int64_t)elems, s));   // explainability.py:55
+    return BCAD_OK;
+}
+
+int conv_block_dgrad(Model* m, int i, int B, float* dst, bool tc, const char* name, cudaStream_t s) {
+    ConvLayer& L = m->conv[i];
+    if (dst == nullptr) {
+        ConvLayer& P = m->conv[i - 1];
+        if (P.gp == nullptr) BCAD_TRY(m->alloc((void**)&P.gp, (size_t)m->cfg.max_batch * P.Hp * P.Wp * P.Cout * sizeof(float)));
+        dst = P.gp;
+    }
+    if (tc) {
+        TcConvArgs t;
+        t.x = L.dz; t.w_img = L.tc_wd; t.bias = nullptr; t.y = dst; t.B = B; t.H = L.Ho; t.W = L.Wo; t.Ho = L.H; t.Wo = L.W;
+        t.pad = L.k - 1 - m->cfg.pad; t.alpha = 1.f; t.a_bf16 = 1;
+        BCAD_LAUNCH(m, "conv_dgrad_tcgen05_x3", launch_conv3x3_x3(t, L.Cout, L.Cin, m->sms, s));
+        return BCAD_OK;
+    }
+    ConvArgs a;
+    a.x = L.dz; a.w = L.d_w_dgrad; a.bias = L.d_zero_bias; a.y = dst; a.p = nullptr;
+    a.B = B; a.H = L.Ho; a.W = L.Wo; a.Cin = L.Cout; a.Cout = L.Cin; a.CoutPad = cdiv(L.Cin, 32) * 32;
+    a.ksize = L.k; a.pad = L.k - 1 - m->cfg.pad; a.Ho = L.H; a.Wo = L.W; a.Hp = 0; a.Wp = 0; a.alpha = 1.f;
+    BCAD_LAUNCH(m, name, launch_conv_fp32(a, s));
+    return BCAD_OK;
+}
+
 static int tail_chunk(Model* m, const void* A, int a_dtype, int n, float* heat, size_t heat_stride, cudaStream_t s) {
     const ConvLayer& T = m->conv.back();
     const float inv_hw = 1.0f / ((float)T.Ho * (float)T.Wo);
@@ -650,6 +687,93 @@ static int run(Model* m, const float* x, int B, const int32_t* class_idx, int gr
     return BCAD_OK;
 }
 
+// Saliency of one target class column ck for the chunk's cached forward (explainability.py:44-73): dense backward to the fc1 input
+// gradient, the conv blocks from the last to the second with the kernels bcad_train_backward uses, then the first block's input
+// gradient with |.| and the per-image min / max.  Image b's map goes to sal + b * stride (d_input: + b * stride * C).
+static int saliency_class(Model* m, int n, const int32_t* ck, int grad_mode, float* sal, float* d_input, size_t stride, uint32_t* mm,
+                          int mm_ld, cudaStream_t s) {
+    DenseLayer& D0 = m->dense[0];
+    const bool tc_fc1 = m->fast_train && dense_bwd_x3_supported(n, D0.out, D0.in);
+    if (!m->fused_head) BCAD_TRY(dense_backward(m, n, ck, grad_mode, tc_fc1 ? nullptr : m->g_flat, s));
+    // dz1: left in dense[0].h by the fused head or the dense chain (d_top itself when the output layer is the only dense layer)
+    const float* dz1 = (m->fused_head || m->dense.size() > 1) ? D0.h : m->d_top;
+    if (tc_fc1) {
+        DenseBwdArgs dg;
+        dg.dz = dz1; dg.src = D0.d_w; dg.out = m->g_flat; dg.B = n; dg.units = D0.out; dg.flat = D0.in;
+        BCAD_LAUNCH(m, "dense_dgrad_tcgen05_x3", launch_dense_bwd_x3(dg, 1, m->sms, s));
+    } else if (m->fused_head) {
+        BCAD_LAUNCH(m, "fc1_dgrad_sgemm", launch_sgemm(dz1, D0.d_w, m->g_flat, n, D0.in, D0.out, false, 1, s));
+    }
+    const float* gp = m->g_flat;
+    for (int i = (int)m->conv.size() - 1; i >= 1; --i) {
+        const bool tc = m->fast_train && tc_train_eligible(m, (size_t)i);
+        BCAD_TRY(conv_block_dz(m, i, gp, n, tc, nullptr, true, s));
+        BCAD_TRY(conv_block_dgrad(m, i, n, nullptr, tc, "conv_fp32", s));
+        gp = m->conv[i - 1].gp;
+    }
+    ConvLayer& L = m->conv[0];
+    const int hw = L.H * L.W;
+    if (saliency_conv0_supported(L.Cin, L.Cout, L.CoutPad, L.k, m->cfg.pad)) {
+        BCAD_LAUNCH(m, "saliency_conv0", launch_saliency_conv0(gp, L.y, L.d_w, n, L.H, L.W, L.Ho, L.Wo, m->cfg.pad,
+                                                             m->cfg.pool_ties == BCAD_TIES_FIRST ? 1 : 0, m->cfg.alpha_conv, d_input, sal,
+                                                             stride, mm, mm_ld, s));
+        return BCAD_OK;
+    }
+    if (m->sal_din == nullptr) BCAD_TRY(m->alloc((void**)&m->sal_din, (size_t)m->cfg.max_batch * hw * L.Cin * sizeof(float)));
+    BCAD_TRY(conv_block_dz(m, 0, gp, n, false, nullptr, true, s));
+    BCAD_TRY(conv_block_dgrad(m, 0, n, m->sal_din, false, "conv_fp32", s));
+    BCAD_LAUNCH(m, "saliency_absmax", launch_saliency_absmax(m->sal_din, n, hw, L.Cin, d_input, sal, stride, mm, mm_ld, s));
+    return BCAD_OK;
+}
+
+static int run_saliency(Model* m, const float* x, int B, int K, const int32_t* classes, int grad_mode, float* logits, float* probs,
+                        int32_t* cls, float* saliency, float* d_input, cudaStream_t s) {
+    BCAD_REQUIRE(m && x, "predict_saliency_classes: null model or input");
+    if (m->tensor_path) {
+        set_error("predict_saliency_classes runs on the fp32 path (the 16-bit forward keeps no first-block output): create the model with BCAD_PREC_FP32");
+        return BCAD_ERR_INVALID;
+    }
+    BCAD_REQUIRE(m->cfg.keep_all_activations, "predict_saliency_classes needs every conv block's output: create the model with keep_all_activations=1");
+    BCAD_REQUIRE(!m->train.drop_B, "predict_saliency_classes is an inference call: clear the dropout masks first (bcad_set_dropout_masks(m, NULL, 0))");
+    BCAD_REQUIRE(K >= 1 && K <= BCAD_MAX_EXPLAIN_CLASSES, "predict_saliency_classes: K=%d out of range 1..%d", K, BCAD_MAX_EXPLAIN_CLASSES);
+    BCAD_REQUIRE(classes || K <= m->cfg.num_classes, "predict_saliency_classes: classes=NULL explains classes 0..K-1, but K=%d > num_classes=%d",
+                 K, m->cfg.num_classes);
+    BCAD_REQUIRE(saliency, "predict_saliency_classes: saliency output pointer is null");
+    BCAD_REQUIRE(B >= 1, "batch must be >= 1, got %d", B);
+    BCAD_REQUIRE(grad_mode == BCAD_GRAD_LOGIT || grad_mode == BCAD_GRAD_SOFTMAX_CE, "bad grad_mode %d", grad_mode);
+    if (!m->committed) { set_error("weights not committed: call bcad_commit first"); return BCAD_ERR_STATE; }
+    DeviceGuard g(m->cfg.device);
+    std::lock_guard<std::mutex> lock(m->mu);
+    BCAD_CUDA_CHECK(cudaStreamWaitEvent(s, m->call_done, 0));
+    if (m->sal_mm == nullptr) BCAD_TRY(m->alloc((void**)&m->sal_mm, (size_t)m->cfg.max_batch * BCAD_MAX_EXPLAIN_CLASSES * 2 * sizeof(uint32_t)));
+    const int mb = m->cfg.max_batch, nc = m->cfg.num_classes;
+    const size_t hw = (size_t)m->cfg.in_h * m->cfg.in_w, img = hw * m->cfg.in_c;
+    m->prof_n = 0;
+    m->multi_class_call = false;
+    for (int b0 = 0; b0 < B; b0 += mb) {
+        const int n = std::min(mb, B - b0);
+        BCAD_LAUNCH(m, "class_columns", launch_class_columns(classes ? classes + (size_t)b0 * K : nullptr, K, n, m->class_cols, mb, s));
+        BCAD_TRY(forward_chunk_fp32(m, x + (size_t)b0 * img, n, true, m->class_cols, grad_mode, s));
+        BCAD_CUDA_CHECK(cudaMemsetAsync(m->sal_mm, 0, (size_t)n * K * 2 * sizeof(uint32_t), s));
+        float* sc = saliency + (size_t)b0 * K * hw;
+        for (int k = 0; k < K; ++k) {
+            const int32_t* ck = m->class_cols + (size_t)k * mb;
+            if (k > 0 && m->fused_head) BCAD_TRY(relaunch_fused_head(m, ck, nullptr, s));     // dz1 of class k
+            BCAD_TRY(saliency_class(m, n, ck, grad_mode, sc + (size_t)k * hw, d_input ? d_input + ((size_t)b0 * K + k) * img : nullptr,
+                                    (size_t)K * hw, m->sal_mm + 2 * k, 2 * K, s));
+        }
+        BCAD_LAUNCH(m, "saliency_norm", launch_saliency_norm(sc, n * K, (int)hw, m->sal_mm, s));
+        if (logits) BCAD_CUDA_CHECK(cudaMemcpyAsync(logits + (size_t)b0 * nc, m->dense.back().z, (size_t)n * nc * sizeof(float), cudaMemcpyDeviceToDevice, s));
+        if (probs) BCAD_CUDA_CHECK(cudaMemcpyAsync(probs + (size_t)b0 * nc, m->probs, (size_t)n * nc * sizeof(float), cudaMemcpyDeviceToDevice, s));
+        if (cls) BCAD_CUDA_CHECK(cudaMemcpyAsync(cls + b0, m->cls, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToDevice, s));
+        m->cached_B = n;
+    }
+    if (B > mb) m->cached_B = 0;   // the cache only describes whole calls
+    BCAD_TRY(m->mark("end", s));
+    BCAD_CUDA_CHECK(cudaEventRecord(m->call_done, s));
+    return BCAD_OK;
+}
+
 }  // namespace bcad
 
 extern "C" {
@@ -679,6 +803,20 @@ int bcad_predict_explain_classes(bcad_model* mm, const float* x, int B, int K, c
     BCAD_REQUIRE(classes || K <= m->cfg.num_classes, "predict_explain_classes: classes=NULL explains classes 0..K-1, but K=%d > num_classes=%d",
                  K, m->cfg.num_classes);
     return run(m, x, B, classes, grad_mode, true, logits, probs, cls, heat, (cudaStream_t)stream, out_h, out_w, K);
+}
+
+int bcad_predict_saliency_classes(bcad_model* mm, const float* x, int B, int K, const int32_t* classes, int grad_mode, float* logits,
+                                  float* probs, int32_t* cls, float* saliency, float* d_input, void* stream) {
+    return run_saliency(reinterpret_cast<Model*>(mm), x, B, K, classes, grad_mode, logits, probs, cls, saliency, d_input, (cudaStream_t)stream);
+}
+
+int bcad_saliency_overlay(const uint8_t* base, int base_c, const float* saliency, int B, int K, int H, int W, uint8_t* overlay,
+                          uint8_t* heat, void* stream) {
+    BCAD_REQUIRE(base && saliency, "saliency_overlay: null base image or saliency");
+    BCAD_REQUIRE(base_c == 1 || base_c == 3, "saliency_overlay: base_c must be 1 or 3, got %d", base_c);
+    BCAD_REQUIRE(B >= 1 && K >= 1 && H >= 1 && W >= 1 && (int64_t)H * W <= 0x7fffffff, "saliency_overlay: bad sizes B=%d K=%d %dx%d", B, K, H, W);
+    if (overlay == nullptr && heat == nullptr) return BCAD_OK;
+    return launch_saliency_overlay(base, base_c, saliency, B, K, H * W, overlay, heat, (cudaStream_t)stream);
 }
 
 int bcad_explain_backward(bcad_model* mm, int B, const int32_t* class_idx, int grad_mode,
@@ -713,26 +851,11 @@ int bcad_explain_backward(bcad_model* mm, int B, const int32_t* class_idx, int g
     BCAD_TRY(dense_backward(m, B, class_idx, grad_mode, m->g_flat, s));
     const float* gp = m->g_flat;
     for (int i = nconv - 1; i >= lowest; --i) {
-        ConvLayer& L = m->conv[i];
-        const size_t elems = (size_t)B * L.Ho * L.Wo * L.Cout;
-        if (L.dz == nullptr) BCAD_TRY(m->alloc((void**)&L.dz, (size_t)m->cfg.max_batch * L.Ho * L.Wo * L.Cout * sizeof(float)));
-        BCAD_LAUNCH(m, "unpool", launch_unpool(gp, L.y, L.dz, B, L.Ho, L.Wo, L.Cout, m->cfg.pool_ties, s));
-        if (conv_act_grads && conv_act_grads[i])
-            BCAD_CUDA_CHECK(cudaMemcpyAsync(conv_act_grads[i], L.dz, elems * sizeof(float), cudaMemcpyDeviceToDevice, s));
-        if (i == lowest && !d_input) break;
-        BCAD_LAUNCH(m, "leaky_mask_mul", launch_leaky_mask_mul(L.dz, L.y, m->cfg.alpha_conv, (int64_t)elems, s));   // explainability.py:55
-        float* dst = d_input;
-        if (i > 0) {
-            ConvLayer& P = m->conv[i - 1];
-            if (P.gp == nullptr) BCAD_TRY(m->alloc((void**)&P.gp, (size_t)m->cfg.max_batch * P.Hp * P.Wp * P.Cout * sizeof(float)));
-            dst = P.gp;
-        }
-        ConvArgs a;
-        a.x = L.dz; a.w = L.d_w_dgrad; a.bias = L.d_zero_bias; a.y = dst; a.p = nullptr;
-        a.B = B; a.H = L.Ho; a.W = L.Wo; a.Cin = L.Cout; a.Cout = L.Cin; a.CoutPad = cdiv(L.Cin, 32) * 32;
-        a.ksize = L.k; a.pad = L.k - 1 - m->cfg.pad; a.Ho = L.H; a.Wo = L.W; a.Hp = 0; a.Wp = 0; a.alpha = 1.f;
-        BCAD_LAUNCH(m, "conv_fp32", launch_conv_fp32(a, s));
-        gp = dst;
+        const bool last = (i == lowest && !d_input);
+        BCAD_TRY(conv_block_dz(m, i, gp, B, false, conv_act_grads ? conv_act_grads[i] : nullptr, !last, s));
+        if (last) break;
+        BCAD_TRY(conv_block_dgrad(m, i, B, i > 0 ? nullptr : d_input, false, "conv_fp32", s));
+        gp = i > 0 ? m->conv[i - 1].gp : d_input;
     }
     BCAD_CUDA_CHECK(cudaEventRecord(m->call_done, s));
     return BCAD_OK;

@@ -194,7 +194,6 @@ int bcad_train_backward_part(bcad_model* mm, const float* x, const int32_t* labe
     const float* gp = m->g_flat;
     for (int i = nconv - 1; i >= 0; --i) {
         ConvLayer& L = m->conv[i];
-        const size_t elems = (size_t)B * L.Ho * L.Wo * L.Cout;
         const int first_only = (m->cfg.pool_ties == BCAD_TIES_FIRST) ? 1 : 0;
         if (m->fast_train && i == 0 && L.Cin == 1 && L.Cout == 32 && L.CoutPad == 32 && L.k == 3 && getenv("BCAD_TC_NO_CONV0") == nullptr) {
             // first block, one input channel: pool backward + LeakyReLU' + dF / db in one pass, the full-resolution gradient is never written
@@ -204,13 +203,7 @@ int bcad_train_backward_part(bcad_model* mm, const float* x, const int32_t* labe
             m->launches += 1;
             continue;
         }
-        if (L.dz == nullptr) TR_TRY(m->alloc((void**)&L.dz, (size_t)m->cfg.max_batch * L.Ho * L.Wo * L.Cout * sizeof(float)));
-        if (m->fast_train && L.Cout % 4 == 0) {
-            TR_LAUNCH(m, "unpool_mask", launch_unpool_mask(gp, L.y, L.dz, B, L.Ho, L.Wo, L.Cout, first_only, m->cfg.alpha_conv, s));
-        } else {
-        TR_LAUNCH(m, "unpool", launch_unpool(gp, L.y, L.dz, B, L.Ho, L.Wo, L.Cout, m->cfg.pool_ties, s));
-        TR_LAUNCH(m, "leaky_mask_mul", launch_leaky_mask_mul(L.dz, L.y, m->cfg.alpha_conv, (int64_t)elems, s));
-        }
+        TR_TRY(conv_block_dz(m, i, gp, B, m->fast_train && L.Cout % 4 == 0, nullptr, true, s));
         const float* in_i = (i == 0) ? x : m->conv[i - 1].p;
         const bool tc = m->fast_train && tc_train_eligible(m, (size_t)i);
         const bool tc_w = tc && getenv("BCAD_TC_NO_WGRAD") == nullptr, tc_d = tc && getenv("BCAD_TC_NO_DGRAD") == nullptr;   // (fault isolation)
@@ -232,24 +225,9 @@ int bcad_train_backward_part(bcad_model* mm, const float* x, const int32_t* labe
                                                     L.Cin, L.Cout, L.CoutPad, L.k, m->cfg.pad, L.Ho, L.Wo, rows, s));
         m->launches += 2;                                    // the two partial reductions
         }
-        if (i > 0 && tc_d) {
-            ConvLayer& P = m->conv[i - 1];
-            if (P.gp == nullptr) TR_TRY(m->alloc((void**)&P.gp, (size_t)m->cfg.max_batch * P.Hp * P.Wp * P.Cout * sizeof(float)));
-            TcConvArgs t;
-            t.x = L.dz; t.w_img = L.tc_wd; t.bias = nullptr; t.y = P.gp; t.B = B; t.H = L.Ho; t.W = L.Wo; t.Ho = L.H; t.Wo = L.W;
-            t.pad = L.k - 1 - m->cfg.pad; t.alpha = 1.f; t.a_bf16 = 1;
-            TR_LAUNCH(m, "conv_dgrad_tcgen05_x3", launch_conv3x3_x3(t, L.Cout, L.Cin, m->sms, s));
-            gp = P.gp;
-        } else
         if (i > 0) {
-            ConvLayer& P = m->conv[i - 1];
-            if (P.gp == nullptr) TR_TRY(m->alloc((void**)&P.gp, (size_t)m->cfg.max_batch * P.Hp * P.Wp * P.Cout * sizeof(float)));
-            ConvArgs a;
-            a.x = L.dz; a.w = L.d_w_dgrad; a.bias = L.d_zero_bias; a.y = P.gp; a.p = nullptr;
-            a.B = B; a.H = L.Ho; a.W = L.Wo; a.Cin = L.Cout; a.Cout = L.Cin; a.CoutPad = cdiv(L.Cin, 32) * 32;
-            a.ksize = L.k; a.pad = L.k - 1 - m->cfg.pad; a.Ho = L.H; a.Wo = L.W; a.Hp = 0; a.Wp = 0; a.alpha = 1.f;
-            TR_LAUNCH(m, "conv_dgrad", launch_conv_fp32(a, s));
-            gp = P.gp;
+            TR_TRY(conv_block_dgrad(m, i, B, nullptr, tc_d, "conv_dgrad", s));
+            gp = m->conv[i - 1].gp;
         }
     }
     TR_TRY(m->mark("end", s));

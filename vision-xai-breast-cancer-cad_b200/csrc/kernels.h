@@ -59,6 +59,24 @@ int launch_avg_pool(const float* x, float* out, int B, int H, int W, int C, int 
 int launch_pad_conv_weights(const float* w, float* out, int taps, int Cin, int Cout, int CoutPad, cudaStream_t s);
 int launch_overlay(const float* img01, const float* cam, int B, int H, int W, uint8_t* overlay_rgb,
                    uint8_t* heat_u8, cudaStream_t s);
+// generate_saliency_overlay for [B][K] maps: base u8 [B][npix][base_c] (1 = grey, replicated; 3 = BGR), sal fp32 [B][K][npix],
+// overlay / heat u8 [B][K][npix][3] BGR (either may be null)
+int launch_saliency_overlay(const uint8_t* base, int base_c, const float* sal, int B, int K, int npix, uint8_t* overlay, uint8_t* heat,
+                            cudaStream_t s);
+
+// ---------------------------------------------------------------- input-gradient saliency (saliency.cu)
+// Outputs of one target class: image b's map at sal + b * out_stride (d_input: + b * out_stride * C), its min / max counters at
+// mm + b * mm_ld (two uint32, zeroed before the class's first kernel).
+// First block of one input channel, 32 filters, 3x3, pad 0 / 1: pool backward + LeakyReLU' + input gradient + |.| + min / max from the
+// block's pooled gradient g and its output y, without the full-resolution gradient
+bool saliency_conv0_supported(int Cin, int Cout, int CoutPad, int k, int pad);
+int launch_saliency_conv0(const float* g, const float* y, const float* w, int B, int H, int W, int Ho, int Wo, int pad, int first_only,
+                          float alpha, float* d_input, float* sal, size_t out_stride, uint32_t* mm, int mm_ld, cudaStream_t s);
+// any other first block: s = max_c |d| and min / max from its input gradient d [B][hw][C]
+int launch_saliency_absmax(const float* d, int B, int hw, int C, float* d_input, float* sal, size_t out_stride, uint32_t* mm, int mm_ld,
+                           cudaStream_t s);
+// (s - min) / (max - min + 1e-8) in place over `maps` consecutive maps of hw pixels, counters mm[2 * map ..]
+int launch_saliency_norm(float* sal, int maps, int hw, const uint32_t* mm, cudaStream_t s);
 
 // ---------------------------------------------------------------- training step (kernels_train.cu)
 int launch_ce_loss_topgrad(const float* probs, const int32_t* labels, float* loss, float* dz, int B, int nc, cudaStream_t s);

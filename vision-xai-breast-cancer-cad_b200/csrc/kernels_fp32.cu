@@ -1012,6 +1012,31 @@ overlay_kernel(const float* __restrict__ img01, const float* __restrict__ cam, i
     for (int i = n4 * 4 + threadIdx.x; i < npix; i += blockDim.x) rgb(cb[i], ib[i], ob + (size_t)i * 3);
 }
 
+// generate_saliency_overlay (explainability.py:74-77) for [B][K] saliency maps: heat = JET_BGR[uint8(s * 255)] (fp32 product,
+// truncation), overlay = addWeighted(base, 0.5, heat, 0.5, 0).  OpenCV's 8-bit path rounds a * 0.5 + b * 0.5 half to even, i.e.
+// (a + b) / 2 with an odd sum rounded to the even neighbour.  The base image (1 channel replicated, or BGR) is shared by an image's K maps.
+__global__ void __launch_bounds__(256) saliency_overlay_kernel(const uint8_t* __restrict__ base, int base_c, const float* __restrict__ sal,
+                                                               int K, size_t npix, size_t total, uint8_t* __restrict__ overlay,
+                                                               uint8_t* __restrict__ heat) {
+    __shared__ uint8_t s_lut[256 * 3];
+    for (int i = threadIdx.x; i < 768; i += blockDim.x) s_lut[i] = c_jet_bgr[i];
+    __syncthreads();
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {   // i = map * npix + p
+        const size_t img = i / npix / K, p = i % npix;
+        const int li = (int)(uint8_t)(int)(sal[i] * 255.f);
+        const uint8_t* px = base + (img * npix + p) * base_c;
+#pragma unroll
+        for (int ch = 0; ch < 3; ++ch) {
+            const int h = s_lut[li * 3 + ch];
+            if (heat) heat[i * 3 + ch] = (uint8_t)h;
+            if (overlay) {
+                const int sum = px[base_c == 3 ? ch : 0] + h, q = sum >> 1;
+                overlay[i * 3 + ch] = (uint8_t)(q + (sum & q & 1));
+            }
+        }
+    }
+}
+
 // heatmap_uint8 = (cam * 255).astype(np.uint8)  (GRADCAM.py:70: truncation), 4 pixels per thread
 __global__ void __launch_bounds__(256) heat_to_u8_kernel(const float* __restrict__ cam, uint8_t* __restrict__ out, size_t n) {
     const size_t n4 = n / 4;
@@ -1120,6 +1145,15 @@ int launch_gray_preprocess(const uint8_t* g8, float* img01, float* x, int B, int
 int launch_overlay(const float* img01, const float* cam, int B, int H, int W, uint8_t* overlay_rgb, uint8_t* heat_u8,
                    cudaStream_t s) {
     overlay_kernel<<<B, 1024, 0, s>>>(img01, cam, H, W, overlay_rgb, heat_u8);
+    BCAD_CUDA_CHECK(cudaGetLastError());
+    return BCAD_OK;
+}
+
+int launch_saliency_overlay(const uint8_t* base, int base_c, const float* sal, int B, int K, int npix, uint8_t* overlay, uint8_t* heat,
+                            cudaStream_t s) {
+    const size_t total = (size_t)B * K * npix;
+    const int blocks = (int)std::min((size_t)148 * 16, (total + 255) / 256);
+    saliency_overlay_kernel<<<blocks, 256, 0, s>>>(base, base_c, sal, K, (size_t)npix, total, overlay, heat);
     BCAD_CUDA_CHECK(cudaGetLastError());
     return BCAD_OK;
 }

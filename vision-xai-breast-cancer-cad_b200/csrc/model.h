@@ -142,6 +142,8 @@ struct Model {
     bool multi_class_call = false;      // the last call explained several classes: alpha / cam_lo describe none of them
     HeadArgs head_last;                 // arguments of the chunk's dense_head_kernel launch, re-launched per extra target class
     int head_n = 0;
+    float* sal_din = nullptr;           // bcad_predict_saliency_classes (first use): input gradient of a first block without the fused kernel
+    uint32_t* sal_mm = nullptr;         //   per-map min / max counters [max_batch][BCAD_MAX_EXPLAIN_CLASSES][2]
     cudaEvent_t call_done = nullptr;
     std::vector<cudaEvent_t> prof_pool;   // profiling marks of the last call: event i precedes kernel i
     std::vector<const char*> prof_names;
@@ -162,6 +164,15 @@ bool tc_train_eligible(const Model* m, size_t i);
 int tc_train_refresh(Model* m, cudaStream_t s);
 
 int dense_backward(Model* m, int n, const int32_t* class_idx, int grad_mode, float* g_flat, cudaStream_t s);
+
+// One step of the conv-block backward shared by explain_backward, the training step and the saliency call.
+// conv_block_dz: conv[i].dz = gradient w.r.t. the block's pre-activation from gp (gradient w.r.t. its pooled output).  fused: pool
+// backward and LeakyReLU' in one pass (unpool_mask); else unpool, then act_grad (when given) receives the gradient w.r.t. the
+// post-activation output, then leaky_mask_mul unless mask is false.
+int conv_block_dz(Model* m, int i, const float* gp, int B, bool fused, float* act_grad, bool mask, cudaStream_t s);
+// conv_block_dgrad: the block's input gradient from conv[i].dz into dst (nullptr = conv[i - 1].gp, allocated on first use).  tc: the
+// split-operand tcgen05 kernel (fast training, tc_train_eligible block); else conv_fp32 with the flipped filters, profiled as `name`.
+int conv_block_dgrad(Model* m, int i, int B, float* dst, bool tc, const char* name, cudaStream_t s);
 
 bool fused_head_ok(const Model* m);
 // everything after the fc1 GEMM in one launch (dense_head_kernel); dz1 / S / alpha_raw are optional outputs

@@ -268,19 +268,7 @@ class Engine:
             h, w = int(out_hw[0]), int(out_hw[1])
             if h < 1 or w < 1:
                 raise ValueError(f"out_hw must be positive, got {out_hw}")
-        if classes is None:
-            K, ci = nc, None
-        else:
-            ci = torch.as_tensor(classes, dtype=torch.int32)
-            if ci.dim() == 1:
-                ci = ci[None].expand(B, -1)
-            if ci.dim() != 2 or ci.shape[0] != B:
-                raise ValueError(f"classes must be a length-K sequence or a [{B},K] array, got shape {tuple(ci.shape)}")
-            K = ci.shape[1]
-            if K >= 1 and (int(ci.min()) < 0 or int(ci.max()) >= nc):
-                raise ValueError("classes out of range")
-        if not 1 <= K <= _lib.MAX_EXPLAIN_CLASSES:
-            raise ValueError(f"{K} target classes per image; 1..{_lib.MAX_EXPLAIN_CLASSES} are supported")
+        K, ci = self._class_rows(classes, B)
         with torch.cuda.device(self.tdev):
             logits = torch.empty((B, nc), device=self.tdev, dtype=torch.float32)
             probs = torch.empty((B, nc), device=self.tdev, dtype=torch.float32)
@@ -294,6 +282,46 @@ class Engine:
             _lib.check(self.lib.bcad_predict_explain_classes(self._h, _ptr(x), B, K, _ptr(ci), _lib.GRAD_MODE[grad_mode],
                                                              _ptr(logits), _ptr(probs), _ptr(cls), oh, ow, _ptr(heat), self._stream()))
         return cls, probs, logits, heat
+
+    def predict_saliency_classes(self, x, classes=None, grad_mode: str = "softmax_ce", want_d_input: bool = False):
+        """Input-gradient saliency (explainability.py:44-73) for K target classes per image from one forward -> (cls, probs, logits,
+        saliency fp32 [B,K,H,W] in [0,1], d_input fp32 [B,K,H,W,C] or None) as CUDA tensors.  ``classes`` as in
+        ``predict_explain_classes``.  fp32 engines with ``keep_all_activations``; with ``set_fast_training(True)`` the eligible blocks'
+        input gradients run on the tensor cores (bcad_predict_saliency_classes)."""
+        self.cache_tag = None
+        x = self._as_device_input(x)
+        B, nc = x.shape[0], self.spec.num_classes
+        h, w, c = self.spec.input_shape
+        K, ci = self._class_rows(classes, B)
+        with torch.cuda.device(self.tdev):
+            logits = torch.empty((B, nc), device=self.tdev, dtype=torch.float32)
+            probs = torch.empty((B, nc), device=self.tdev, dtype=torch.float32)
+            cls = torch.empty((B,), device=self.tdev, dtype=torch.int32)
+            sal = torch.empty((B, K, h, w), device=self.tdev, dtype=torch.float32)
+            d_in = torch.empty((B, K, h, w, c), device=self.tdev, dtype=torch.float32) if want_d_input else None
+            if ci is not None:
+                ci = ci.to(self.tdev).contiguous()
+            _lib.check(self.lib.bcad_predict_saliency_classes(self._h, _ptr(x), B, K, _ptr(ci), _lib.GRAD_MODE[grad_mode], _ptr(logits),
+                                                              _ptr(probs), _ptr(cls), _ptr(sal), _ptr(d_in), self._stream()))
+        return cls, probs, logits, sal, d_in
+
+    def _class_rows(self, classes, B):
+        """classes of the multi-class calls -> (K, int32 [B,K] tensor or None = column k is class k)."""
+        nc = self.spec.num_classes
+        if classes is None:
+            K, ci = nc, None
+        else:
+            ci = torch.as_tensor(classes, dtype=torch.int32)
+            if ci.dim() == 1:
+                ci = ci[None].expand(B, -1)
+            if ci.dim() != 2 or ci.shape[0] != B:
+                raise ValueError(f"classes must be a length-K sequence or a [{B},K] array, got shape {tuple(ci.shape)}")
+            K = ci.shape[1]
+            if K >= 1 and (int(ci.min()) < 0 or int(ci.max()) >= nc):
+                raise ValueError("classes out of range")
+        if not 1 <= K <= _lib.MAX_EXPLAIN_CLASSES:
+            raise ValueError(f"{K} target classes per image; 1..{_lib.MAX_EXPLAIN_CLASSES} are supported")
+        return K, ci
 
     def _class_idx(self, class_idx, B):
         if class_idx is None:
@@ -558,6 +586,29 @@ def overlay(img01: torch.Tensor, cam: torch.Tensor, want_overlay=True, want_heat
         _lib.check(lib.bcad_overlay(_ptr(img01), _ptr(cam), B, H, W, _ptr(ov), _ptr(hu),
                                     C.c_void_p(torch.cuda.current_stream(cam.device).cuda_stream)))
     return ov, hu
+
+
+def saliency_overlay(base_u8, saliency: torch.Tensor):
+    """generate_saliency_overlay's colouring (explainability.py:74-77) for [B,K] maps on the GPU: ``base_u8`` uint8 [B,H,W], [B,H,W,1]
+    (grey, replicated) or [B,H,W,3] (BGR), shared by an image's K maps; ``saliency`` fp32 [B,K,H,W] in [0,1]
+    -> (overlay u8 [B,K,H,W,3], heat-map u8 [B,K,H,W,3]), both BGR as cv2 returns them."""
+    lib = _lib.load()
+    sal = saliency.to(torch.float32).contiguous()
+    if sal.dim() != 4:
+        raise ValueError(f"saliency must be [B,K,H,W], got shape {tuple(sal.shape)}")
+    B, K, H, W = sal.shape
+    base = torch.as_tensor(base_u8).to(device=sal.device)
+    if base.dim() == 3:
+        base = base[..., None]
+    if base.dtype != torch.uint8 or base.dim() != 4 or tuple(base.shape[:3]) != (B, H, W) or base.shape[3] not in (1, 3):
+        raise ValueError(f"base_u8 must be uint8 [{B},{H},{W}] or [{B},{H},{W},1|3], got {base.dtype} {tuple(base.shape)}")
+    base = base.contiguous()
+    ov = torch.empty((B, K, H, W, 3), device=sal.device, dtype=torch.uint8)
+    heat = torch.empty((B, K, H, W, 3), device=sal.device, dtype=torch.uint8)
+    with torch.cuda.device(sal.device):
+        _lib.check(lib.bcad_saliency_overlay(_ptr(base), int(base.shape[3]), _ptr(sal), B, K, H, W, _ptr(ov), _ptr(heat),
+                                             C.c_void_p(torch.cuda.current_stream(sal.device).cuda_stream)))
+    return ov, heat
 
 
 # --------------------------------------------------------------------------------------------------

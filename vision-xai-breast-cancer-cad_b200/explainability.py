@@ -96,3 +96,21 @@ def generate_dual_class_overlays(model, img, classes_to_test=[0, 1], save_folder
         overlays[class_idx] = (overlay, heatmap)
         print(f"Saved overlay and heatmap for class {class_idx} in {save_folder}")
     return overlays
+
+
+def generate_dual_class_overlays_batch(model, X, classes_to_test=[0, 1]):
+    """``generate_dual_class_overlays`` for a batch, without the PNGs: one forward per chunk of images, one backward per class, the
+    colouring on the GPU.  ``X``: (B,H,W,C) or (H,W,C) model inputs; the blend base is ``X.astype(np.uint8)`` with 1-channel (or
+    other non-3-channel) inputs replicated from channel 0, as the single-image mirror builds ``vis``.  Runs on
+    ``model.saliency_engine``.  -> (classes int64 [B], probs [B,nc], saliency float32 [B,K,H,W], overlays uint8 [B,K,H,W,3],
+    heatmaps uint8 [B,K,H,W,3]); overlays and heat-maps are BGR, as cv2 returns them."""
+    X = np.asarray(X)
+    if X.ndim == 3:
+        X = X[None]
+    base = X.astype(np.uint8)
+    if base.shape[-1] != 3:
+        base = base[..., :1]
+    eng = model.saliency_engine
+    cls, probs, _, sal, _ = eng.predict_saliency_classes(X.astype(np.float32), list(classes_to_test), "softmax_ce")
+    overlay, heat = _engine.saliency_overlay(torch.from_numpy(np.ascontiguousarray(base)), sal)
+    return (cls.cpu().numpy().astype(np.int64), probs.cpu().numpy(), sal.cpu().numpy(), overlay.cpu().numpy(), heat.cpu().numpy())
