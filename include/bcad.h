@@ -210,6 +210,19 @@ BCAD_API int bcad_gradcam_overlays_host(bcad_model* m, const uint8_t* gray_u8_ho
                                int grad_mode, int standardise, float* logits_host, float* probs_host, int32_t* cls_host,
                                uint8_t* overlay_rgb_host, uint8_t* heat_u8_host);
 
+/* The deployed dual-class call (app.py:649-657 -> GRADCAM.py:31-81) for a BATCH of 8-bit grey images of ANY size, end to end:
+ * gray_u8_host uint8 [B][img_h][img_w] -> CNN input = standardise(cv2.resize(u8 / 255, model size, INTER_LINEAR)) (bcad_gray_resize_preprocess)
+ * -> one forward and K Grad-CAM maps per image scaled to img_h x img_w (bcad_predict_explain_classes) -> per map show_cam_on_image on
+ * img01 = u8 / 255 and heatmap_uint8 (bcad_overlay_classes).  classes_host_or_null int32 [B][K] or NULL (column k = class k, K <=
+ * num_classes); 1 <= K <= BCAD_MAX_EXPLAIN_CLASSES.  overlay_rgb_host uint8 [B][K][img_h][img_w][3] and heat_u8_host uint8
+ * [B][K][img_h][img_w]; one of the two may be NULL.  logits / probs / cls host (each may be NULL).  The chunked three-stream pipeline
+ * of bcad_gradcam_overlays_host; its staging (both slots' images and K maps of the image size) is held under 512 MB of device memory
+ * by shrinking the chunk.  Pinned host arrays make the copies asynchronous.  At the model's input size, map k is byte for byte what
+ * bcad_gradcam_overlays_host returns for class column k. */
+BCAD_API int bcad_gradcam_overlays_classes_host(bcad_model* m, const uint8_t* gray_u8_host, int B, int img_h, int img_w, int K,
+                                                const int32_t* classes_host_or_null, int grad_mode, int standardise, float* logits_host,
+                                                float* probs_host, int32_t* cls_host, uint8_t* overlay_rgb_host, uint8_t* heat_u8_host);
+
 /* ---- stand-alone Grad-CAM tail (pytorch_grad_cam BaseCAM.forward / scale_cam_image) ------------ */
 /* A, dA: [B,h,w,K] NHWC device, dtype 0 = fp32, 1 = bf16; out: fp32 [B,H,W].
  * alpha_k = mean_hw dA_k ; cam = ReLU(sum_k alpha_k A_k) ; min-max ; bilinear (cv2.resize) ; min-max. */
@@ -227,6 +240,18 @@ BCAD_API int bcad_gray_preprocess(const uint8_t* gray_u8_dev, int B, int H, int 
  * (NULL to skip); heat_u8_dev: u8 [B,H,W] (NULL to skip). */
 BCAD_API int bcad_overlay(const float* img01_dev, const float* cam_dev, int B, int H, int W,
                  uint8_t* overlay_rgb_dev, uint8_t* heat_u8_dev, void* stream);
+
+/* ---- the two stages of bcad_gradcam_overlays_classes_host, DEVICE buffers ---------------------------------------------------- */
+/* gray_u8_dev uint8 [B][img_h][img_w] -> x_dev fp32 [B][H][W][C] = cv2.resize(u8 / 255.0f, (W, H), INTER_LINEAR) (one-channel
+ * arithmetic of bcad_bottleneck_resize: bit-identical to it), standardise = 1: (v - mean) / (std + 1e-8) with mean / std of the
+ * resized image in float64, 0: v; replicated C times.  At img_h x img_w == H x W exactly the x of bcad_gray_preprocess. */
+BCAD_API int bcad_gray_resize_preprocess(const uint8_t* gray_u8_dev, int B, int img_h, int img_w, int H, int W, int C, int standardise,
+                                         float* x_dev, void* stream);
+/* bcad_overlay for K maps per image on img01 = u8 / 255: gray_u8_dev uint8 [B][H][W] (read once for all K maps), cam_dev fp32
+ * [B][K][H][W] -> overlay_rgb_dev uint8 [B][K][H][W][3], heat_u8_dev uint8 [B][K][H][W] (one may be NULL); 1 <= K <=
+ * BCAD_MAX_EXPLAIN_CLASSES.  Map k is byte for byte bcad_overlay(u8 / 255, cam[:, k]). */
+BCAD_API int bcad_overlay_classes(const uint8_t* gray_u8_dev, const float* cam_dev, int B, int K, int H, int W, uint8_t* overlay_rgb_dev,
+                                  uint8_t* heat_u8_dev, void* stream);
 
 /* ---- tiny U-Net encoder front (SURVEY 8 row f1): conv2d + relu + max_pool of Classes/unet.py:13-73 ------- */
 /* y = LeakyReLU_alpha(conv(x, kernel) + bias), NHWC fp32, kernel DEVICE fp32 (k,k,Cin,Cout) as unet.py holds it, bias

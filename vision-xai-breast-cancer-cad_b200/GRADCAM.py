@@ -86,27 +86,20 @@ def generate_gradcam_overlays_batch(imgs_u8, class_idx=None, model=None, standar
     return cls.astype(np.int64), probs, ov, hu
 
 
-def generate_dual_class_gradcam_overlays_batch(imgs_u8, classes_to_test=[0, 1], model=None, standardise=True):
-    """The batched form of the deployed dual-class call (app.py:649-657 -> GRADCAM.py:31-81): 8-bit grey images [B,H,W] at the
-    model's input size, ONE forward per image for all of ``classes_to_test`` (K <= 8), everything on the device, no PNGs.
-    -> (classes int64 [B], probs [B,nc], overlays uint8 [B,K,H,W,3], heatmaps uint8 [B,K,H,W]); ``[:, k]`` is byte for byte what
-    ``generate_gradcam_overlays_batch(imgs_u8, class_idx=classes_to_test[k])`` returns."""
+def generate_dual_class_gradcam_overlays_batch(imgs_u8, classes_to_test=[0, 1], model=None, standardise=True, overlay_out=None,
+                                               heat_out=None):
+    """The batched form of the deployed dual-class call (app.py:649-657 -> GRADCAM.py:31-81): 8-bit grey images [B,H,W] of any size
+    (the CNN sees ``cv2.resize(img / 255, model size)``, the maps have the image's size, as in the single-image call above), ONE
+    forward per image for all of ``classes_to_test`` (K <= 8), through ONE host-buffer C-ABI call (bcad_gradcam_overlays_classes_host),
+    no PNGs.  ``overlay_out`` / ``heat_out``: optional C-contiguous uint8 arrays to write into (pinned ones make the copies asynchronous).
+    -> (classes int64 [B], probs [B,nc], overlays uint8 [B,K,H,W,3], heatmaps uint8 [B,K,H,W]); at the model's input size ``[:, k]`` is
+    byte for byte what ``generate_gradcam_overlays_batch(imgs_u8, class_idx=classes_to_test[k])`` returns."""
     mdl = model if model is not None else globals()["model"]
     if mdl is None:
         raise RuntimeError("GRADCAM.model is not set: assign a CNNModel (bcad_b200.CNNModel / ADCNNM) first")
     eng = getattr(mdl, "fast_engine", None) or mdl.engine
-    g = np.ascontiguousarray(imgs_u8)
+    g = np.asarray(imgs_u8)
     if g.dtype != np.uint8:
         raise ValueError("imgs_u8 must be uint8 (0-255 grey levels)")
-    if g.ndim == 2:
-        g = g[None]
-    h, w, c = eng.spec.input_shape
-    if g.shape[1:] != (h, w):
-        raise ValueError(f"image shape {g.shape} does not match [B,{h},{w}]")
-    B, K = g.shape[0], len(classes_to_test)
-    img01, x = _engine.gray_preprocess(torch.from_numpy(g).to(eng.tdev), c, standardise)
-    cls, probs, _, heat = eng.predict_explain_classes(x, list(classes_to_test), "logit")
-    img_k = img01[:, None].expand(B, K, h, w).reshape(B * K, h, w)
-    ov, hu = _engine.overlay(img_k, heat.reshape(B * K, h, w))
-    return (cls.cpu().numpy().astype(np.int64), probs.cpu().numpy(), ov.reshape(B, K, h, w, 3).cpu().numpy(),
-            hu.reshape(B, K, h, w).cpu().numpy())
+    cls, probs, _, ov, hu = eng.gradcam_overlays_classes_host(g, list(classes_to_test), "logit", standardise, overlay_out, heat_out)
+    return cls.astype(np.int64), probs, ov, hu

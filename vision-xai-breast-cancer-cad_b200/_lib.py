@@ -57,6 +57,10 @@ _SIGNATURES = {
     "bcad_predict_explain_sized": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, _P, _P, C.c_int, C.c_int, _P, _P]),
     "bcad_predict_explain_classes": (C.c_int, [_P, _P, C.c_int, C.c_int, _P, C.c_int, _P, _P, _P, C.c_int, C.c_int, _P, _P]),
     "bcad_gradcam_overlays_host": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, _P, _P, _P, _P, _P]),
+    "bcad_gradcam_overlays_classes_host": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, C.c_int, C.c_int, _P, _P, _P,
+                                                     _P, _P]),
+    "bcad_gray_resize_preprocess": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P]),
+    "bcad_overlay_classes": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P]),
     "bcad_explain_backward": (C.c_int, [_P, C.c_int, _P, C.c_int, C.POINTER(_P), _P, _P]),
     "bcad_predict_saliency_classes": (C.c_int, [_P, _P, C.c_int, C.c_int, _P, C.c_int, _P, _P, _P, _P, _P, _P]),
     "bcad_saliency_overlay": (C.c_int, [_P, C.c_int, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P]),

@@ -4,6 +4,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <mutex>
 #include <new>
 #include <vector>
@@ -920,6 +921,49 @@ int bcad_get_tensor(bcad_model* mm, int kind, int index, int B, float* dst, void
 // -----------------------------------------------------------------------------------------------------
 // host-buffer end-to-end call: H2D / compute / D2H in chunks on three streams, double-buffered
 // -----------------------------------------------------------------------------------------------------
+// streams, events and the model-size slot buffers of the pipeline, on first use (caller holds m->mu)
+static int xfer_init(Model* m) {
+    Xfer& X = m->xfer;
+    if (X.inited) return BCAD_OK;
+    const size_t img = (size_t)m->cfg.in_h * m->cfg.in_w * m->cfg.in_c, hm = (size_t)m->cfg.in_h * m->cfg.in_w;
+    int chunk = std::min(m->cfg.max_batch, 128);
+    if (const char* e = getenv("BCAD_HOST_CHUNK")) chunk = std::max(1, std::min(m->cfg.max_batch, atoi(e)));
+    BCAD_CUDA_CHECK(cudaStreamCreateWithFlags(&X.s_in, cudaStreamNonBlocking));
+    BCAD_CUDA_CHECK(cudaStreamCreateWithFlags(&X.s_compute, cudaStreamNonBlocking));
+    BCAD_CUDA_CHECK(cudaStreamCreateWithFlags(&X.s_out, cudaStreamNonBlocking));
+    for (int i = 0; i < 2; ++i) {
+        BCAD_CUDA_CHECK(cudaEventCreateWithFlags(&X.in_done[i], cudaEventDisableTiming));
+        BCAD_CUDA_CHECK(cudaEventCreateWithFlags(&X.compute_done[i], cudaEventDisableTiming));
+        BCAD_CUDA_CHECK(cudaEventCreateWithFlags(&X.out_done[i], cudaEventDisableTiming));
+        BCAD_TRY(m->alloc((void**)&X.x[i], (size_t)chunk * img * sizeof(float)));
+        BCAD_TRY(m->alloc((void**)&X.heat[i], (size_t)chunk * hm * sizeof(float)));
+        BCAD_TRY(m->alloc((void**)&X.cidx[i], (size_t)chunk * sizeof(int32_t)));
+    }
+    X.chunk = chunk;
+    X.inited = true;
+    return BCAD_OK;
+}
+
+// small outputs (logits, probabilities, classes) go through pinned staging sized for the whole call (caller holds m->host_mu)
+static int stage_small(Model* m, size_t bytes) {
+    Xfer& X = m->xfer;
+    if (X.h_small_bytes < bytes) {
+        if (X.h_small) cudaFreeHost(X.h_small);
+        X.h_small = nullptr;
+        X.h_small_bytes = 0;
+        BCAD_CUDA_CHECK(cudaMallocHost(&X.h_small, bytes));
+        X.h_small_bytes = bytes;
+    }
+    if (X.d_small_bytes < bytes) {
+        std::lock_guard<std::mutex> lock(m->mu);             // grows only when a call is larger than every call before it; the handle
+        X.d_small = nullptr;                                 // owns (and frees at destroy) the smaller ones it replaces: tens of bytes per image
+        X.d_small_bytes = 0;
+        BCAD_TRY(m->alloc(&X.d_small, bytes));
+        X.d_small_bytes = bytes;
+    }
+    return BCAD_OK;
+}
+
 static int predict_explain_host_impl(bcad_model* mm, const float* x_host, const uint8_t* x8_host, int B, const int32_t* class_idx_host,
                                      int grad_mode, float* logits_host, float* probs_host, int32_t* cls_host, float* heat_host,
                                      uint8_t* heat_u8_host, const uint8_t* gray8_host = nullptr, int standardise = 0,
@@ -944,25 +988,9 @@ static int predict_explain_host_impl(bcad_model* mm, const float* x_host, const 
     // end-to-end bound), large enough to keep the kernels efficient.  BCAD_HOST_CHUNK overrides (tuning).
     // Buffers are sized for 128 images; a call uses about a quarter of its batch per chunk (32..128 images: measured at 512
     // images, float32 in/out 3.6-3.7 ms with 64, 3.7-3.8 with 128; 8-bit in/out 2.11 ms with 64, 1.73 ms with 128, 1.80 ms with 256).
-    int chunk = std::min(m->cfg.max_batch, 128);
-    if (const char* e = getenv("BCAD_HOST_CHUNK")) chunk = std::max(1, std::min(m->cfg.max_batch, atoi(e)));
     {
         std::lock_guard<std::mutex> lock(m->mu);
-        if (!X.inited) {
-            BCAD_CUDA_CHECK(cudaStreamCreateWithFlags(&X.s_in, cudaStreamNonBlocking));
-            BCAD_CUDA_CHECK(cudaStreamCreateWithFlags(&X.s_compute, cudaStreamNonBlocking));
-            BCAD_CUDA_CHECK(cudaStreamCreateWithFlags(&X.s_out, cudaStreamNonBlocking));
-            for (int i = 0; i < 2; ++i) {
-                BCAD_CUDA_CHECK(cudaEventCreateWithFlags(&X.in_done[i], cudaEventDisableTiming));
-                BCAD_CUDA_CHECK(cudaEventCreateWithFlags(&X.compute_done[i], cudaEventDisableTiming));
-                BCAD_CUDA_CHECK(cudaEventCreateWithFlags(&X.out_done[i], cudaEventDisableTiming));
-                BCAD_TRY(m->alloc((void**)&X.x[i], (size_t)chunk * img * sizeof(float)));
-                BCAD_TRY(m->alloc((void**)&X.heat[i], (size_t)chunk * hm * sizeof(float)));
-                BCAD_TRY(m->alloc((void**)&X.cidx[i], (size_t)chunk * sizeof(int32_t)));
-            }
-            X.chunk = chunk;
-            X.inited = true;
-        }
+        BCAD_TRY(xfer_init(m));
         if (heat_u8_host != nullptr && X.heat8[0] == nullptr)
             for (int i = 0; i < 2; ++i) BCAD_TRY(m->alloc((void**)&X.heat8[i], (size_t)X.chunk * hm));
         if ((x8_host != nullptr || gray8_host != nullptr) && X.x8[0] == nullptr)
@@ -973,22 +1001,8 @@ static int predict_explain_host_impl(bcad_model* mm, const float* x_host, const 
                 BCAD_TRY(m->alloc((void**)&X.ov8[i], (size_t)X.chunk * hm * 3));
             }
     }
-    // small outputs go through pinned staging sized for the whole call
     const size_t per_img = (size_t)(2 * nc) * sizeof(float) + sizeof(int32_t);
-    if (X.h_small_bytes < per_img * B) {
-        if (X.h_small) cudaFreeHost(X.h_small);
-        X.h_small = nullptr;
-        X.h_small_bytes = 0;
-        BCAD_CUDA_CHECK(cudaMallocHost(&X.h_small, per_img * B));
-        X.h_small_bytes = per_img * B;
-    }
-    if (X.d_small_bytes < per_img * B) {
-        std::lock_guard<std::mutex> lock(m->mu);             // grows only when a call is larger than every call before it; the handle
-        X.d_small = nullptr;                                 // owns (and frees at destroy) the smaller ones it replaces: tens of bytes per image
-        X.d_small_bytes = 0;
-        BCAD_TRY(m->alloc(&X.d_small, per_img * B));
-        X.d_small_bytes = per_img * B;
-    }
+    BCAD_TRY(stage_small(m, per_img * B));
     float* st_logits = reinterpret_cast<float*>(X.h_small);
     float* st_probs = st_logits + (size_t)B * nc;
     int32_t* st_cls = reinterpret_cast<int32_t*>(st_probs + (size_t)B * nc);
@@ -1106,6 +1120,113 @@ int bcad_gradcam_overlays_host(bcad_model* mm, const uint8_t* gray_u8_host, int 
                                      heat_u8_host, gray_u8_host, standardise, overlay_rgb_host);
 }
 
+// Staging bound of bcad_gradcam_overlays_classes_host: both slots' 8-bit images, classes and K float / RGB / u8 maps of the image size
+// stay within this many bytes of the handle's memory (the chunk shrinks to fit; a single image larger than half of it still runs, one
+// image per chunk).  512 x 512 images with K = 2: 4.25 MB per image and slot, chunks of up to 60 images.
+static const size_t kClassesStagingBytes = (size_t)512 << 20;
+
+static size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
+
+int bcad_gradcam_overlays_classes_host(bcad_model* mm, const uint8_t* gray_u8_host, int B, int img_h, int img_w, int K,
+                                       const int32_t* classes_host_or_null, int grad_mode, int standardise, float* logits_host,
+                                       float* probs_host, int32_t* cls_host, uint8_t* overlay_rgb_host, uint8_t* heat_u8_host) {
+    Model* m = reinterpret_cast<Model*>(mm);
+    BCAD_REQUIRE(m && gray_u8_host, "gradcam_overlays_classes_host: null model or image pointer");
+    BCAD_REQUIRE(overlay_rgb_host || heat_u8_host, "gradcam_overlays_classes_host: overlay and heat-map pointers are both null");
+    BCAD_REQUIRE(B >= 1, "batch must be >= 1, got %d", B);
+    BCAD_REQUIRE(img_h >= 1 && img_w >= 1 && img_h <= 16384 && img_w <= 16384, "gradcam_overlays_classes_host: bad image size %dx%d", img_h, img_w);
+    BCAD_REQUIRE(K >= 1 && K <= BCAD_MAX_EXPLAIN_CLASSES, "gradcam_overlays_classes_host: K=%d out of range 1..%d", K, BCAD_MAX_EXPLAIN_CLASSES);
+    BCAD_REQUIRE(standardise == 0 || standardise == 1, "gradcam_overlays_classes_host: standardise must be 0 or 1");
+    BCAD_REQUIRE(grad_mode == BCAD_GRAD_LOGIT || grad_mode == BCAD_GRAD_SOFTMAX_CE, "bad grad_mode %d", grad_mode);
+    const int nc = m->cfg.num_classes;
+    BCAD_REQUIRE(classes_host_or_null || K <= nc, "gradcam_overlays_classes_host: classes=NULL explains classes 0..K-1, but K=%d > num_classes=%d", K, nc);
+    if (classes_host_or_null != nullptr)
+        for (size_t i = 0; i < (size_t)B * K; ++i)
+            BCAD_REQUIRE(classes_host_or_null[i] >= 0 && classes_host_or_null[i] < nc, "classes[%zu][%zu] = %d is outside [0, %d)", i / K, i % K,
+                         classes_host_or_null[i], nc);
+    if (!m->committed) { set_error("weights not committed: call bcad_commit first"); return BCAD_ERR_STATE; }
+    DeviceGuard g(m->cfg.device);
+    std::lock_guard<std::mutex> host_lock(m->host_mu);
+    Xfer& X = m->xfer;
+    const size_t hw = (size_t)img_h * img_w;
+    // per image and slot: 8-bit image, class row, float maps, RGB overlays, u8 heat-maps
+    const size_t b_img = align256(hw), b_cls = align256((size_t)K * sizeof(int32_t)), b_heat = align256((size_t)K * hw * sizeof(float));
+    const size_t b_ov = overlay_rgb_host ? align256((size_t)K * hw * 3) : 0, b_h8 = heat_u8_host ? align256((size_t)K * hw) : 0;
+    const size_t per_img_slot = b_img + b_cls + b_heat + b_ov + b_h8;
+    int C0;
+    {
+        std::lock_guard<std::mutex> lock(m->mu);
+        BCAD_TRY(xfer_init(m));
+        // the chunk of bcad_gradcam_overlays_host (a quarter of the batch, 32..128 images), shrunk to the staging bound
+        C0 = std::min(std::min(X.chunk, 128), std::max(32, ((B + 3) / 4 + 31) / 32 * 32));
+        if (const char* e = getenv("BCAD_HOST_CHUNK")) C0 = std::max(1, std::min(X.chunk, atoi(e)));
+        C0 = (int)std::max<size_t>(1, std::min<size_t>((size_t)C0, kClassesStagingBytes / (2 * per_img_slot)));
+        const size_t need = 2 * (size_t)C0 * per_img_slot;
+        if (X.cls_arena_bytes < need) {
+            if (X.cls_arena != nullptr) {                     // replaced, not kept until destroy: it can be hundreds of MB
+                BCAD_CUDA_CHECK(cudaFree(X.cls_arena));       // (synchronises the device: no earlier call still reads it)
+                m->allocs.erase(std::find(m->allocs.begin(), m->allocs.end(), X.cls_arena));
+                m->ws_bytes -= X.cls_arena_bytes;
+                X.cls_arena = nullptr;
+                X.cls_arena_bytes = 0;
+            }
+            BCAD_TRY(m->alloc(&X.cls_arena, need));
+            X.cls_arena_bytes = need;
+        }
+    }
+    uint8_t *d_img[2], *d_ov[2], *d_h8[2];
+    int32_t* d_cls[2];
+    float* d_heat[2];
+    for (int i = 0; i < 2; ++i) {
+        uint8_t* p = reinterpret_cast<uint8_t*>(X.cls_arena) + (size_t)i * C0 * per_img_slot;
+        d_img[i] = p;                                         p += (size_t)C0 * b_img;
+        d_cls[i] = reinterpret_cast<int32_t*>(p);             p += (size_t)C0 * b_cls;
+        d_heat[i] = reinterpret_cast<float*>(p);              p += (size_t)C0 * b_heat;
+        d_ov[i] = overlay_rgb_host ? p : nullptr;             p += (size_t)C0 * b_ov;
+        d_h8[i] = heat_u8_host ? p : nullptr;
+    }
+    const size_t per_img = (size_t)(2 * nc) * sizeof(float) + sizeof(int32_t);
+    BCAD_TRY(stage_small(m, per_img * B));
+    float* st_logits = reinterpret_cast<float*>(X.h_small);
+    float* st_probs = st_logits + (size_t)B * nc;
+    int32_t* st_cls = reinterpret_cast<int32_t*>(st_probs + (size_t)B * nc);
+    float* dv_logits = reinterpret_cast<float*>(X.d_small);
+    float* dv_probs = dv_logits + (size_t)B * nc;
+    int32_t* dv_cls = reinterpret_cast<int32_t*>(dv_probs + (size_t)B * nc);
+    const int nchunks = (B + C0 - 1) / C0;
+    for (int c = 0, b0 = 0; c < nchunks; ++c, b0 += C0) {
+        const int slot = c & 1, n = std::min(C0, B - b0);
+        if (c >= 2) {                                         // slot reuse, as in predict_explain_host_impl
+            BCAD_CUDA_CHECK(cudaStreamWaitEvent(X.s_in, X.compute_done[slot], 0));
+            BCAD_CUDA_CHECK(cudaStreamWaitEvent(X.s_compute, X.out_done[slot], 0));
+        }
+        BCAD_CUDA_CHECK(cudaMemcpyAsync(d_img[slot], gray_u8_host + (size_t)b0 * hw, (size_t)n * hw, cudaMemcpyHostToDevice, X.s_in));
+        if (classes_host_or_null)
+            BCAD_CUDA_CHECK(cudaMemcpyAsync(d_cls[slot], classes_host_or_null + (size_t)b0 * K, (size_t)n * K * sizeof(int32_t), cudaMemcpyHostToDevice, X.s_in));
+        BCAD_CUDA_CHECK(cudaEventRecord(X.in_done[slot], X.s_in));
+        BCAD_CUDA_CHECK(cudaStreamWaitEvent(X.s_compute, X.in_done[slot], 0));
+        int rc = launch_gray_resize_preprocess(d_img[slot], X.x[slot], n, img_h, img_w, m->cfg.in_h, m->cfg.in_w, m->cfg.in_c, standardise, X.s_compute);
+        if (rc == BCAD_OK)
+            rc = run(m, X.x[slot], n, classes_host_or_null ? d_cls[slot] : nullptr, grad_mode, true, dv_logits + (size_t)b0 * nc,
+                     dv_probs + (size_t)b0 * nc, dv_cls + b0, d_heat[slot], X.s_compute, img_h, img_w, K);
+        if (rc == BCAD_OK) rc = launch_overlay_classes(d_img[slot], d_heat[slot], n, K, (int)hw, d_ov[slot], d_h8[slot], X.s_compute);
+        if (rc != BCAD_OK) { cudaDeviceSynchronize(); return rc; }
+        BCAD_CUDA_CHECK(cudaEventRecord(X.compute_done[slot], X.s_compute));
+        BCAD_CUDA_CHECK(cudaStreamWaitEvent(X.s_out, X.compute_done[slot], 0));
+        const size_t maps = (size_t)b0 * K * hw, nmaps = (size_t)n * K * hw;
+        if (overlay_rgb_host) BCAD_CUDA_CHECK(cudaMemcpyAsync(overlay_rgb_host + maps * 3, d_ov[slot], nmaps * 3, cudaMemcpyDeviceToHost, X.s_out));
+        if (heat_u8_host) BCAD_CUDA_CHECK(cudaMemcpyAsync(heat_u8_host + maps, d_h8[slot], nmaps, cudaMemcpyDeviceToHost, X.s_out));
+        if (c + 1 == nchunks) BCAD_CUDA_CHECK(cudaMemcpyAsync(X.h_small, X.d_small, per_img * B, cudaMemcpyDeviceToHost, X.s_out));
+        BCAD_CUDA_CHECK(cudaEventRecord(X.out_done[slot], X.s_out));
+    }
+    BCAD_CUDA_CHECK(cudaStreamSynchronize(X.s_out));
+    BCAD_CUDA_CHECK(cudaStreamSynchronize(X.s_compute));
+    if (logits_host) memcpy(logits_host, st_logits, (size_t)B * nc * sizeof(float));
+    if (probs_host) memcpy(probs_host, st_probs, (size_t)B * nc * sizeof(float));
+    if (cls_host) memcpy(cls_host, st_cls, (size_t)B * sizeof(int32_t));
+    return BCAD_OK;
+}
+
 // -----------------------------------------------------------------------------------------------------
 // stand-alone tail and overlay
 // -----------------------------------------------------------------------------------------------------
@@ -1141,6 +1262,24 @@ int bcad_overlay(const float* img01, const float* cam, int B, int H, int W, uint
     BCAD_REQUIRE(img01 && cam, "overlay: null argument");
     BCAD_REQUIRE(B >= 1 && H >= 1 && W >= 1, "overlay: bad sizes");
     return launch_overlay(img01, cam, B, H, W, overlay_rgb, heat_u8, (cudaStream_t)stream);
+}
+
+int bcad_gray_resize_preprocess(const uint8_t* gray_u8, int B, int img_h, int img_w, int H, int W, int C, int standardise, float* x,
+                                void* stream) {
+    BCAD_REQUIRE(gray_u8 && x, "gray_resize_preprocess: null argument");
+    BCAD_REQUIRE(B >= 1 && img_h >= 1 && img_w >= 1 && H >= 1 && W >= 1 && C >= 1 && (int64_t)img_h * img_w <= 0x7fffffff &&
+                     (int64_t)H * W <= 0x7fffffff, "gray_resize_preprocess: bad sizes B=%d %dx%d -> %dx%dx%d", B, img_h, img_w, H, W, C);
+    BCAD_REQUIRE(standardise == 0 || standardise == 1, "gray_resize_preprocess: standardise must be 0 or 1");
+    return launch_gray_resize_preprocess(gray_u8, x, B, img_h, img_w, H, W, C, standardise, (cudaStream_t)stream);
+}
+
+int bcad_overlay_classes(const uint8_t* gray_u8, const float* cam, int B, int K, int H, int W, uint8_t* overlay_rgb, uint8_t* heat_u8,
+                         void* stream) {
+    BCAD_REQUIRE(gray_u8 && cam, "overlay_classes: null image or cam");
+    BCAD_REQUIRE(overlay_rgb || heat_u8, "overlay_classes: overlay and heat-map pointers are both null");
+    BCAD_REQUIRE(K >= 1 && K <= BCAD_MAX_EXPLAIN_CLASSES, "overlay_classes: K=%d out of range 1..%d", K, BCAD_MAX_EXPLAIN_CLASSES);
+    BCAD_REQUIRE(B >= 1 && H >= 1 && W >= 1 && (int64_t)H * W <= 0x7fffffff, "overlay_classes: bad sizes B=%d %dx%d", B, H, W);
+    return launch_overlay_classes(gray_u8, cam, B, K, H * W, overlay_rgb, heat_u8, (cudaStream_t)stream);
 }
 
 // -----------------------------------------------------------------------------------------------------

@@ -84,6 +84,13 @@ int launch_heat_to_u8(const float* cam, uint8_t* out, size_t n, cudaStream_t s);
 int launch_u8_to_unit(const uint8_t* src, float* dst, size_t n, cudaStream_t s);
 // GRADCAM.py:46 + the CNN-input normalisation of app.py:179-182: img01 = u8 / 255; x[.., c] = standardise ? (img01 - mean) / (std + 1e-8) : img01
 int launch_gray_preprocess(const uint8_t* g8, float* img01, float* x, int B, int npix, int C, int standardise, cudaStream_t s);
+// u8 grey [B][hi][wi] -> x [B][H][W][C] = standardise(cv2.resize(u8 / 255.0f, (W, H), INTER_LINEAR)) (mean / std of the resized image
+// in float64), the channel replicated to C; at hi x wi == H x W exactly launch_gray_preprocess (without img01)
+int launch_gray_resize_preprocess(const uint8_t* g8, float* x, int B, int hi, int wi, int H, int W, int C, int standardise, cudaStream_t s);
+// launch_overlay for K maps per image on img01 = u8 / 255: g8 u8 [B][npix], cam fp32 [B][K][npix] -> overlay_rgb u8 [B][K][npix][3],
+// heat_u8 [B][K][npix] (either may be null); 1 <= K <= BCAD_MAX_EXPLAIN_CLASSES
+int launch_overlay_classes(const uint8_t* g8, const float* cam, int B, int K, int npix, uint8_t* overlay_rgb, uint8_t* heat_u8,
+                           cudaStream_t s);
 int launch_bottleneck_resize(const float* src, float* dst, int B, int C, int H, int W, int chw, int oh, int ow, cudaStream_t s);
 int launch_leaky_from_z(const float* z, float* h, float alpha, int64_t n, cudaStream_t s);
 int launch_mul_mask(float* h, const float* mask, int B, int units, int ld, cudaStream_t s);

@@ -1085,6 +1085,7 @@ int launch_u8_to_unit(const uint8_t* src, float* dst, size_t n, cudaStream_t s) 
 
 // 8-bit grey image -> img01 = u8 / 255 (GRADCAM.py:46) and the CNN input: per-image standardisation (x - mean) / (std + 1e-8) as the
 // reference prepares its CNN inputs (app.py:179-182), the single channel replicated to C.  mean / std from exact integer sums.
+// img01 may be null (gray_resize_preprocess at the model's size: the overlay reads the 8-bit image itself).
 __global__ void __launch_bounds__(512) gray_preprocess_kernel(const uint8_t* __restrict__ g8, float* __restrict__ img01, float* __restrict__ x,
                                                               int npix, int C, int standardise) {
     __shared__ unsigned long long s_sum[16], s_sq[16];
@@ -1123,14 +1124,14 @@ __global__ void __launch_bounds__(512) gray_preprocess_kernel(const uint8_t* __r
         for (int i = tid; i < npix / 4; i += 512) {           // 4 pixels per thread: one 4-byte load, two 16-byte stores
             const uchar4 q = reinterpret_cast<const uchar4*>(src)[i];
             const float4 v = make_float4((float)q.x / 255.0f, (float)q.y / 255.0f, (float)q.z / 255.0f, (float)q.w / 255.0f);
-            reinterpret_cast<float4*>(ib)[i] = v;
+            if (img01) reinterpret_cast<float4*>(ib)[i] = v;
             reinterpret_cast<float4*>(xb)[i] = standardise ? make_float4((v.x - mean) / den, (v.y - mean) / den, (v.z - mean) / den, (v.w - mean) / den) : v;
         }
         return;
     }
     for (int i = tid; i < npix; i += 512) {
         const float v = (float)src[i] / 255.0f;
-        ib[i] = v;
+        if (img01) ib[i] = v;
         const float xv = standardise ? (v - mean) / den : v;
         for (int c = 0; c < C; ++c) xb[(size_t)i * C + c] = xv;
     }
@@ -1154,6 +1155,180 @@ int launch_saliency_overlay(const uint8_t* base, int base_c, const float* sal, i
     const size_t total = (size_t)B * K * npix;
     const int blocks = (int)std::min((size_t)148 * 16, (total + 255) / 256);
     saliency_overlay_kernel<<<blocks, 256, 0, s>>>(base, base_c, sal, K, (size_t)npix, total, overlay, heat);
+    BCAD_CUDA_CHECK(cudaGetLastError());
+    return BCAD_OK;
+}
+
+// =====================================================================================================
+// The dual-class overlay call for grey images of any size (bcad_gradcam_overlays_classes_host)
+// =====================================================================================================
+// cv2.resize(u8 / 255.0f, (W, H), INTER_LINEAR) of one channel with the <= 4-channel arithmetic of bottleneck_resize_kernel
+// (coordinate in double, weight = float(frac), no FMA contraction): the two kernels agree bit for bit.
+__device__ __forceinline__ void resize_coord_d(int d, int ns, int nd, int& i0, int& i1, float& f) {
+    const double sd = ((double)d + 0.5) * ((double)ns / (double)nd) - 0.5;
+    i0 = (int)floor(sd);
+    f = (float)(sd - (double)i0);
+    if (i0 < 0) { i0 = 0; f = 0.f; }
+    if (i0 >= ns - 1) { i0 = ns - 1; f = 0.f; }
+    i1 = min(i0 + 1, ns - 1);
+}
+
+__device__ __forceinline__ float resize_gray_px(const uint8_t* __restrict__ src, int hi, int wi, int H, int W, int p) {
+    int x0, x1, y0, y1;
+    float fx, fy;
+    resize_coord_d(p % W, wi, W, x0, x1, fx);
+    resize_coord_d(p / W, hi, H, y0, y1, fy);
+    auto at = [&](int y, int x) { return (float)__ldg(src + (size_t)y * wi + x) / 255.0f; };
+    const float gx = __fsub_rn(1.f, fx), gy = __fsub_rn(1.f, fy);
+    const float top = __fadd_rn(__fmul_rn(at(y0, x0), gx), __fmul_rn(at(y0, x1), fx));
+    const float bot = __fadd_rn(__fmul_rn(at(y1, x0), gx), __fmul_rn(at(y1, x1), fx));
+    return __fadd_rn(__fmul_rn(top, gy), __fmul_rn(bot, fy));
+}
+
+// One CTA per image.  Pass 1: resized pixels and their sum / sum of squares in float64, thread-strided then a fixed-order warp and
+// block reduction (deterministic); pass 2 recomputes each pixel (four 8-bit reads) and stores (v - mean) / (std + 1e-8), or v.
+constexpr int GRP_THREADS = 512;
+__global__ void __launch_bounds__(GRP_THREADS) gray_resize_preprocess_kernel(const uint8_t* __restrict__ g8, float* __restrict__ x, int hi,
+                                                                             int wi, int H, int W, int C, int standardise) {
+    __shared__ double s_sum[GRP_THREADS / 32], s_sq[GRP_THREADS / 32];
+    __shared__ float s_mean, s_den;
+    const int b = blockIdx.x, tid = threadIdx.x, npix = H * W;
+    const uint8_t* src = g8 + (size_t)b * hi * wi;
+    if (standardise) {
+        double sum = 0.0, sq = 0.0;
+        for (int p = tid; p < npix; p += GRP_THREADS) {
+            const double v = (double)resize_gray_px(src, hi, wi, H, W, p);
+            sum += v;
+            sq += v * v;
+        }
+        for (int o = 16; o > 0; o >>= 1) { sum += __shfl_xor_sync(0xffffffffu, sum, o); sq += __shfl_xor_sync(0xffffffffu, sq, o); }
+        if ((tid & 31) == 0) { s_sum[tid >> 5] = sum; s_sq[tid >> 5] = sq; }
+        __syncthreads();
+        if (tid == 0) {
+            double ts = 0.0, tq = 0.0;
+            for (int w = 0; w < GRP_THREADS / 32; ++w) { ts += s_sum[w]; tq += s_sq[w]; }
+            const double mean = ts / npix;
+            const double var = tq / npix - mean * mean;
+            s_mean = (float)mean;
+            s_den = (float)sqrt(var > 0.0 ? var : 0.0) + 1e-8f;
+        }
+        __syncthreads();
+    }
+    const float mean = standardise ? s_mean : 0.f, den = standardise ? s_den : 1.f;
+    float* xb = x + (size_t)b * npix * C;
+    for (int p = tid; p < npix; p += GRP_THREADS) {
+        const float v = resize_gray_px(src, hi, wi, H, W, p);
+        const float xv = standardise ? (v - mean) / den : v;
+        for (int c = 0; c < C; ++c) xb[(size_t)p * C + c] = xv;
+    }
+}
+
+int launch_gray_resize_preprocess(const uint8_t* g8, float* x, int B, int hi, int wi, int H, int W, int C, int standardise, cudaStream_t s) {
+    if (hi == H && wi == W) {
+        // the model's own size: exactly gray_preprocess (exact integer sums), without its image-size float copy
+        gray_preprocess_kernel<<<B, 512, 0, s>>>(g8, nullptr, x, H * W, C, standardise);
+    } else {
+        gray_resize_preprocess_kernel<<<B, GRP_THREADS, 0, s>>>(g8, x, hi, wi, H, W, C, standardise);
+    }
+    BCAD_CUDA_CHECK(cudaGetLastError());
+    return BCAD_OK;
+}
+
+// overlay_kernel for the K maps of each grey image, reading the 8-bit image once per pixel for all of them: g = (float)q / 255.0f (the
+// gray_preprocess expression), the same JET table, blend and two passes, so every map is byte for byte overlay_kernel on img01 = u8 / 255.
+// One CTA per image; a thread takes 4 consecutive pixels: a 4-byte image load and a 16-byte cam load per map, 12-byte RGB stores.
+template <int K>
+__global__ void __launch_bounds__(1024)
+overlay_classes_kernel(const uint8_t* __restrict__ g8, const float* __restrict__ cam, int npix, uint8_t* __restrict__ overlay_rgb,
+                       uint8_t* __restrict__ heat_u8) {
+    __shared__ float s_red[64];
+    __shared__ float s_lut[256 * 3];                                       // RGB order, already / 255
+    const int b = blockIdx.x;
+    for (int i = threadIdx.x; i < 768; i += blockDim.x) s_lut[i] = (float)c_jet_bgr[(i / 3) * 3 + (2 - i % 3)] / 255.f;   // BGR -> RGB
+    __syncthreads();
+    const uint8_t* gb = g8 + (size_t)b * npix;
+    const float* cb = cam + (size_t)b * K * npix;                          // map k at cb + k * npix
+    const bool vec = (npix % 4 == 0) && (reinterpret_cast<uintptr_t>(gb) % 4 == 0) && (reinterpret_cast<uintptr_t>(cb) % 16 == 0);
+    const int n4 = vec ? npix / 4 : 0;
+    float vmax[K];
+#pragma unroll
+    for (int k = 0; k < K; ++k) vmax[k] = -3.4e38f;
+    auto blend_max = [&](float& m, float cv, float g) {
+        const int li = (int)(uint8_t)(int)(255.f * cv);                   // np.uint8(255*cam): truncation
+        const float* l = s_lut + li * 3;
+        m = fmaxf(m, fmaxf(fmaxf(0.5f * l[0] + 0.5f * g, 0.5f * l[1] + 0.5f * g), 0.5f * l[2] + 0.5f * g));
+    };
+    for (int i = threadIdx.x; i < n4; i += blockDim.x) {
+        const uchar4 q = reinterpret_cast<const uchar4*>(gb)[i];
+        const float4 g4 = make_float4((float)q.x / 255.0f, (float)q.y / 255.0f, (float)q.z / 255.0f, (float)q.w / 255.0f);
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+            const float4 c4 = __ldg(reinterpret_cast<const float4*>(cb + (size_t)k * npix) + i);
+            blend_max(vmax[k], c4.x, g4.x); blend_max(vmax[k], c4.y, g4.y); blend_max(vmax[k], c4.z, g4.z); blend_max(vmax[k], c4.w, g4.w);
+            if (heat_u8 != nullptr) {
+                uchar4 o;
+                o.x = (uint8_t)(int)(c4.x * 255.f); o.y = (uint8_t)(int)(c4.y * 255.f); o.z = (uint8_t)(int)(c4.z * 255.f); o.w = (uint8_t)(int)(c4.w * 255.f);
+                reinterpret_cast<uchar4*>(heat_u8 + ((size_t)b * K + k) * npix)[i] = o;
+            }
+        }
+    }
+    for (int i = n4 * 4 + threadIdx.x; i < npix; i += blockDim.x) {
+        const float g = (float)gb[i] / 255.0f;
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+            const float cv = cb[(size_t)k * npix + i];
+            blend_max(vmax[k], cv, g);
+            if (heat_u8 != nullptr) heat_u8[((size_t)b * K + k) * npix + i] = (uint8_t)(int)(cv * 255.f);
+        }
+    }
+    if (overlay_rgb == nullptr) return;
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+        float vmin = 0.f;
+        block_minmax(vmin, vmax[k], s_red);
+    }
+    auto rgb = [&](float m, float cv, float g, uint8_t* o) {
+        const int li = (int)(uint8_t)(int)(255.f * cv);
+        const float* l = s_lut + li * 3;
+#pragma unroll
+        for (int ch = 0; ch < 3; ++ch) o[ch] = (uint8_t)(int)(255.f * ((0.5f * l[ch] + 0.5f * g) / m));
+    };
+    uint8_t* ob = overlay_rgb + (size_t)b * K * npix * 3;                  // map k at ob + k * npix * 3
+    const bool vst = vec && (reinterpret_cast<uintptr_t>(ob) % 4 == 0);
+    for (int i = threadIdx.x; i < n4; i += blockDim.x) {
+        const uchar4 q = reinterpret_cast<const uchar4*>(gb)[i];
+        const float4 g4 = make_float4((float)q.x / 255.0f, (float)q.y / 255.0f, (float)q.z / 255.0f, (float)q.w / 255.0f);
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+            const float4 c4 = __ldg(reinterpret_cast<const float4*>(cb + (size_t)k * npix) + i);
+            uint8_t o[12];
+            rgb(vmax[k], c4.x, g4.x, o); rgb(vmax[k], c4.y, g4.y, o + 3); rgb(vmax[k], c4.z, g4.z, o + 6); rgb(vmax[k], c4.w, g4.w, o + 9);
+            uint8_t* d8 = ob + (size_t)k * npix * 3 + (size_t)i * 12;
+            if (vst) {
+                uint32_t* d = reinterpret_cast<uint32_t*>(d8);
+#pragma unroll
+                for (int w = 0; w < 3; ++w) d[w] = (uint32_t)o[4 * w] | ((uint32_t)o[4 * w + 1] << 8) | ((uint32_t)o[4 * w + 2] << 16) | ((uint32_t)o[4 * w + 3] << 24);
+            } else {
+#pragma unroll
+                for (int w = 0; w < 12; ++w) d8[w] = o[w];
+            }
+        }
+    }
+    for (int i = n4 * 4 + threadIdx.x; i < npix; i += blockDim.x) {
+        const float g = (float)gb[i] / 255.0f;
+#pragma unroll
+        for (int k = 0; k < K; ++k) rgb(vmax[k], cb[(size_t)k * npix + i], g, ob + ((size_t)k * npix + i) * 3);
+    }
+}
+
+int launch_overlay_classes(const uint8_t* g8, const float* cam, int B, int K, int npix, uint8_t* overlay_rgb, uint8_t* heat_u8,
+                           cudaStream_t s) {
+    switch (K) {
+#define BCAD_OVC(k) case k: overlay_classes_kernel<k><<<B, 1024, 0, s>>>(g8, cam, npix, overlay_rgb, heat_u8); break;
+        BCAD_OVC(1) BCAD_OVC(2) BCAD_OVC(3) BCAD_OVC(4) BCAD_OVC(5) BCAD_OVC(6) BCAD_OVC(7) BCAD_OVC(8)
+#undef BCAD_OVC
+        default: set_error("overlay_classes: K=%d out of range 1..%d", K, BCAD_MAX_EXPLAIN_CLASSES); return BCAD_ERR_INVALID;
+    }
     BCAD_CUDA_CHECK(cudaGetLastError());
     return BCAD_OK;
 }

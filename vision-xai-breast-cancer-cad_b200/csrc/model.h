@@ -68,6 +68,10 @@ struct Xfer {                          // host-buffer pipeline (bcad_predict_exp
     // the end brings them back (three tiny D2H copies per chunk sat between the heat-map copies of the link-bound output stream)
     void* d_small = nullptr;
     size_t d_small_bytes = 0;
+    // both slots' staging of bcad_gradcam_overlays_classes_host (8-bit images, classes, K float / RGB / u8 maps of the image size),
+    // one allocation that is replaced when a call needs more
+    void* cls_arena = nullptr;
+    size_t cls_arena_bytes = 0;
 };
 
 struct TrainState {                     // row f4: buffers of the training step (allocated on first use)

@@ -542,6 +542,62 @@ def _gradcam_overlays_host(self, gray_u8: np.ndarray, class_idx=None, grad_mode:
 Engine.gradcam_overlays_host = _gradcam_overlays_host
 
 
+def _host_class_rows(classes, B, nc):
+    """classes of the host multi-class calls -> (K, C-contiguous int32 [B,K] array or None = column k is class k)."""
+    if classes is None:
+        K, ci = nc, None
+    else:
+        ci = np.asarray(classes, dtype=np.int32)
+        if ci.ndim == 1:
+            ci = np.broadcast_to(ci[None], (B, ci.shape[0]))
+        if ci.ndim != 2 or ci.shape[0] != B:
+            raise ValueError(f"classes must be a length-K sequence or a [{B},K] array, got shape {ci.shape}")
+        K = ci.shape[1]
+        if K >= 1 and (int(ci.min()) < 0 or int(ci.max()) >= nc):
+            raise ValueError("classes out of range")
+        ci = np.ascontiguousarray(ci)
+    if not 1 <= K <= _lib.MAX_EXPLAIN_CLASSES:
+        raise ValueError(f"{K} target classes per image; 1..{_lib.MAX_EXPLAIN_CLASSES} are supported")
+    return K, ci
+
+
+def _gradcam_overlays_classes_host(self, gray_u8: np.ndarray, classes=(0, 1), grad_mode: str = "logit", standardise: bool = True,
+                                   overlay_out: Optional[np.ndarray] = None, heat_out: Optional[np.ndarray] = None,
+                                   want_overlay: bool = True, want_heat: bool = True):
+    """The deployed dual-class call (app.py:649-657 -> GRADCAM.py:31-81) for a batch, end to end through one C-ABI call
+    (bcad_gradcam_overlays_classes_host): uint8 grey images [B,h,w] of ANY size -> (cls int32 [B], probs [B,nc], logits [B,nc],
+    overlay uint8 RGB [B,K,h,w,3] = show_cam_on_image, heatmap_uint8 [B,K,h,w]).  The CNN sees cv2.resize(img / 255, model size)
+    (standardised per image when ``standardise``); the maps have the size of the image.  ``classes``: a length-K sequence shared by
+    the batch, a [B,K] array or None (every class); K <= 8.  Pinned host arrays make the copies asynchronous."""
+    self.cache_tag = None
+    g = np.ascontiguousarray(gray_u8)
+    if g.dtype != np.uint8:
+        raise ValueError("gray_u8 must be uint8 (0-255 grey levels)")
+    if g.ndim == 2:
+        g = g[None]
+    if g.ndim != 3:
+        raise ValueError(f"gray_u8 must be [B,H,W] or [H,W], got shape {g.shape}")
+    B, h, w = g.shape
+    nc = self.spec.num_classes
+    K, ci = _host_class_rows(classes, B, nc)
+    logits, probs, cls = np.empty((B, nc), np.float32), np.empty((B, nc), np.float32), np.empty((B,), np.int32)
+    ov = hu = None
+    if want_overlay:
+        ov = overlay_out if overlay_out is not None else np.empty((B, K, h, w, 3), np.uint8)
+    if want_heat:
+        hu = heat_out if heat_out is not None else np.empty((B, K, h, w), np.uint8)
+    for a, shp in ((ov, (B, K, h, w, 3)), (hu, (B, K, h, w))):
+        if a is not None and (a.dtype != np.uint8 or a.shape != shp or not a.flags["C_CONTIGUOUS"]):
+            raise ValueError(f"output arrays must be C-contiguous uint8 of shape {shp}")
+    _lib.check(self.lib.bcad_gradcam_overlays_classes_host(self._h, _ptr(g), B, h, w, K, _ptr(ci), _lib.GRAD_MODE[grad_mode],
+                                                           1 if standardise else 0, _ptr(logits), _ptr(probs), _ptr(cls), _ptr(ov),
+                                                           _ptr(hu)))
+    return cls, probs, logits, ov, hu
+
+
+Engine.gradcam_overlays_classes_host = _gradcam_overlays_classes_host
+
+
 def gradcam_tail(A: torch.Tensor, dA: torch.Tensor, out_hw: Tuple[int, int]) -> torch.Tensor:
     """Stand-alone Grad-CAM tail on NHWC CUDA tensors [B,h,w,K] (fp32 or bf16) -> fp32 [B,H,W]."""
     lib = _lib.load()
@@ -572,6 +628,41 @@ def gray_preprocess(gray_u8: torch.Tensor, channels: int = 1, standardise: bool 
         _lib.check(lib.bcad_gray_preprocess(_ptr(g), B, H, W, int(channels), 1 if standardise else 0, _ptr(img01), _ptr(x),
                                             C.c_void_p(torch.cuda.current_stream(g.device).cuda_stream)))
     return img01, x
+
+
+def gray_resize_preprocess(gray_u8: torch.Tensor, out_hw: Tuple[int, int], channels: int = 1, standardise: bool = True) -> torch.Tensor:
+    """uint8 grey images [B,h,w] of any size on the GPU -> the CNN input x fp32 [B,H,W,channels] = cv2.resize(u8 / 255, (W, H),
+    INTER_LINEAR), standardised per image (mean / std of the resized image) when ``standardise``; ``out_hw`` = (H, W)."""
+    lib = _lib.load()
+    g = gray_u8.contiguous()
+    if g.dtype != torch.uint8 or g.dim() != 3 or not g.is_cuda:
+        raise ValueError("gray_u8 must be a CUDA uint8 tensor [B,H,W]")
+    B, h, w = g.shape
+    H, W = int(out_hw[0]), int(out_hw[1])
+    x = torch.empty((B, H, W, channels), device=g.device, dtype=torch.float32)
+    with torch.cuda.device(g.device):
+        _lib.check(lib.bcad_gray_resize_preprocess(_ptr(g), B, h, w, H, W, int(channels), 1 if standardise else 0, _ptr(x),
+                                                   C.c_void_p(torch.cuda.current_stream(g.device).cuda_stream)))
+    return x
+
+
+def overlay_classes(gray_u8: torch.Tensor, cams: torch.Tensor, want_overlay=True, want_heat_u8=True):
+    """show_cam_on_image + heatmap_uint8 for K maps per grey image on CUDA tensors: ``gray_u8`` uint8 [B,H,W] (img01 = u8 / 255, read
+    once for the K maps), ``cams`` fp32 [B,K,H,W] -> (u8 [B,K,H,W,3], u8 [B,K,H,W]); map k is byte for byte ``overlay(u8 / 255, cams[:, k])``."""
+    lib = _lib.load()
+    g = gray_u8.contiguous()
+    cam = cams.to(torch.float32).contiguous()
+    if cam.dim() != 4:
+        raise ValueError(f"cams must be [B,K,H,W], got shape {tuple(cam.shape)}")
+    B, K, H, W = cam.shape
+    if g.dtype != torch.uint8 or tuple(g.shape) != (B, H, W) or g.device != cam.device:
+        raise ValueError(f"gray_u8 must be a uint8 [{B},{H},{W}] tensor on the cams' device")
+    ov = torch.empty((B, K, H, W, 3), device=cam.device, dtype=torch.uint8) if want_overlay else None
+    hu = torch.empty((B, K, H, W), device=cam.device, dtype=torch.uint8) if want_heat_u8 else None
+    with torch.cuda.device(cam.device):
+        _lib.check(lib.bcad_overlay_classes(_ptr(g), _ptr(cam), B, K, H, W, _ptr(ov), _ptr(hu),
+                                            C.c_void_p(torch.cuda.current_stream(cam.device).cuda_stream)))
+    return ov, hu
 
 
 def overlay(img01: torch.Tensor, cam: torch.Tensor, want_overlay=True, want_heat_u8=True):
@@ -678,6 +769,47 @@ class ShardedEngine:
         if errs:
             raise errs[0]
         return cls, probs, logits, heat
+
+    def gradcam_overlays_classes_host(self, gray_u8: np.ndarray, classes=(0, 1), grad_mode="logit", standardise=True):
+        """Engine.gradcam_overlays_classes_host over the GPUs of the box: contiguous split, one host thread per GPU
+        -> (cls, probs, logits, overlays [B,K,h,w,3], heatmap_uint8 [B,K,h,w]).  The arrays are the driver's pinned buffers: they are
+        overwritten by the next call of the same shape (copy what must outlive it)."""
+        g = np.ascontiguousarray(gray_u8)
+        if g.dtype != np.uint8 or g.ndim not in (2, 3):
+            raise ValueError("gray_u8 must be uint8 [B,H,W] or [H,W]")
+        if g.ndim == 2:
+            g = g[None]
+        B, h, w = g.shape
+        nc = self.spec.num_classes
+        K, ci = _host_class_rows(classes, B, nc)
+        key = ("classes", B, K, h, w)
+        if self._out is None or self._out[0] != key:
+            bufs = (torch.empty((B,), dtype=torch.int32).pin_memory(), torch.empty((B, nc), dtype=torch.float32).pin_memory(),
+                    torch.empty((B, nc), dtype=torch.float32).pin_memory(), torch.empty((B, K, h, w, 3), dtype=torch.uint8).pin_memory(),
+                    torch.empty((B, K, h, w), dtype=torch.uint8).pin_memory())
+            self._out = (key, bufs)
+        cls, probs, logits, ov, hu = (t.numpy() for t in self._out[1])
+        errs = []
+
+        def work(e, s, t):
+            try:
+                if t <= s:
+                    return
+                c, p, l, _, _ = e.gradcam_overlays_classes_host(g[s:t], None if ci is None else ci[s:t], grad_mode, standardise,
+                                                                overlay_out=ov[s:t], heat_out=hu[s:t])
+                cls[s:t], probs[s:t], logits[s:t] = c, p, l
+            except Exception as ex:  # surfaced after join
+                errs.append(ex)
+
+        ths = [threading.Thread(target=work, args=(e, s, t))
+               for e, (s, t) in zip(self.engines, shard_bounds(B, len(self.engines)))]
+        for t in ths:
+            t.start()
+        for t in ths:
+            t.join()
+        if errs:
+            raise errs[0]
+        return cls, probs, logits, ov, hu
 
     def close(self):
         for e in self.engines:
