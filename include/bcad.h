@@ -223,6 +223,22 @@ BCAD_API int bcad_gradcam_overlays_classes_host(bcad_model* m, const uint8_t* gr
                                                 const int32_t* classes_host_or_null, int grad_mode, int standardise, float* logits_host,
                                                 float* probs_host, int32_t* cls_host, uint8_t* overlay_rgb_host, uint8_t* heat_u8_host);
 
+/* The dual-class input-gradient saliency overlays (explainability.py:81-108) for a BATCH of 8-bit grey images of ANY size, end to end:
+ * gray_u8_host uint8 [B][img_h][img_w] -> the CNN input of bcad_gradcam_overlays_classes_host (bcad_gray_resize_preprocess) -> one
+ * forward and K saliency maps per image at the model's size (bcad_predict_saliency_classes) -> per map generate_saliency_overlay at the
+ * image's size with the grey image as the blend base (bcad_saliency_overlay_resized).  fp32 handles with keep_all_activations = 1 and
+ * no dropout masks set; the kernels follow bcad_set_fast_training.  classes_host_or_null int32 [B][K] or NULL (column k = class k,
+ * K <= num_classes); 1 <= K <= BCAD_MAX_EXPLAIN_CLASSES; grad_mode BCAD_GRAD_* (the reference uses SOFTMAX_CE).  Outputs, each may be
+ * NULL but not all three: saliency_host fp32 [B][K][H][W] (model size, as bcad_predict_saliency_classes), overlay_bgr_host and
+ * heat_bgr_host uint8 [B][K][img_h][img_w][3] (BGR, as cv2 returns them).  logits / probs / cls host (each may be NULL).  The chunked
+ * three-stream pipeline of bcad_gradcam_overlays_classes_host, its staging held under 512 MB of device memory in the same way.  Every
+ * output is byte for byte the device composition bcad_gray_resize_preprocess -> bcad_predict_saliency_classes ->
+ * bcad_saliency_overlay_resized. */
+BCAD_API int bcad_saliency_overlays_classes_host(bcad_model* m, const uint8_t* gray_u8_host, int B, int img_h, int img_w, int K,
+                                                 const int32_t* classes_host_or_null, int grad_mode, int standardise, float* logits_host,
+                                                 float* probs_host, int32_t* cls_host, float* saliency_host, uint8_t* overlay_bgr_host,
+                                                 uint8_t* heat_bgr_host);
+
 /* ---- stand-alone Grad-CAM tail (pytorch_grad_cam BaseCAM.forward / scale_cam_image) ------------ */
 /* A, dA: [B,h,w,K] NHWC device, dtype 0 = fp32, 1 = bf16; out: fp32 [B,H,W].
  * alpha_k = mean_hw dA_k ; cam = ReLU(sum_k alpha_k A_k) ; min-max ; bilinear (cv2.resize) ; min-max. */
@@ -252,6 +268,13 @@ BCAD_API int bcad_gray_resize_preprocess(const uint8_t* gray_u8_dev, int B, int 
  * BCAD_MAX_EXPLAIN_CLASSES.  Map k is byte for byte bcad_overlay(u8 / 255, cam[:, k]). */
 BCAD_API int bcad_overlay_classes(const uint8_t* gray_u8_dev, const float* cam_dev, int B, int K, int H, int W, uint8_t* overlay_rgb_dev,
                                   uint8_t* heat_u8_dev, void* stream);
+/* The colouring stage of bcad_saliency_overlays_classes_host: gray_u8_dev uint8 [B][img_h][img_w], saliency_dev fp32 [B][K][H][W] in
+ * [0, 1] -> heat = cv2.resize(applyColorMap(uint8(sal * 255), JET), (img_w, img_h)) (OpenCV's 8-bit INTER_LINEAR, bit for bit) and
+ * overlay = addWeighted(grey3, 0.5, heat, 0.5, 0), both uint8 [B][K][img_h][img_w][3] BGR (either may be NULL).  The grey image is read
+ * once per pixel for all K maps; 1 <= K <= BCAD_MAX_EXPLAIN_CLASSES, B <= 65535.  At img_h x img_w == H x W exactly
+ * bcad_saliency_overlay with base_c = 1. */
+BCAD_API int bcad_saliency_overlay_resized(const uint8_t* gray_u8_dev, const float* saliency_dev, int B, int K, int H, int W, int img_h,
+                                           int img_w, uint8_t* overlay_bgr_dev, uint8_t* heat_bgr_dev, void* stream);
 
 /* ---- tiny U-Net encoder front (SURVEY 8 row f1): conv2d + relu + max_pool of Classes/unet.py:13-73 ------- */
 /* y = LeakyReLU_alpha(conv(x, kernel) + bias), NHWC fp32, kernel DEVICE fp32 (k,k,Cin,Cout) as unet.py holds it, bias

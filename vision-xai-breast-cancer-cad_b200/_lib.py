@@ -59,6 +59,9 @@ _SIGNATURES = {
     "bcad_gradcam_overlays_host": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, _P, _P, _P, _P, _P]),
     "bcad_gradcam_overlays_classes_host": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, C.c_int, C.c_int, _P, _P, _P,
                                                      _P, _P]),
+    "bcad_saliency_overlays_classes_host": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, C.c_int, C.c_int, _P, _P, _P,
+                                                      _P, _P, _P]),
+    "bcad_saliency_overlay_resized": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P]),
     "bcad_gray_resize_preprocess": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P]),
     "bcad_overlay_classes": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P]),
     "bcad_explain_backward": (C.c_int, [_P, C.c_int, _P, C.c_int, C.POINTER(_P), _P, _P]),

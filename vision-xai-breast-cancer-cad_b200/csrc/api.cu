@@ -1120,79 +1120,95 @@ int bcad_gradcam_overlays_host(bcad_model* mm, const uint8_t* gray_u8_host, int 
                                      heat_u8_host, gray_u8_host, standardise, overlay_rgb_host);
 }
 
-// Staging bound of bcad_gradcam_overlays_classes_host: both slots' 8-bit images, classes and K float / RGB / u8 maps of the image size
-// stay within this many bytes of the handle's memory (the chunk shrinks to fit; a single image larger than half of it still runs, one
-// image per chunk).  512 x 512 images with K = 2: 4.25 MB per image and slot, chunks of up to 60 images.
+// Staging bound of the host-buffer classes calls (bcad_gradcam_overlays_classes_host, bcad_saliency_overlays_classes_host): both slots'
+// 8-bit images, classes and maps stay within this many bytes of the handle's memory (the chunk shrinks to fit; a single image larger
+// than half of it still runs, one image per chunk).  Grad-CAM, 512 x 512 images with K = 2: 4.25 MB per image and slot, chunks of up
+// to 60 images.
 static const size_t kClassesStagingBytes = (size_t)512 << 20;
 
 static size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
 
-int bcad_gradcam_overlays_classes_host(bcad_model* mm, const uint8_t* gray_u8_host, int B, int img_h, int img_w, int K,
-                                       const int32_t* classes_host_or_null, int grad_mode, int standardise, float* logits_host,
-                                       float* probs_host, int32_t* cls_host, uint8_t* overlay_rgb_host, uint8_t* heat_u8_host) {
-    Model* m = reinterpret_cast<Model*>(mm);
-    BCAD_REQUIRE(m && gray_u8_host, "gradcam_overlays_classes_host: null model or image pointer");
-    BCAD_REQUIRE(overlay_rgb_host || heat_u8_host, "gradcam_overlays_classes_host: overlay and heat-map pointers are both null");
+// The checks shared by the classes calls, all made before any copy.  fn names the call in the messages.
+static int check_classes_host(const char* fn, Model* m, const uint8_t* gray_u8_host, int B, int img_h, int img_w, int K,
+                              const int32_t* classes_host_or_null, int grad_mode, int standardise, bool any_output) {
+    BCAD_REQUIRE(m && gray_u8_host, "%s: null model or image pointer", fn);
+    BCAD_REQUIRE(any_output, "%s: the output pointers are all null", fn);
     BCAD_REQUIRE(B >= 1, "batch must be >= 1, got %d", B);
-    BCAD_REQUIRE(img_h >= 1 && img_w >= 1 && img_h <= 16384 && img_w <= 16384, "gradcam_overlays_classes_host: bad image size %dx%d", img_h, img_w);
-    BCAD_REQUIRE(K >= 1 && K <= BCAD_MAX_EXPLAIN_CLASSES, "gradcam_overlays_classes_host: K=%d out of range 1..%d", K, BCAD_MAX_EXPLAIN_CLASSES);
-    BCAD_REQUIRE(standardise == 0 || standardise == 1, "gradcam_overlays_classes_host: standardise must be 0 or 1");
+    BCAD_REQUIRE(img_h >= 1 && img_w >= 1 && img_h <= 16384 && img_w <= 16384, "%s: bad image size %dx%d", fn, img_h, img_w);
+    BCAD_REQUIRE(K >= 1 && K <= BCAD_MAX_EXPLAIN_CLASSES, "%s: K=%d out of range 1..%d", fn, K, BCAD_MAX_EXPLAIN_CLASSES);
+    BCAD_REQUIRE(standardise == 0 || standardise == 1, "%s: standardise must be 0 or 1", fn);
     BCAD_REQUIRE(grad_mode == BCAD_GRAD_LOGIT || grad_mode == BCAD_GRAD_SOFTMAX_CE, "bad grad_mode %d", grad_mode);
     const int nc = m->cfg.num_classes;
-    BCAD_REQUIRE(classes_host_or_null || K <= nc, "gradcam_overlays_classes_host: classes=NULL explains classes 0..K-1, but K=%d > num_classes=%d", K, nc);
+    BCAD_REQUIRE(classes_host_or_null || K <= nc, "%s: classes=NULL explains classes 0..K-1, but K=%d > num_classes=%d", fn, K, nc);
     if (classes_host_or_null != nullptr)
         for (size_t i = 0; i < (size_t)B * K; ++i)
             BCAD_REQUIRE(classes_host_or_null[i] >= 0 && classes_host_or_null[i] < nc, "classes[%zu][%zu] = %d is outside [0, %d)", i / K, i % K,
                          classes_host_or_null[i], nc);
     if (!m->committed) { set_error("weights not committed: call bcad_commit first"); return BCAD_ERR_STATE; }
-    DeviceGuard g(m->cfg.device);
-    std::lock_guard<std::mutex> host_lock(m->host_mu);
+    return BCAD_OK;
+}
+
+// Chunk size of a classes call and the arena holding both slots of per_img_slot bytes per image (caller holds m->host_mu): the chunk of
+// bcad_gradcam_overlays_host (a quarter of the batch, 32..128 images), shrunk to the staging bound.  Slot i starts at
+// arena + i * C0 * per_img_slot.
+static int classes_staging(Model* m, int B, size_t per_img_slot, int& C0, uint8_t*& arena) {
     Xfer& X = m->xfer;
-    const size_t hw = (size_t)img_h * img_w;
-    // per image and slot: 8-bit image, class row, float maps, RGB overlays, u8 heat-maps
-    const size_t b_img = align256(hw), b_cls = align256((size_t)K * sizeof(int32_t)), b_heat = align256((size_t)K * hw * sizeof(float));
-    const size_t b_ov = overlay_rgb_host ? align256((size_t)K * hw * 3) : 0, b_h8 = heat_u8_host ? align256((size_t)K * hw) : 0;
-    const size_t per_img_slot = b_img + b_cls + b_heat + b_ov + b_h8;
-    int C0;
-    {
-        std::lock_guard<std::mutex> lock(m->mu);
-        BCAD_TRY(xfer_init(m));
-        // the chunk of bcad_gradcam_overlays_host (a quarter of the batch, 32..128 images), shrunk to the staging bound
-        C0 = std::min(std::min(X.chunk, 128), std::max(32, ((B + 3) / 4 + 31) / 32 * 32));
-        if (const char* e = getenv("BCAD_HOST_CHUNK")) C0 = std::max(1, std::min(X.chunk, atoi(e)));
-        C0 = (int)std::max<size_t>(1, std::min<size_t>((size_t)C0, kClassesStagingBytes / (2 * per_img_slot)));
-        const size_t need = 2 * (size_t)C0 * per_img_slot;
-        if (X.cls_arena_bytes < need) {
-            if (X.cls_arena != nullptr) {                     // replaced, not kept until destroy: it can be hundreds of MB
-                BCAD_CUDA_CHECK(cudaFree(X.cls_arena));       // (synchronises the device: no earlier call still reads it)
-                m->allocs.erase(std::find(m->allocs.begin(), m->allocs.end(), X.cls_arena));
-                m->ws_bytes -= X.cls_arena_bytes;
-                X.cls_arena = nullptr;
-                X.cls_arena_bytes = 0;
-            }
-            BCAD_TRY(m->alloc(&X.cls_arena, need));
-            X.cls_arena_bytes = need;
+    std::lock_guard<std::mutex> lock(m->mu);
+    BCAD_TRY(xfer_init(m));
+    C0 = std::min(std::min(X.chunk, 128), std::max(32, ((B + 3) / 4 + 31) / 32 * 32));
+    if (const char* e = getenv("BCAD_HOST_CHUNK")) C0 = std::max(1, std::min(X.chunk, atoi(e)));
+    C0 = (int)std::max<size_t>(1, std::min<size_t>((size_t)C0, kClassesStagingBytes / (2 * per_img_slot)));
+    const size_t need = 2 * (size_t)C0 * per_img_slot;
+    if (X.cls_arena_bytes < need) {
+        if (X.cls_arena != nullptr) {                     // replaced, not kept until destroy: it can be hundreds of MB
+            BCAD_CUDA_CHECK(cudaFree(X.cls_arena));       // (synchronises the device: no earlier call still reads it)
+            m->allocs.erase(std::find(m->allocs.begin(), m->allocs.end(), X.cls_arena));
+            m->ws_bytes -= X.cls_arena_bytes;
+            X.cls_arena = nullptr;
+            X.cls_arena_bytes = 0;
         }
+        BCAD_TRY(m->alloc(&X.cls_arena, need));
+        X.cls_arena_bytes = need;
     }
-    uint8_t *d_img[2], *d_ov[2], *d_h8[2];
-    int32_t* d_cls[2];
-    float* d_heat[2];
-    for (int i = 0; i < 2; ++i) {
-        uint8_t* p = reinterpret_cast<uint8_t*>(X.cls_arena) + (size_t)i * C0 * per_img_slot;
-        d_img[i] = p;                                         p += (size_t)C0 * b_img;
-        d_cls[i] = reinterpret_cast<int32_t*>(p);             p += (size_t)C0 * b_cls;
-        d_heat[i] = reinterpret_cast<float*>(p);              p += (size_t)C0 * b_heat;
-        d_ov[i] = overlay_rgb_host ? p : nullptr;             p += (size_t)C0 * b_ov;
-        d_h8[i] = heat_u8_host ? p : nullptr;
-    }
-    const size_t per_img = (size_t)(2 * nc) * sizeof(float) + sizeof(int32_t);
-    BCAD_TRY(stage_small(m, per_img * B));
-    float* st_logits = reinterpret_cast<float*>(X.h_small);
-    float* st_probs = st_logits + (size_t)B * nc;
-    int32_t* st_cls = reinterpret_cast<int32_t*>(st_probs + (size_t)B * nc);
-    float* dv_logits = reinterpret_cast<float*>(X.d_small);
-    float* dv_probs = dv_logits + (size_t)B * nc;
-    int32_t* dv_cls = reinterpret_cast<int32_t*>(dv_probs + (size_t)B * nc);
+    arena = reinterpret_cast<uint8_t*>(X.cls_arena);
+    return BCAD_OK;
+}
+
+// logits / probabilities / classes of a whole classes call: written on the device per chunk, brought back by one copy behind the last
+// chunk through the pinned staging of stage_small
+struct SmallOutputs {
+    size_t bytes = 0;
+    float *dv_logits = nullptr, *dv_probs = nullptr;
+    int32_t* dv_cls = nullptr;
+};
+
+static int small_outputs(Model* m, int B, SmallOutputs& o) {
+    const int nc = m->cfg.num_classes;
+    o.bytes = ((size_t)(2 * nc) * sizeof(float) + sizeof(int32_t)) * B;
+    BCAD_TRY(stage_small(m, o.bytes));
+    o.dv_logits = reinterpret_cast<float*>(m->xfer.d_small);
+    o.dv_probs = o.dv_logits + (size_t)B * nc;
+    o.dv_cls = reinterpret_cast<int32_t*>(o.dv_probs + (size_t)B * nc);
+    return BCAD_OK;
+}
+
+static void copy_small_outputs(Model* m, int B, float* logits_host, float* probs_host, int32_t* cls_host) {
+    const int nc = m->cfg.num_classes;
+    const float* st_logits = reinterpret_cast<const float*>(m->xfer.h_small);
+    const float* st_probs = st_logits + (size_t)B * nc;
+    const int32_t* st_cls = reinterpret_cast<const int32_t*>(st_probs + (size_t)B * nc);
+    if (logits_host) memcpy(logits_host, st_logits, (size_t)B * nc * sizeof(float));
+    if (probs_host) memcpy(probs_host, st_probs, (size_t)B * nc * sizeof(float));
+    if (cls_host) memcpy(cls_host, st_cls, (size_t)B * sizeof(int32_t));
+}
+
+// The chunk loop of the classes calls: per chunk c (slot c & 1, images b0 .. b0 + n) h2d(slot, b0, n) on s_in, compute(slot, b0, n) on
+// s_compute, d2h(slot, b0, n) on s_out, ordered by the slot's events; the small outputs follow the last chunk's D2H.  Returns after
+// both streams have drained.
+extern "C++" {
+template <class H2D, class Compute, class D2H>
+static int classes_pipeline(Model* m, int B, int C0, const SmallOutputs& so, H2D h2d, Compute compute, D2H d2h) {
+    Xfer& X = m->xfer;
     const int nchunks = (B + C0 - 1) / C0;
     for (int c = 0, b0 = 0; c < nchunks; ++c, b0 += C0) {
         const int slot = c & 1, n = std::min(C0, B - b0);
@@ -1200,30 +1216,147 @@ int bcad_gradcam_overlays_classes_host(bcad_model* mm, const uint8_t* gray_u8_ho
             BCAD_CUDA_CHECK(cudaStreamWaitEvent(X.s_in, X.compute_done[slot], 0));
             BCAD_CUDA_CHECK(cudaStreamWaitEvent(X.s_compute, X.out_done[slot], 0));
         }
-        BCAD_CUDA_CHECK(cudaMemcpyAsync(d_img[slot], gray_u8_host + (size_t)b0 * hw, (size_t)n * hw, cudaMemcpyHostToDevice, X.s_in));
-        if (classes_host_or_null)
-            BCAD_CUDA_CHECK(cudaMemcpyAsync(d_cls[slot], classes_host_or_null + (size_t)b0 * K, (size_t)n * K * sizeof(int32_t), cudaMemcpyHostToDevice, X.s_in));
+        BCAD_TRY(h2d(slot, b0, n));
         BCAD_CUDA_CHECK(cudaEventRecord(X.in_done[slot], X.s_in));
         BCAD_CUDA_CHECK(cudaStreamWaitEvent(X.s_compute, X.in_done[slot], 0));
-        int rc = launch_gray_resize_preprocess(d_img[slot], X.x[slot], n, img_h, img_w, m->cfg.in_h, m->cfg.in_w, m->cfg.in_c, standardise, X.s_compute);
-        if (rc == BCAD_OK)
-            rc = run(m, X.x[slot], n, classes_host_or_null ? d_cls[slot] : nullptr, grad_mode, true, dv_logits + (size_t)b0 * nc,
-                     dv_probs + (size_t)b0 * nc, dv_cls + b0, d_heat[slot], X.s_compute, img_h, img_w, K);
-        if (rc == BCAD_OK) rc = launch_overlay_classes(d_img[slot], d_heat[slot], n, K, (int)hw, d_ov[slot], d_h8[slot], X.s_compute);
+        const int rc = compute(slot, b0, n);
         if (rc != BCAD_OK) { cudaDeviceSynchronize(); return rc; }
         BCAD_CUDA_CHECK(cudaEventRecord(X.compute_done[slot], X.s_compute));
         BCAD_CUDA_CHECK(cudaStreamWaitEvent(X.s_out, X.compute_done[slot], 0));
-        const size_t maps = (size_t)b0 * K * hw, nmaps = (size_t)n * K * hw;
-        if (overlay_rgb_host) BCAD_CUDA_CHECK(cudaMemcpyAsync(overlay_rgb_host + maps * 3, d_ov[slot], nmaps * 3, cudaMemcpyDeviceToHost, X.s_out));
-        if (heat_u8_host) BCAD_CUDA_CHECK(cudaMemcpyAsync(heat_u8_host + maps, d_h8[slot], nmaps, cudaMemcpyDeviceToHost, X.s_out));
-        if (c + 1 == nchunks) BCAD_CUDA_CHECK(cudaMemcpyAsync(X.h_small, X.d_small, per_img * B, cudaMemcpyDeviceToHost, X.s_out));
+        BCAD_TRY(d2h(slot, b0, n));
+        if (c + 1 == nchunks) BCAD_CUDA_CHECK(cudaMemcpyAsync(X.h_small, X.d_small, so.bytes, cudaMemcpyDeviceToHost, X.s_out));
         BCAD_CUDA_CHECK(cudaEventRecord(X.out_done[slot], X.s_out));
     }
     BCAD_CUDA_CHECK(cudaStreamSynchronize(X.s_out));
     BCAD_CUDA_CHECK(cudaStreamSynchronize(X.s_compute));
-    if (logits_host) memcpy(logits_host, st_logits, (size_t)B * nc * sizeof(float));
-    if (probs_host) memcpy(probs_host, st_probs, (size_t)B * nc * sizeof(float));
-    if (cls_host) memcpy(cls_host, st_cls, (size_t)B * sizeof(int32_t));
+    return BCAD_OK;
+}
+}  // extern "C++"
+
+int bcad_gradcam_overlays_classes_host(bcad_model* mm, const uint8_t* gray_u8_host, int B, int img_h, int img_w, int K,
+                                       const int32_t* classes_host_or_null, int grad_mode, int standardise, float* logits_host,
+                                       float* probs_host, int32_t* cls_host, uint8_t* overlay_rgb_host, uint8_t* heat_u8_host) {
+    Model* m = reinterpret_cast<Model*>(mm);
+    BCAD_TRY(check_classes_host("gradcam_overlays_classes_host", m, gray_u8_host, B, img_h, img_w, K, classes_host_or_null, grad_mode,
+                                standardise, overlay_rgb_host || heat_u8_host));
+    DeviceGuard g(m->cfg.device);
+    std::lock_guard<std::mutex> host_lock(m->host_mu);
+    Xfer& X = m->xfer;
+    const int nc = m->cfg.num_classes;
+    const size_t hw = (size_t)img_h * img_w;
+    // per image and slot: 8-bit image, class row, float maps, RGB overlays, u8 heat-maps
+    const size_t b_img = align256(hw), b_cls = align256((size_t)K * sizeof(int32_t)), b_heat = align256((size_t)K * hw * sizeof(float));
+    const size_t b_ov = overlay_rgb_host ? align256((size_t)K * hw * 3) : 0, b_h8 = heat_u8_host ? align256((size_t)K * hw) : 0;
+    const size_t per_img_slot = b_img + b_cls + b_heat + b_ov + b_h8;
+    int C0;
+    uint8_t* arena;
+    BCAD_TRY(classes_staging(m, B, per_img_slot, C0, arena));
+    uint8_t *d_img[2], *d_ov[2], *d_h8[2];
+    int32_t* d_cls[2];
+    float* d_heat[2];
+    for (int i = 0; i < 2; ++i) {
+        uint8_t* p = arena + (size_t)i * C0 * per_img_slot;
+        d_img[i] = p;                                         p += (size_t)C0 * b_img;
+        d_cls[i] = reinterpret_cast<int32_t*>(p);             p += (size_t)C0 * b_cls;
+        d_heat[i] = reinterpret_cast<float*>(p);              p += (size_t)C0 * b_heat;
+        d_ov[i] = overlay_rgb_host ? p : nullptr;             p += (size_t)C0 * b_ov;
+        d_h8[i] = heat_u8_host ? p : nullptr;
+    }
+    SmallOutputs so;
+    BCAD_TRY(small_outputs(m, B, so));
+    BCAD_TRY(classes_pipeline(m, B, C0, so,
+        [&](int slot, int b0, int n) {
+            BCAD_CUDA_CHECK(cudaMemcpyAsync(d_img[slot], gray_u8_host + (size_t)b0 * hw, (size_t)n * hw, cudaMemcpyHostToDevice, X.s_in));
+            if (classes_host_or_null)
+                BCAD_CUDA_CHECK(cudaMemcpyAsync(d_cls[slot], classes_host_or_null + (size_t)b0 * K, (size_t)n * K * sizeof(int32_t),
+                                                cudaMemcpyHostToDevice, X.s_in));
+            return BCAD_OK;
+        },
+        [&](int slot, int b0, int n) {
+            int rc = launch_gray_resize_preprocess(d_img[slot], X.x[slot], n, img_h, img_w, m->cfg.in_h, m->cfg.in_w, m->cfg.in_c, standardise,
+                                                   X.s_compute);
+            if (rc == BCAD_OK)
+                rc = run(m, X.x[slot], n, classes_host_or_null ? d_cls[slot] : nullptr, grad_mode, true, so.dv_logits + (size_t)b0 * nc,
+                         so.dv_probs + (size_t)b0 * nc, so.dv_cls + b0, d_heat[slot], X.s_compute, img_h, img_w, K);
+            if (rc == BCAD_OK) rc = launch_overlay_classes(d_img[slot], d_heat[slot], n, K, (int)hw, d_ov[slot], d_h8[slot], X.s_compute);
+            return rc;
+        },
+        [&](int slot, int b0, int n) {
+            const size_t maps = (size_t)b0 * K * hw, nmaps = (size_t)n * K * hw;
+            if (overlay_rgb_host) BCAD_CUDA_CHECK(cudaMemcpyAsync(overlay_rgb_host + maps * 3, d_ov[slot], nmaps * 3, cudaMemcpyDeviceToHost, X.s_out));
+            if (heat_u8_host) BCAD_CUDA_CHECK(cudaMemcpyAsync(heat_u8_host + maps, d_h8[slot], nmaps, cudaMemcpyDeviceToHost, X.s_out));
+            return BCAD_OK;
+        }));
+    copy_small_outputs(m, B, logits_host, probs_host, cls_host);
+    return BCAD_OK;
+}
+
+int bcad_saliency_overlays_classes_host(bcad_model* mm, const uint8_t* gray_u8_host, int B, int img_h, int img_w, int K,
+                                        const int32_t* classes_host_or_null, int grad_mode, int standardise, float* logits_host,
+                                        float* probs_host, int32_t* cls_host, float* saliency_host, uint8_t* overlay_bgr_host,
+                                        uint8_t* heat_bgr_host) {
+    Model* m = reinterpret_cast<Model*>(mm);
+    BCAD_TRY(check_classes_host("saliency_overlays_classes_host", m, gray_u8_host, B, img_h, img_w, K, classes_host_or_null, grad_mode,
+                                standardise, saliency_host || overlay_bgr_host || heat_bgr_host));
+    // what run_saliency would refuse, refused before any copy
+    BCAD_REQUIRE(!m->tensor_path, "saliency_overlays_classes_host runs on the fp32 path (the 16-bit forward keeps no first-block output): "
+                                  "create the model with BCAD_PREC_FP32");
+    BCAD_REQUIRE(m->cfg.keep_all_activations, "saliency_overlays_classes_host needs every conv block's output: create the model with "
+                                              "keep_all_activations=1");
+    BCAD_REQUIRE(!m->train.drop_B, "saliency_overlays_classes_host is an inference call: clear the dropout masks first "
+                                   "(bcad_set_dropout_masks(m, NULL, 0))");
+    DeviceGuard g(m->cfg.device);
+    std::lock_guard<std::mutex> host_lock(m->host_mu);
+    Xfer& X = m->xfer;
+    const int nc = m->cfg.num_classes, H = m->cfg.in_h, W = m->cfg.in_w;
+    const size_t hw = (size_t)img_h * img_w, mhw = (size_t)H * W;
+    // per image and slot: 8-bit image, class row, model-size float saliency, BGR overlays, BGR heat-maps
+    const size_t b_img = align256(hw), b_cls = align256((size_t)K * sizeof(int32_t)), b_sal = align256((size_t)K * mhw * sizeof(float));
+    const size_t b_ov = overlay_bgr_host ? align256((size_t)K * hw * 3) : 0, b_ht = heat_bgr_host ? align256((size_t)K * hw * 3) : 0;
+    const size_t per_img_slot = b_img + b_cls + b_sal + b_ov + b_ht;
+    int C0;
+    uint8_t* arena;
+    BCAD_TRY(classes_staging(m, B, per_img_slot, C0, arena));
+    uint8_t *d_img[2], *d_ov[2], *d_ht[2];
+    int32_t* d_cls[2];
+    float* d_sal[2];
+    for (int i = 0; i < 2; ++i) {
+        uint8_t* p = arena + (size_t)i * C0 * per_img_slot;
+        d_img[i] = p;                                         p += (size_t)C0 * b_img;
+        d_cls[i] = reinterpret_cast<int32_t*>(p);             p += (size_t)C0 * b_cls;
+        d_sal[i] = reinterpret_cast<float*>(p);               p += (size_t)C0 * b_sal;
+        d_ov[i] = overlay_bgr_host ? p : nullptr;             p += (size_t)C0 * b_ov;
+        d_ht[i] = heat_bgr_host ? p : nullptr;
+    }
+    SmallOutputs so;
+    BCAD_TRY(small_outputs(m, B, so));
+    BCAD_TRY(classes_pipeline(m, B, C0, so,
+        [&](int slot, int b0, int n) {
+            BCAD_CUDA_CHECK(cudaMemcpyAsync(d_img[slot], gray_u8_host + (size_t)b0 * hw, (size_t)n * hw, cudaMemcpyHostToDevice, X.s_in));
+            if (classes_host_or_null)
+                BCAD_CUDA_CHECK(cudaMemcpyAsync(d_cls[slot], classes_host_or_null + (size_t)b0 * K, (size_t)n * K * sizeof(int32_t),
+                                                cudaMemcpyHostToDevice, X.s_in));
+            return BCAD_OK;
+        },
+        [&](int slot, int b0, int n) {
+            int rc = launch_gray_resize_preprocess(d_img[slot], X.x[slot], n, img_h, img_w, H, W, m->cfg.in_c, standardise, X.s_compute);
+            if (rc == BCAD_OK)
+                rc = run_saliency(m, X.x[slot], n, K, classes_host_or_null ? d_cls[slot] : nullptr, grad_mode, so.dv_logits + (size_t)b0 * nc,
+                                  so.dv_probs + (size_t)b0 * nc, so.dv_cls + b0, d_sal[slot], nullptr, X.s_compute);
+            if (rc == BCAD_OK && (overlay_bgr_host || heat_bgr_host))
+                rc = launch_saliency_overlay_resized(d_img[slot], d_sal[slot], n, K, H, W, img_h, img_w, d_ov[slot], d_ht[slot], X.s_compute);
+            return rc;
+        },
+        [&](int slot, int b0, int n) {
+            const size_t maps = (size_t)b0 * K * hw * 3, bytes = (size_t)n * K * hw * 3;
+            if (saliency_host)
+                BCAD_CUDA_CHECK(cudaMemcpyAsync(saliency_host + (size_t)b0 * K * mhw, d_sal[slot], (size_t)n * K * mhw * sizeof(float),
+                                                cudaMemcpyDeviceToHost, X.s_out));
+            if (overlay_bgr_host) BCAD_CUDA_CHECK(cudaMemcpyAsync(overlay_bgr_host + maps, d_ov[slot], bytes, cudaMemcpyDeviceToHost, X.s_out));
+            if (heat_bgr_host) BCAD_CUDA_CHECK(cudaMemcpyAsync(heat_bgr_host + maps, d_ht[slot], bytes, cudaMemcpyDeviceToHost, X.s_out));
+            return BCAD_OK;
+        }));
+    copy_small_outputs(m, B, logits_host, probs_host, cls_host);
     return BCAD_OK;
 }
 
@@ -1280,6 +1413,16 @@ int bcad_overlay_classes(const uint8_t* gray_u8, const float* cam, int B, int K,
     BCAD_REQUIRE(K >= 1 && K <= BCAD_MAX_EXPLAIN_CLASSES, "overlay_classes: K=%d out of range 1..%d", K, BCAD_MAX_EXPLAIN_CLASSES);
     BCAD_REQUIRE(B >= 1 && H >= 1 && W >= 1 && (int64_t)H * W <= 0x7fffffff, "overlay_classes: bad sizes B=%d %dx%d", B, H, W);
     return launch_overlay_classes(gray_u8, cam, B, K, H * W, overlay_rgb, heat_u8, (cudaStream_t)stream);
+}
+
+int bcad_saliency_overlay_resized(const uint8_t* gray_u8, const float* saliency, int B, int K, int H, int W, int img_h, int img_w,
+                                  uint8_t* overlay_bgr, uint8_t* heat_bgr, void* stream) {
+    BCAD_REQUIRE(gray_u8 && saliency, "saliency_overlay_resized: null image or saliency");
+    BCAD_REQUIRE(K >= 1 && K <= BCAD_MAX_EXPLAIN_CLASSES, "saliency_overlay_resized: K=%d out of range 1..%d", K, BCAD_MAX_EXPLAIN_CLASSES);
+    BCAD_REQUIRE(B >= 1 && B <= 65535 && H >= 1 && W >= 1 && (int64_t)H * W <= 0x7fffffff && img_h >= 1 && img_w >= 1 && img_h <= 16384 &&
+                     img_w <= 16384, "saliency_overlay_resized: bad sizes B=%d %dx%d -> %dx%d", B, H, W, img_h, img_w);
+    if (overlay_bgr == nullptr && heat_bgr == nullptr) return BCAD_OK;
+    return launch_saliency_overlay_resized(gray_u8, saliency, B, K, H, W, img_h, img_w, overlay_bgr, heat_bgr, (cudaStream_t)stream);
 }
 
 // -----------------------------------------------------------------------------------------------------

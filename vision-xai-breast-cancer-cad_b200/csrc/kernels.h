@@ -63,6 +63,10 @@ int launch_overlay(const float* img01, const float* cam, int B, int H, int W, ui
 // overlay / heat u8 [B][K][npix][3] BGR (either may be null)
 int launch_saliency_overlay(const uint8_t* base, int base_c, const float* sal, int B, int K, int npix, uint8_t* overlay, uint8_t* heat,
                             cudaStream_t s);
+// the same at the image's size: g8 u8 grey [B][hi][wi], sal fp32 [B][K][H][W] -> overlay / heat u8 [B][K][hi][wi][3] BGR (either may be
+// null) = addWeighted(grey3, 0.5, cv2.resize(JET(sal), (wi, hi), INTER_LINEAR), 0.5, 0); 1 <= K <= BCAD_MAX_EXPLAIN_CLASSES, hi <= 65535
+int launch_saliency_overlay_resized(const uint8_t* g8, const float* sal, int B, int K, int H, int W, int hi, int wi, uint8_t* overlay,
+                                    uint8_t* heat, cudaStream_t s);
 
 // ---------------------------------------------------------------- input-gradient saliency (saliency.cu)
 // Outputs of one target class: image b's map at sal + b * out_stride (d_input: + b * out_stride * C), its min / max counters at

@@ -1159,6 +1159,120 @@ int launch_saliency_overlay(const uint8_t* base, int base_c, const float* sal, i
     return BCAD_OK;
 }
 
+// OpenCV's INTER_LINEAR source coordinate of destination index d (ns source, nd destination pixels): scale = 1 / (nd / ns) in double as
+// cv::resize forms it, f = float((d + 0.5) * scale - 0.5) without FMA contraction, s = floor(f), f -= s.
+__device__ __forceinline__ void cv_linear_coord(int d, int ns, int nd, int& s, float& f) {
+    const double scale = 1.0 / ((double)nd / (double)ns);
+    f = (float)__dsub_rn(__dmul_rn((double)d + 0.5, scale), 0.5);
+    const float fl = floorf(f);
+    s = (int)fl;
+    f -= fl;
+}
+
+// generate_saliency_overlay (explainability.py:74-77) at the image's size for [B][K] model-size maps: the JET heat-map of the map
+// (applyColorMap(uint8(s * 255)), built on the fly for the 2x2 source neighbourhood of each output pixel), cv2.resize of that 3-channel
+// 8-bit image to img_h x img_w with OpenCV's fixed-point INTER_LINEAR (11-bit weights c = rint(w * 2048); columns clamp the coordinate at
+// both borders, rows only their indices; vertical step ((b0 * (h0 >> 4)) >> 16) + ((b1 * (h1 >> 4)) >> 16) + 2) >> 2, saturated), then
+// addWeighted(grey3, 0.5, heat, 0.5, 0) with saliency_overlay_kernel's round-half-even blend.  The grey image is read once per pixel for
+// all K maps.  CTA = SOR_ROWS output rows of SOR_THREADS x 4 consecutive pixels; a row's weights are warp-uniform.  The table comes
+// from a global copy, 4 bytes per thread: read from constant memory, the divergent addresses serialise, and with many small CTAs that
+// load cost more than the colouring (64 images at 512 x 512, K = 2: 0.40 ms with one-row CTAs and the constant table, 0.21 ms so; one
+// B200 at a 1000 W limit).
+constexpr int SOR_THREADS = 64, SOR_ROWS = 4;
+__device__ __align__(4) uint8_t g_jet_bgr[256 * 3] = {
+#include "jet_lut.inc"
+};
+
+template <int K>
+__global__ void __launch_bounds__(SOR_THREADS * SOR_ROWS) saliency_overlay_resized_kernel(const uint8_t* __restrict__ g8,
+                                                                                          const float* __restrict__ sal, int H, int W,
+                                                                                          int hi, int wi, uint8_t* __restrict__ overlay,
+                                                                                          uint8_t* __restrict__ heat) {
+    __shared__ __align__(4) uint8_t s_lut[256 * 3];
+    const int tid = threadIdx.y * SOR_THREADS + threadIdx.x;
+    if (tid < 192) reinterpret_cast<uint32_t*>(s_lut)[tid] = __ldg(reinterpret_cast<const uint32_t*>(g_jet_bgr) + tid);
+    __syncthreads();
+    const int b = blockIdx.z, dy = blockIdx.y * SOR_ROWS + threadIdx.y, dx0 = (blockIdx.x * SOR_THREADS + threadIdx.x) * 4;
+    if (dx0 >= wi || dy >= hi) return;
+    int sy;
+    float fy;
+    cv_linear_coord(dy, H, hi, sy, fy);
+    const int b0 = __float2int_rn((1.f - fy) * 2048.f), b1 = __float2int_rn(fy * 2048.f);
+    const int y0 = min(max(sy, 0), H - 1), y1 = min(max(sy + 1, 0), H - 1);
+    int x0[4], x1[4], c0[4], c1[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+        int sx;
+        float fx;
+        cv_linear_coord(min(dx0 + j, wi - 1), W, wi, sx, fx);
+        if (sx < 0) { fx = 0.f; sx = 0; }
+        if (sx >= W - 1) { fx = 0.f; sx = W - 1; }
+        x0[j] = sx;
+        x1[j] = min(sx + 1, W - 1);
+        c0[j] = __float2int_rn((1.f - fx) * 2048.f);
+        c1[j] = __float2int_rn(fx * 2048.f);
+    }
+    const size_t hw = (size_t)hi * wi, px0 = (size_t)dy * wi + dx0;
+    const int npx = min(4, wi - dx0);
+    int g[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) g[j] = j < npx ? __ldg(g8 + (size_t)b * hw + px0 + j) : 0;
+    const bool vst = npx == 4 && (wi & 3) == 0 && ((reinterpret_cast<uintptr_t>(overlay) | reinterpret_cast<uintptr_t>(heat)) & 3) == 0;
+    auto lut_index = [](float v) { return 3 * (int)(uint8_t)(int)(v * 255.f); };
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+        const float* m = sal + ((size_t)b * K + k) * H * W;
+        const float* r0 = m + (size_t)y0 * W;
+        const float* r1 = m + (size_t)y1 * W;
+        uint8_t hv[12], ov[12];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const int i00 = lut_index(__ldg(r0 + x0[j])), i01 = lut_index(__ldg(r0 + x1[j]));
+            const int i10 = lut_index(__ldg(r1 + x0[j])), i11 = lut_index(__ldg(r1 + x1[j]));
+#pragma unroll
+            for (int ch = 0; ch < 3; ++ch) {
+                const int h0 = s_lut[i00 + ch] * c0[j] + s_lut[i01 + ch] * c1[j];
+                const int h1 = s_lut[i10 + ch] * c0[j] + s_lut[i11 + ch] * c1[j];
+                const int v = min(max((((b0 * (h0 >> 4)) >> 16) + ((b1 * (h1 >> 4)) >> 16) + 2) >> 2, 0), 255);
+                const int sum = g[j] + v, q = sum >> 1;
+                hv[3 * j + ch] = (uint8_t)v;
+                ov[3 * j + ch] = (uint8_t)(q + (sum & q & 1));
+            }
+        }
+        const size_t o = (((size_t)b * K + k) * hw + px0) * 3;
+        if (vst) {
+#pragma unroll
+            for (int w = 0; w < 3; ++w) {
+                if (heat) reinterpret_cast<uint32_t*>(heat + o)[w] = (uint32_t)hv[4 * w] | ((uint32_t)hv[4 * w + 1] << 8) |
+                                                                      ((uint32_t)hv[4 * w + 2] << 16) | ((uint32_t)hv[4 * w + 3] << 24);
+                if (overlay) reinterpret_cast<uint32_t*>(overlay + o)[w] = (uint32_t)ov[4 * w] | ((uint32_t)ov[4 * w + 1] << 8) |
+                                                                            ((uint32_t)ov[4 * w + 2] << 16) | ((uint32_t)ov[4 * w + 3] << 24);
+            }
+        } else {
+#pragma unroll
+            for (int q = 0; q < 12; ++q) {
+                if (q >= 3 * npx) break;
+                if (heat) heat[o + q] = hv[q];
+                if (overlay) overlay[o + q] = ov[q];
+            }
+        }
+    }
+}
+
+int launch_saliency_overlay_resized(const uint8_t* g8, const float* sal, int B, int K, int H, int W, int hi, int wi, uint8_t* overlay,
+                                    uint8_t* heat, cudaStream_t s) {
+    if (hi == H && wi == W) return launch_saliency_overlay(g8, 1, sal, B, K, H * W, overlay, heat, s);   // cv2.resize to the same size copies
+    const dim3 grid(cdiv(wi, 4 * SOR_THREADS), cdiv(hi, SOR_ROWS), B), block(SOR_THREADS, SOR_ROWS);
+    switch (K) {
+#define BCAD_SOR(k) case k: saliency_overlay_resized_kernel<k><<<grid, block, 0, s>>>(g8, sal, H, W, hi, wi, overlay, heat); break;
+        BCAD_SOR(1) BCAD_SOR(2) BCAD_SOR(3) BCAD_SOR(4) BCAD_SOR(5) BCAD_SOR(6) BCAD_SOR(7) BCAD_SOR(8)
+#undef BCAD_SOR
+        default: set_error("saliency_overlay_resized: K=%d out of range 1..%d", K, BCAD_MAX_EXPLAIN_CLASSES); return BCAD_ERR_INVALID;
+    }
+    BCAD_CUDA_CHECK(cudaGetLastError());
+    return BCAD_OK;
+}
+
 // =====================================================================================================
 // The dual-class overlay call for grey images of any size (bcad_gradcam_overlays_classes_host)
 // =====================================================================================================

@@ -1,5 +1,6 @@
 // Input-gradient saliency (explainability.py:44-78): the first conv block's input gradient, s = max_c |d_input| and its per-image
-// min-max normalisation, for bcad_predict_saliency_classes.  The overlay kernel sits beside overlay_kernel in kernels_fp32.cu.
+// min-max normalisation, for bcad_predict_saliency_classes.  The two colouring kernels (saliency_overlay_kernel at the model's size,
+// saliency_overlay_resized_kernel at the image's) sit beside overlay_kernel in kernels_fp32.cu, with the JET table they share.
 #include "common.cuh"
 #include "kernels.h"
 

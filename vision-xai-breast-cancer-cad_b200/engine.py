@@ -598,6 +598,56 @@ def _gradcam_overlays_classes_host(self, gray_u8: np.ndarray, classes=(0, 1), gr
 Engine.gradcam_overlays_classes_host = _gradcam_overlays_classes_host
 
 
+def _gray_batch(gray_u8) -> np.ndarray:
+    """uint8 grey images [B,H,W] or [H,W] -> a C-contiguous uint8 [B,H,W] array."""
+    g = np.ascontiguousarray(gray_u8)
+    if g.dtype != np.uint8:
+        raise ValueError("gray_u8 must be uint8 (0-255 grey levels)")
+    if g.ndim == 2:
+        g = g[None]
+    if g.ndim != 3:
+        raise ValueError(f"gray_u8 must be [B,H,W] or [H,W], got shape {g.shape}")
+    return g
+
+
+def _out_array(out, shape, dtype, name):
+    a = out if out is not None else np.empty(shape, dtype)
+    if a.dtype != dtype or a.shape != shape or not a.flags["C_CONTIGUOUS"]:
+        raise ValueError(f"{name} must be a C-contiguous {np.dtype(dtype).name} array of shape {shape}")
+    return a
+
+
+def _saliency_overlays_classes_host(self, gray_u8: np.ndarray, classes=(0, 1), grad_mode: str = "softmax_ce", standardise: bool = True,
+                                    overlay_out: Optional[np.ndarray] = None, heat_out: Optional[np.ndarray] = None,
+                                    saliency_out: Optional[np.ndarray] = None, want_overlay: bool = True, want_heat: bool = True,
+                                    want_saliency: bool = False):
+    """The dual-class input-gradient saliency overlays (explainability.py:81-108) for a batch, end to end through one C-ABI call
+    (bcad_saliency_overlays_classes_host): uint8 grey images [B,h,w] of ANY size -> (cls int32 [B], probs [B,nc], logits [B,nc],
+    overlays uint8 BGR [B,K,h,w,3], heat-maps uint8 BGR [B,K,h,w,3], saliency fp32 [B,K,H,W] at the model's size or None).  The CNN
+    sees the input ``gradcam_overlays_classes_host`` builds (cv2.resize(img / 255, model size), standardised per image when
+    ``standardise``); each map is coloured with JET, resized to the image's size as cv2.resize does on 8-bit BGR, and blended 50/50 with
+    the grey image.  ``classes`` as in ``gradcam_overlays_classes_host``; ``grad_mode`` defaults to the reference's softmax
+    cross-entropy gradient.  fp32 engines with ``keep_all_activations`` (a model's ``saliency_engine``).  The saliency maps are copied
+    back only when ``want_saliency`` or ``saliency_out`` is given.  Pinned host arrays make the copies asynchronous."""
+    self.cache_tag = None
+    g = _gray_batch(gray_u8)
+    B, h, w = g.shape
+    H, W, _ = self.spec.input_shape
+    nc = self.spec.num_classes
+    K, ci = _host_class_rows(classes, B, nc)
+    logits, probs, cls = np.empty((B, nc), np.float32), np.empty((B, nc), np.float32), np.empty((B,), np.int32)
+    ov = _out_array(overlay_out, (B, K, h, w, 3), np.uint8, "overlay_out") if want_overlay else None
+    hm = _out_array(heat_out, (B, K, h, w, 3), np.uint8, "heat_out") if want_heat else None
+    sal = _out_array(saliency_out, (B, K, H, W), np.float32, "saliency_out") if (want_saliency or saliency_out is not None) else None
+    _lib.check(self.lib.bcad_saliency_overlays_classes_host(self._h, _ptr(g), B, h, w, K, _ptr(ci), _lib.GRAD_MODE[grad_mode],
+                                                            1 if standardise else 0, _ptr(logits), _ptr(probs), _ptr(cls), _ptr(sal),
+                                                            _ptr(ov), _ptr(hm)))
+    return cls, probs, logits, ov, hm, sal
+
+
+Engine.saliency_overlays_classes_host = _saliency_overlays_classes_host
+
+
 def gradcam_tail(A: torch.Tensor, dA: torch.Tensor, out_hw: Tuple[int, int]) -> torch.Tensor:
     """Stand-alone Grad-CAM tail on NHWC CUDA tensors [B,h,w,K] (fp32 or bf16) -> fp32 [B,H,W]."""
     lib = _lib.load()
@@ -699,6 +749,28 @@ def saliency_overlay(base_u8, saliency: torch.Tensor):
     with torch.cuda.device(sal.device):
         _lib.check(lib.bcad_saliency_overlay(_ptr(base), int(base.shape[3]), _ptr(sal), B, K, H, W, _ptr(ov), _ptr(heat),
                                              C.c_void_p(torch.cuda.current_stream(sal.device).cuda_stream)))
+    return ov, heat
+
+
+def saliency_overlay_resized(gray_u8: torch.Tensor, saliency: torch.Tensor, want_overlay=True, want_heat=True):
+    """generate_saliency_overlay (explainability.py:74-77) at the image's size for [B,K] maps on CUDA tensors: ``gray_u8`` uint8 [B,h,w]
+    (the blend base, replicated to 3 channels, read once for the K maps), ``saliency`` fp32 [B,K,H,W] in [0,1] at any (model) size
+    -> (overlay u8 [B,K,h,w,3], heat-map u8 [B,K,h,w,3]), both BGR: heat = cv2.resize(applyColorMap(uint8(s * 255), JET), (w, h)) with
+    OpenCV's 8-bit INTER_LINEAR arithmetic, overlay = addWeighted(grey3, 0.5, heat, 0.5, 0)."""
+    lib = _lib.load()
+    g = gray_u8.contiguous()
+    sal = saliency.to(torch.float32).contiguous()
+    if sal.dim() != 4:
+        raise ValueError(f"saliency must be [B,K,H,W], got shape {tuple(sal.shape)}")
+    B, K, H, W = sal.shape
+    if g.dtype != torch.uint8 or g.dim() != 3 or g.shape[0] != B or g.device != sal.device:
+        raise ValueError(f"gray_u8 must be a uint8 [{B},h,w] tensor on the saliency maps' device")
+    h, w = g.shape[1:]
+    ov = torch.empty((B, K, h, w, 3), device=sal.device, dtype=torch.uint8) if want_overlay else None
+    heat = torch.empty((B, K, h, w, 3), device=sal.device, dtype=torch.uint8) if want_heat else None
+    with torch.cuda.device(sal.device):
+        _lib.check(lib.bcad_saliency_overlay_resized(_ptr(g), _ptr(sal), B, K, H, W, h, w, _ptr(ov), _ptr(heat),
+                                                     C.c_void_p(torch.cuda.current_stream(sal.device).cuda_stream)))
     return ov, heat
 
 
@@ -810,6 +882,55 @@ class ShardedEngine:
         if errs:
             raise errs[0]
         return cls, probs, logits, ov, hu
+
+    def set_fast_training(self, on: bool = True):
+        """Engine.set_fast_training on every GPU's engine (a model's ``saliency_engine`` has it on where the shape allows)."""
+        for e in self.engines:
+            e.set_fast_training(on)
+
+    def saliency_overlays_classes_host(self, gray_u8: np.ndarray, classes=(0, 1), grad_mode="softmax_ce", standardise=True,
+                                       want_saliency=False):
+        """Engine.saliency_overlays_classes_host over the GPUs of the box (fp32 engines with ``keep_all_activations``): contiguous
+        split, one host thread per GPU -> (cls, probs, logits, overlays [B,K,h,w,3], heat-maps [B,K,h,w,3], saliency [B,K,H,W] or
+        None).  The arrays are the driver's pinned buffers: they are overwritten by the next call of the same shape (copy what must
+        outlive it)."""
+        g = _gray_batch(gray_u8)
+        B, h, w = g.shape
+        H, W, _ = self.spec.input_shape
+        nc = self.spec.num_classes
+        K, ci = _host_class_rows(classes, B, nc)
+        key = ("saliency", B, K, h, w, bool(want_saliency))
+        if self._out is None or self._out[0] != key:
+            bufs = (torch.empty((B,), dtype=torch.int32).pin_memory(), torch.empty((B, nc), dtype=torch.float32).pin_memory(),
+                    torch.empty((B, nc), dtype=torch.float32).pin_memory(), torch.empty((B, K, h, w, 3), dtype=torch.uint8).pin_memory(),
+                    torch.empty((B, K, h, w, 3), dtype=torch.uint8).pin_memory())
+            if want_saliency:
+                bufs += (torch.empty((B, K, H, W), dtype=torch.float32).pin_memory(),)
+            self._out = (key, bufs)
+        cls, probs, logits, ov, hm, *rest = (t.numpy() for t in self._out[1])
+        sal = rest[0] if want_saliency else None
+        errs = []
+
+        def work(e, s, t):
+            try:
+                if t <= s:
+                    return
+                c, p, l, _, _, _ = e.saliency_overlays_classes_host(g[s:t], None if ci is None else ci[s:t], grad_mode, standardise,
+                                                                    overlay_out=ov[s:t], heat_out=hm[s:t],
+                                                                    saliency_out=None if sal is None else sal[s:t])
+                cls[s:t], probs[s:t], logits[s:t] = c, p, l
+            except Exception as ex:  # surfaced after join
+                errs.append(ex)
+
+        ths = [threading.Thread(target=work, args=(e, s, t))
+               for e, (s, t) in zip(self.engines, shard_bounds(B, len(self.engines)))]
+        for t in ths:
+            t.start()
+        for t in ths:
+            t.join()
+        if errs:
+            raise errs[0]
+        return cls, probs, logits, ov, hm, sal
 
     def close(self):
         for e in self.engines:

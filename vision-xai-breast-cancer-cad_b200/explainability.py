@@ -114,3 +114,21 @@ def generate_dual_class_overlays_batch(model, X, classes_to_test=[0, 1]):
     cls, probs, _, sal, _ = eng.predict_saliency_classes(X.astype(np.float32), list(classes_to_test), "softmax_ce")
     overlay, heat = _engine.saliency_overlay(torch.from_numpy(np.ascontiguousarray(base)), sal)
     return (cls.cpu().numpy().astype(np.int64), probs.cpu().numpy(), sal.cpu().numpy(), overlay.cpu().numpy(), heat.cpu().numpy())
+
+
+def generate_dual_class_saliency_overlays_batch(model, imgs_u8, classes_to_test=[0, 1], standardise=True, overlay_out=None, heat_out=None,
+                                                want_saliency=False):
+    """``generate_dual_class_overlays`` for a batch of 8-bit grey images of ANY size (the app's 512x512 mammograms), without the PNGs,
+    through ONE host-buffer C-ABI call (bcad_saliency_overlays_classes_host) on ``model.saliency_engine`` (either mirror).  The CNN sees
+    ``cv2.resize(img / 255, model size)``, standardised per image when ``standardise``; each class's saliency map is coloured with JET,
+    resized to the image's size and blended 50/50 with the grey image itself, as ``generate_saliency_overlay`` does for an image of that
+    size.  ``overlay_out`` / ``heat_out``: optional C-contiguous uint8 arrays to write into (pinned ones make the copies asynchronous).
+    -> (classes int64 [B], probs [B,nc], overlays uint8 [B,K,h,w,3], heatmaps uint8 [B,K,h,w,3], saliency float32 [B,K,H,W] at the
+    model's size when ``want_saliency``, else None); overlays and heat-maps are BGR, as cv2 returns them."""
+    g = np.asarray(imgs_u8)
+    if g.dtype != np.uint8:
+        raise ValueError("imgs_u8 must be uint8 (0-255 grey levels)")
+    eng = model.saliency_engine
+    cls, probs, _, ov, hm, sal = eng.saliency_overlays_classes_host(g, list(classes_to_test), "softmax_ce", standardise, overlay_out,
+                                                                    heat_out, want_saliency=want_saliency)
+    return cls.astype(np.int64), probs, ov, hm, sal
