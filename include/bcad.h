@@ -350,7 +350,9 @@ BCAD_API int bcad_get_conv_weights(bcad_model* m, int conv_idx, float* filters_f
 BCAD_API int bcad_get_dense_weights(bcad_model* m, int dense_idx, float* w_units_in_host, float* bias_host);
 
 /* ---- introspection ---------------------------------------------------------------------------- */
-/* Grad-CAM target tensor for the following explain calls of this handle (BCAD_TARGET_*; fp32 path only for CONV_PREACT) */
+/* Grad-CAM target tensor for the following explain calls of this handle (BCAD_TARGET_*), passed on to the refinement twin.  CONV_PREACT
+ * needs alpha_conv > 0; on the tensor paths with first-index pooling also a first dense layer of a multiple of 64 units (<= 256) --
+ * other shapes keep it on the fp32 path (BCAD_ERR_INVALID) */
 BCAD_API int bcad_set_explain_target(bcad_model* m, int target);
 /* refinement counters since creation (cfg.refine_margin > 0): images re-run at fp32 grade, flagged images that did not fit
  * cfg.refine_capacity (kept their 16-bit result).  Synchronises the device.  Both 0 when refinement is off. */

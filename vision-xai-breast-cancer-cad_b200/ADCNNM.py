@@ -178,11 +178,23 @@ class CNNModel(nn.Module):
             eng.set_explain_target("conv")
         return cls.long(), logits, heat
 
-    def predict_explain_classes_batch(self, x, classes=(0, 1), grad_mode="logit"):
+    def predict_explain_classes_batch(self, x, classes=(0, 1), grad_mode="logit", target="conv"):
         """Grad-CAM for several target classes per image from one forward (the dual-class call of app.py:649-657)
         -> (classes [B], logits [B,nc], heatmaps fp32 [B,K,H,W]) on the GPU.  ``classes``: a length-K sequence shared by the batch,
-        a [B,K] array, or None = every class; ``heat[:, k]`` equals ``predict_explain_batch(x, classes[:, k])``'s heat-maps."""
-        cls, probs, logits, heat = self.engine.predict_explain_classes(x, classes, grad_mode)
+        a [B,K] array, or None = every class; ``heat[:, k]`` equals ``predict_explain_batch(x, classes[:, k])``'s heat-maps.
+        ``target="conv_preact"``: the ``nn.Conv2d`` module's own output (what pytorch_grad_cam hooks), on the same handle as the default
+        target, which is restored afterwards."""
+        if target not in ("conv", "conv_preact"):
+            raise ValueError(f"unknown target {target!r} (conv | conv_preact)")
+        eng = self.engine
+        if target == "conv":
+            cls, probs, logits, heat = eng.predict_explain_classes(x, classes, grad_mode)
+            return cls.long(), logits, heat
+        eng.set_explain_target(target)
+        try:
+            cls, probs, logits, heat = eng.predict_explain_classes(x, classes, grad_mode)
+        finally:
+            eng.set_explain_target("conv")
         return cls.long(), logits, heat
 
     def predict_saliency_classes_batch(self, x, classes=(0, 1), grad_mode="logit"):

@@ -87,13 +87,15 @@ def generate_gradcam_overlays_batch(imgs_u8, class_idx=None, model=None, standar
 
 
 def generate_dual_class_gradcam_overlays_batch(imgs_u8, classes_to_test=[0, 1], model=None, standardise=True, overlay_out=None,
-                                               heat_out=None):
+                                               heat_out=None, target="conv"):
     """The batched form of the deployed dual-class call (app.py:649-657 -> GRADCAM.py:31-81): 8-bit grey images [B,H,W] of any size
     (the CNN sees ``cv2.resize(img / 255, model size)``, the maps have the image's size, as in the single-image call above), ONE
     forward per image for all of ``classes_to_test`` (K <= 8), through ONE host-buffer C-ABI call (bcad_gradcam_overlays_classes_host),
     no PNGs.  ``overlay_out`` / ``heat_out``: optional C-contiguous uint8 arrays to write into (pinned ones make the copies asynchronous).
     -> (classes int64 [B], probs [B,nc], overlays uint8 [B,K,H,W,3], heatmaps uint8 [B,K,H,W]); at the model's input size ``[:, k]`` is
-    byte for byte what ``generate_gradcam_overlays_batch(imgs_u8, class_idx=classes_to_test[k])`` returns."""
+    byte for byte what ``generate_gradcam_overlays_batch(imgs_u8, class_idx=classes_to_test[k])`` returns.  ``target="conv_preact"``:
+    maps of the conv module's output before its activation (what pytorch_grad_cam hooks on the torch model), set on the engine for this
+    call only."""
     mdl = model if model is not None else globals()["model"]
     if mdl is None:
         raise RuntimeError("GRADCAM.model is not set: assign a CNNModel (bcad_b200.CNNModel / ADCNNM) first")
@@ -101,5 +103,14 @@ def generate_dual_class_gradcam_overlays_batch(imgs_u8, classes_to_test=[0, 1], 
     g = np.asarray(imgs_u8)
     if g.dtype != np.uint8:
         raise ValueError("imgs_u8 must be uint8 (0-255 grey levels)")
-    cls, probs, _, ov, hu = eng.gradcam_overlays_classes_host(g, list(classes_to_test), "logit", standardise, overlay_out, heat_out)
+    if target not in ("conv", "conv_preact"):
+        raise ValueError(f"unknown target {target!r} (conv | conv_preact)")
+    if target == "conv":
+        cls, probs, _, ov, hu = eng.gradcam_overlays_classes_host(g, list(classes_to_test), "logit", standardise, overlay_out, heat_out)
+        return cls.astype(np.int64), probs, ov, hu
+    eng.set_explain_target(target)
+    try:
+        cls, probs, _, ov, hu = eng.gradcam_overlays_classes_host(g, list(classes_to_test), "logit", standardise, overlay_out, heat_out)
+    finally:
+        eng.set_explain_target("conv")
     return cls.astype(np.int64), probs, ov, hu

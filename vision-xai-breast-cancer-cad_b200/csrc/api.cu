@@ -1476,12 +1476,16 @@ int bcad_set_explain_target(bcad_model* mm, int target) {
     BCAD_REQUIRE(m, "null model");
     BCAD_REQUIRE(target == BCAD_TARGET_CONV_ACT || target == BCAD_TARGET_CONV_PREACT, "bad explain target %d", target);
     if (target == BCAD_TARGET_CONV_PREACT) {
-        BCAD_REQUIRE(!m->tensor_path, "the pre-activation target needs the dense pooled gradient, which only the fp32 path forms: create the model "
-                                      "with BCAD_PREC_FP32 (the tensor paths derive the channel weights from dz1 and never build it)");
-        BCAD_REQUIRE(m->cfg.alpha_conv > 0.f, "the pre-activation map is recovered from the stored post-LeakyReLU map: needs alpha_conv > 0");
+        BCAD_REQUIRE(m->cfg.alpha_conv > 0.f, "the pre-activation map is recovered from the stored post-LeakyReLU map: needs alpha_conv > 0, "
+                                              "on the tensor paths as on the fp32 path");
+        if (m->tensor_path) BCAD_TRY(tensor_preact_supported(*m));
     }
-    std::lock_guard<std::mutex> lock(m->mu);
-    m->target = target;
+    {
+        std::lock_guard<std::mutex> lock(m->mu);
+        m->target = target;
+    }
+    // the refinement twin re-runs small-margin images inside this handle's calls: it explains the same target
+    if (m->refine.twin) return bcad_set_explain_target(reinterpret_cast<bcad_model*>(m->refine.twin), target);
     return BCAD_OK;
 }
 

@@ -80,5 +80,9 @@ __device__ __forceinline__ uint32_t pack_f16(float lo, float hi) {
 __device__ __forceinline__ float2 unpack_f16(uint32_t v) {
     return __half22float2(*reinterpret_cast<const __half2*>(&v));
 }
+// undo a LeakyReLU (pre-activation Grad-CAM target): z = a > 0 ? a : a * inv_slope, the fp32 cam_kernel's form
+__device__ __forceinline__ float2 unleaky2(float2 v, float inv_slope) {
+    return make_float2(v.x > 0.f ? v.x : v.x * inv_slope, v.y > 0.f ? v.y : v.y * inv_slope);
+}
 
 }  // namespace bcad

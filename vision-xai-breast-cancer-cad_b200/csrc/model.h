@@ -189,6 +189,7 @@ int relaunch_fused_head(Model* m, const int32_t* class_idx, float* alpha_raw, cu
 
 // ---- tensor (tcgen05) path, tensor_path.cu
 int tensor_path_supported(const Model& m);          // BCAD_OK or BCAD_ERR_INVALID (+ message)
+int tensor_preact_supported(const Model& m);        // the pre-activation Grad-CAM target on this tensor-path handle
 int tensor_path_commit(Model& m);
 int tensor_forward_chunk(Model& m, const float* x, int n, bool explain, const int32_t* class_idx, int grad_mode, cudaStream_t s);
 // K target classes: class column k at class_idx + k * col_ld, the map of class k of image b at heat + b * heat_stride + k * H * W

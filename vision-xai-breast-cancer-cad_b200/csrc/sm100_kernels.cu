@@ -935,6 +935,241 @@ int launch_fc_splitk(const FcArgs& a, cudaStream_t s) {
     return BCAD_OK;
 }
 
+// =====================================================================================================
+// Grad-CAM channel weights of the PRE-activation target (the nn.Conv2d output that a hook on the reference torch CNN's last conv
+// captures, ADCNNM.py:76) under first-index pooling, without the dense pooled gradient:
+//   alpha_raw[b][k] = sum_q g[b][q][k] * (P[b][q][k] > 0 ? 1 : slope),     g[b][q][k] = sum_u dz1[b][u] W1[u][(q, k)]
+// (only the window's first maximum receives g; LeakyReLU is monotone, so that element's z has the sign of the pooled P).
+//   GEMM on tcgen05: M = 128 images, N = the 64 channels of one pooled pixel q, K = units.  A = dz1 tiles, resident for the CTA;
+//   B = the fc1 forward tile of q ([unit][64 channels x 2 B], SW128) read MN-major -- no second copy of W1.
+//   Epilogue: LeakyReLU' of each column from the pooled map (the fc1 A tiles: one 128-byte row per image and q), accumulated per
+//   (image, channel) in registers over the CTA's range of q; partials [split][m_pad][64] -> alpha_preact_reduce (fixed order).
+//   dz1 rows arrive scaled by 2^e and split into fp16 hi + lo parts (dz_rows_to_tiles): full precision whatever the gradient's
+//   magnitude; the reduce undoes the scale exactly.  fp16: A_hi.W + A_lo.W (the W1 rounding the forward has is the only operand error);
+//   fp16x3: A_hi.W_hi + A_lo.W_hi + A_hi.W_lo, the mask sign from hi + lo.
+// Warp roles: 0 = bulk-copy producer, 1 = MMA issuer, 2..5 = epilogue (TMEM lane quadrant = warp % 4).
+// =====================================================================================================
+constexpr int PA_THREADS = 192;
+constexpr int PA_ACC = 4;             // TMEM accumulator buffers of 64 columns: the epilogue of q overlaps the MMAs of q + 1 .. q + 3
+constexpr int PA_MAXST = 4;           // W-tile ring stages (fewer when the resident dz1 tiles leave no room)
+
+static int pa_nst(int units) {
+    const int a_bytes = (units / 64) * 2 * 16384, w_bytes = units * 128;
+    return std::min(PA_MAXST, (227 * 1024 - a_bytes - 256) / w_bytes);
+}
+
+__global__ void __launch_bounds__(PA_THREADS, 1) alpha_preact_kernel(PreactArgs a) {
+    if (a.n_dev != nullptr && *a.n_dev <= 0) return;
+    extern __shared__ __align__(1024) uint8_t smem[];
+    const int parts = a.x3 ? 2 : 1;
+    const int nkb = a.units / 64;
+    const int a_bytes = nkb * 2 * 16384;           // resident dz1 tiles [kb][hi | lo][128 rows][128 B]
+    const int w_bytes = a.units * 128;             // one W tile (q, part): [unit][64 channels]
+    uint8_t* s_a = smem;
+    uint8_t* s_w = smem + a_bytes;
+    uint64_t* bars = reinterpret_cast<uint64_t*>(s_w + a.nst * w_bytes);
+    uint64_t* full = bars;                         // [PA_MAXST] producer -> MMA
+    uint64_t* empty = bars + PA_MAXST;             // [PA_MAXST] MMA -> producer
+    uint64_t* tfull = bars + 2 * PA_MAXST;         // [PA_ACC] MMA -> epilogue
+    uint64_t* tempty = tfull + PA_ACC;             // [PA_ACC] epilogue -> MMA (4 warps)
+    uint64_t* abar = tempty + PA_ACC;              // resident A landed
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(abar + 1);
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    if (tid == 0) {
+        for (int i = 0; i < PA_MAXST; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
+        for (int i = 0; i < PA_ACC; ++i) { mbar_init(&tfull[i], 1); mbar_init(&tempty[i], 4); }
+        mbar_init(abar, 1);
+        fence_barrier_init();
+    }
+    if (warp == 0) {
+        tmem_alloc(tmem_slot, 64 * PA_ACC);
+        tmem_relinquish();
+    }
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tmem = *tmem_slot;
+    const int mt = blockIdx.x, split = blockIdx.y;
+    const int q0 = split * a.q_per_split, q1 = min(a.npix, q0 + a.q_per_split);
+    const int nq = max(0, q1 - q0);
+
+    if (warp == 0) {
+        if (lane == 0) {
+            mbar_arrive_expect_tx(abar, a_bytes);
+            for (int off = 0; off < a_bytes; off += 16384)
+                bulk_g2s(s_a + off, a.dz_tiles + (size_t)mt * a_bytes + off, 16384, abar);
+            for (int i = 0; i < nq * parts; ++i) {
+                const int st = i % a.nst, q = q0 + i / parts, p = i % parts;
+                if (i >= a.nst) mbar_wait(&empty[st], ((i / a.nst) - 1) & 1);
+                mbar_arrive_expect_tx(&full[st], w_bytes);
+                const uint8_t* src = a.w_tiles + ((size_t)q * parts + p) * w_bytes;
+                for (int off = 0; off < w_bytes; off += 16384)
+                    bulk_g2s(s_w + st * w_bytes + off, src + off, min(16384, w_bytes - off), &full[st]);
+            }
+        }
+    } else if (warp == 1) {
+        if (lane == 0) {
+            // B MN-major (bit 16): the 64 channels of a unit are contiguous; SW128 atoms of 8 units x 128 B, SBO = 1024 B between them
+            constexpr uint32_t idesc = (1u << 4) | (1u << 16) | ((uint32_t)(64 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+            const uint32_t sa = smem_u32(s_a);
+            mbar_wait(abar, 0);
+            for (int iq = 0; iq < nq; ++iq) {
+                const int j = iq % PA_ACC;
+                if (iq >= PA_ACC) mbar_wait(&tempty[j], ((iq / PA_ACC) - 1) & 1);
+                tc_fence_after();
+                uint32_t acc = 0;
+                for (int p = 0; p < parts; ++p) {
+                    const int i = iq * parts + p, st = i % a.nst;
+                    mbar_wait(&full[st], (i / a.nst) & 1);
+                    tc_fence_after();
+                    const uint32_t sw = smem_u32(s_w + st * w_bytes);
+                    const int na = (p == 0) ? 2 : 1;               // W (W_hi) meets A_hi and A_lo, W_lo meets A_hi
+                    for (int ap = 0; ap < na; ++ap)
+                        for (int kb = 0; kb < nkb; ++kb)
+#pragma unroll
+                            for (int k = 0; k < 4; ++k) {
+                                const uint64_t ad = make_smem_desc(sa + (kb * 2 + ap) * 16384 + k * 32, 16, 1024, LAYOUT_SW128);
+                                const uint64_t bd = make_smem_desc(sw + kb * 8192 + k * 2048, 8192, 1024, LAYOUT_SW128);
+                                umma_bf16(tmem + j * 64, ad, bd, idesc, acc);
+                                acc = 1u;
+                            }
+                    umma_commit(&empty[st]);
+                }
+                umma_commit(&tfull[j]);
+            }
+        }
+    } else {
+        const int quad = warp & 3, row = quad * 32 + lane, sw = row & 7;
+        const uint32_t lane_off = (uint32_t)(quad * 32) << 16;
+        float acc[64];
+#pragma unroll
+        for (int c = 0; c < 64; ++c) acc[c] = 0.f;
+        const uint8_t* mrow = a.mask_tiles + (size_t)mt * a.npix * parts * 16384 + (size_t)row * 128;
+        for (int iq = 0; iq < nq; ++iq) {
+            const int j = iq % PA_ACC;
+            // LeakyReLU' of each channel at the window's maximum: bit c set <=> P > 0 (factor 1), else the slope
+            const uint4* mh = reinterpret_cast<const uint4*>(mrow + (size_t)(q0 + iq) * parts * 16384);
+            uint32_t pos0 = 0, pos1 = 0;
+#pragma unroll
+            for (int c = 0; c < 8; ++c) {
+                const uint4 h = ldg_stream_u4(mh + (c ^ sw));
+                float2 f[4] = {unpack_f16(h.x), unpack_f16(h.y), unpack_f16(h.z), unpack_f16(h.w)};
+                if (a.x3) {
+                    const uint4 l = ldg_stream_u4(mh + 1024 + (c ^ sw));               // the lo tile, 16 KB further
+                    const float2 g[4] = {unpack_f16(l.x), unpack_f16(l.y), unpack_f16(l.z), unpack_f16(l.w)};
+#pragma unroll
+                    for (int e = 0; e < 4; ++e) { f[e].x += g[e].x; f[e].y += g[e].y; }
+                }
+                uint32_t bits = 0;
+#pragma unroll
+                for (int e = 0; e < 4; ++e) bits |= ((f[e].x > 0.f) ? 1u : 0u) << (2 * e) | ((f[e].y > 0.f) ? 1u : 0u) << (2 * e + 1);
+                if (c < 4) pos0 |= bits << (8 * c);
+                else pos1 |= bits << (8 * (c - 4));
+            }
+            mbar_wait(&tfull[j], (iq / PA_ACC) & 1);
+            tc_fence_after();
+#pragma unroll
+            for (int h = 0; h < 2; ++h) {
+                float d[32];
+                tmem_ld32(tmem + lane_off + j * 64 + h * 32, d);
+                tmem_ld_wait();
+                const uint32_t pos = h ? pos1 : pos0;
+#pragma unroll
+                for (int c = 0; c < 32; ++c) acc[h * 32 + c] = fmaf(d[c], ((pos >> c) & 1u) ? 1.f : a.slope, acc[h * 32 + c]);
+            }
+            tc_fence_before();
+            __syncwarp();
+            if (lane == 0) mbar_arrive(&tempty[j]);
+        }
+        float4* dst = reinterpret_cast<float4*>(a.partials + ((size_t)split * a.m_pad + (size_t)mt * 128 + row) * 64);
+#pragma unroll
+        for (int c = 0; c < 16; ++c) dst[c] = make_float4(acc[4 * c], acc[4 * c + 1], acc[4 * c + 2], acc[4 * c + 3]);
+    }
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 0) tmem_dealloc(tmem, 64 * PA_ACC);
+}
+
+// alpha_raw[b][k] = 2^-e[b] * sum_s partial[s][b][k], splits in order
+__global__ void alpha_preact_reduce_kernel(const float* __restrict__ part, int splits, size_t ld_split, const int* __restrict__ row_exp,
+                                           float* __restrict__ alpha_raw, int n) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n * 64) return;
+    float v = 0.f;
+    for (int s = 0; s < splits; ++s) v += part[(size_t)s * ld_split + i];
+    alpha_raw[i] = ldexpf(v, -row_exp[i / 64]);
+}
+
+bool alpha_preact_supported(int units, int C) { return C == 64 && units % 64 == 0 && units <= 256 && pa_nst(units) >= 2; }
+
+int launch_alpha_preact(const PreactArgs& a0, int m_tiles, int splits, cudaStream_t s) {
+    BCAD_REQUIRE(alpha_preact_supported(a0.units, 64), "alpha_preact: %d units (a multiple of 64 up to 256)", a0.units);
+    PreactArgs a = a0;
+    a.nst = pa_nst(a.units);
+    const int smem = (a.units / 64) * 2 * 16384 + a.nst * a.units * 128 + 256;
+    BCAD_CUDA_CHECK(cudaFuncSetAttribute(alpha_preact_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    alpha_preact_kernel<<<dim3(m_tiles, splits), PA_THREADS, smem, s>>>(a);
+    BCAD_CUDA_CHECK(cudaGetLastError());
+    return BCAD_OK;
+}
+
+int launch_alpha_preact_reduce(const float* part, int splits, int m_pad, const int* row_exp, float* alpha_raw, int n, cudaStream_t s) {
+    alpha_preact_reduce_kernel<<<cdiv(n * 64, 256), 256, 0, s>>>(part, splits, (size_t)m_pad * 64, row_exp, alpha_raw, n);
+    BCAD_CUDA_CHECK(cudaGetLastError());
+    return BCAD_OK;
+}
+
+// dz1 rows [B][K] -> split fp16 SW128 A tiles as rows_to_fc_tiles_x3, each row first scaled by 2^e (exact; e -> row_exp) so that
+// its largest magnitude lies in [2^14, 2^15): the hi part then carries 11 significant bits of the row's large elements for any
+// gradient scale (a softmax gradient of a confident image can sit far below fp16's normal range).  One warp per row.
+__global__ void __launch_bounds__(256) dz_rows_to_tiles_kernel(const float* __restrict__ src, uint8_t* __restrict__ tiles,
+                                                               int* __restrict__ row_exp, int B, int K, int m_pad) {
+    const int row = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (row >= m_pad) return;
+    const int nkb = K / 64, items = nkb * 8;
+    float mx = 0.f;
+    for (int i = lane; i < items && row < B; i += 32) {
+        const float4* p = reinterpret_cast<const float4*>(src + (size_t)row * K + i * 8);
+        const float4 v0 = p[0], v1 = p[1];
+        mx = fmaxf(mx, fmaxf(fmaxf(fmaxf(fabsf(v0.x), fabsf(v0.y)), fmaxf(fabsf(v0.z), fabsf(v0.w))),
+                             fmaxf(fmaxf(fabsf(v1.x), fabsf(v1.y)), fmaxf(fabsf(v1.z), fabsf(v1.w)))));
+    }
+    mx = warp_max(mx);
+    int e = 0;
+    if (mx > 0.f && mx <= 3.4e38f) {
+        int E;
+        frexpf(mx, &E);
+        e = 15 - E;
+    }
+    if (lane == 0) row_exp[row] = e;
+    const int rr = row & 127;
+    for (int i = lane; i < items; i += 32) {
+        const int kb = i >> 3, ch = i & 7;
+        float v[8];
+#pragma unroll
+        for (int q = 0; q < 8; ++q) v[q] = (row < B) ? ldexpf(src[(size_t)row * K + i * 8 + q], e) : 0.f;
+        uint32_t hi[4], lo[4];
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            const __half2 h = __floats2half2_rn(v[2 * q], v[2 * q + 1]);
+            const float2 f = __half22float2(h);
+            hi[q] = h2u(h);
+            lo[q] = pack_f16(v[2 * q] - f.x, v[2 * q + 1] - f.y);
+        }
+        uint8_t* tile = tiles + (((size_t)(row >> 7) * nkb + kb) * 2) * (128 * 128);
+        const int swz = (ch ^ (rr & 7)) * 16;
+        *reinterpret_cast<uint4*>(tile + rr * 128 + swz) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+        *reinterpret_cast<uint4*>(tile + 128 * 128 + rr * 128 + swz) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+    }
+}
+
+int launch_dz_rows_to_tiles(const float* src, uint8_t* tiles, int* row_exp, int B, int K, int m_pad, cudaStream_t s) {
+    BCAD_REQUIRE(K % 64 == 0 && m_pad % 128 == 0, "dz_rows_to_tiles: K=%d m_pad=%d", K, m_pad);
+    dz_rows_to_tiles_kernel<<<m_pad / 8, 256, 0, s>>>(src, tiles, row_exp, B, K, m_pad);
+    BCAD_CUDA_CHECK(cudaGetLastError());
+    return BCAD_OK;
+}
+
 // fp32 rows [B][K] (K % 64 == 0) -> split fp16 SW128 A tiles [b/128][K/64][(hi|lo)][128][128 B]; rows >= B are zero
 __global__ void rows_to_fc_tiles_x3_kernel(const float* __restrict__ src, uint8_t* __restrict__ tiles, int B, int K, int m_pad) {
     const int nkb = K / 64;
@@ -997,11 +1232,11 @@ int launch_fc_reduce(const float* part, int splits, size_t ld_split, const float
 // Grad-CAM channel reduction on C8-planar fp16 activations: cam = ReLU(sum_k alpha_k A_k) + min/max partials
 // grid (splits, B), 256 threads, thread = pixel; every load is a coalesced 16 B per lane.
 // =====================================================================================================
-template <bool X3>
+template <bool X3, bool PRE>
 __global__ void __launch_bounds__(256)
 cam_c8_kernel(const __half* __restrict__ A, const float* __restrict__ alpha_raw, float scale,
               float* __restrict__ alpha_out, float* __restrict__ cam_lo, float* __restrict__ mm, int h, int w, int C,
-              const int* __restrict__ n_dev) {
+              const int* __restrict__ n_dev, float inv_slope) {
     extern __shared__ float s_alpha[];
     __shared__ float s_min[8], s_max[8];
     const int b = blockIdx.y, split = blockIdx.x, splits = gridDim.x;
@@ -1032,6 +1267,7 @@ cam_c8_kernel(const __half* __restrict__ A, const float* __restrict__ alpha_raw,
                 const float2 g0 = unpack_f16(ql.x), g1 = unpack_f16(ql.y), g2 = unpack_f16(ql.z), g3 = unpack_f16(ql.w);
                 f0.x += g0.x; f0.y += g0.y; f1.x += g1.x; f1.y += g1.y; f2.x += g2.x; f2.y += g2.y; f3.x += g3.x; f3.y += g3.y;
             }
+            if constexpr (PRE) { f0 = unleaky2(f0, inv_slope); f1 = unleaky2(f1, inv_slope); f2 = unleaky2(f2, inv_slope); f3 = unleaky2(f3, inv_slope); }
             acc = fmaf(f0.x, al[0], acc); acc = fmaf(f0.y, al[1], acc);
             acc = fmaf(f1.x, al[2], acc); acc = fmaf(f1.y, al[3], acc);
             acc = fmaf(f2.x, al[4], acc); acc = fmaf(f2.y, al[5], acc);
@@ -1054,10 +1290,14 @@ cam_c8_kernel(const __half* __restrict__ A, const float* __restrict__ alpha_raw,
 }
 
 int launch_cam_c8(const __half* A, const float* alpha_raw, float scale, float* alpha_out, float* cam_lo, float* mm,
-                  int B, int h, int w, int C, int splits, bool x3, cudaStream_t s, const int* n_dev) {
+                  int B, int h, int w, int C, int splits, bool x3, cudaStream_t s, const int* n_dev, float inv_slope) {
     dim3 grid(splits, B);
-    if (x3) cam_c8_kernel<true><<<grid, 256, C * sizeof(float), s>>>(A, alpha_raw, scale, alpha_out, cam_lo, mm, h, w, C, n_dev);
-    else cam_c8_kernel<false><<<grid, 256, C * sizeof(float), s>>>(A, alpha_raw, scale, alpha_out, cam_lo, mm, h, w, C, n_dev);
+    const size_t sm = C * sizeof(float);
+    const bool pre = inv_slope > 0.f;
+    if (x3 && pre) cam_c8_kernel<true, true><<<grid, 256, sm, s>>>(A, alpha_raw, scale, alpha_out, cam_lo, mm, h, w, C, n_dev, inv_slope);
+    else if (x3) cam_c8_kernel<true, false><<<grid, 256, sm, s>>>(A, alpha_raw, scale, alpha_out, cam_lo, mm, h, w, C, n_dev, 0.f);
+    else if (pre) cam_c8_kernel<false, true><<<grid, 256, sm, s>>>(A, alpha_raw, scale, alpha_out, cam_lo, mm, h, w, C, n_dev, inv_slope);
+    else cam_c8_kernel<false, false><<<grid, 256, sm, s>>>(A, alpha_raw, scale, alpha_out, cam_lo, mm, h, w, C, n_dev, 0.f);
     BCAD_CUDA_CHECK(cudaGetLastError());
     return BCAD_OK;
 }
@@ -1068,7 +1308,7 @@ int launch_cam_c8(const __half* A, const float* alpha_raw, float scale, float* a
 // gradient [B][Hp][Wp][C].  One CTA per image, warp = channel octet (C = 64: 8 warps), lanes across windows; the activation value
 // is hi + lo in fp32 -- the same number c8_to_nhwc_kernel reports, so the equality structure is the one the tests see.
 __global__ void __launch_bounds__(256) alpha_ties_c8_kernel(const __half* __restrict__ A, const float* __restrict__ g,
-                                                            float* __restrict__ alpha_raw, int h, int w, int C) {
+                                                            float* __restrict__ alpha_raw, int h, int w, int C, float pre_slope) {
     const int octets = C / 8, planes = 2 * octets;
     const int Hp = h / 2, Wp = w / 2;
     const int b = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
@@ -1100,7 +1340,9 @@ __global__ void __launch_bounds__(256) alpha_ties_c8_kernel(const __half* __rest
                 for (int j = 0; j < 8; ++j) {
                     const float m = fmaxf(fmaxf(v[0][j], v[1][j]), fmaxf(v[2][j], v[3][j]));
                     const int cnt = (v[0][j] == m) + (v[1][j] == m) + (v[2][j] == m) + (v[3][j] == m);
-                    acc[j] = fmaf(gv[j], (float)cnt, acc[j]);
+                    float f = (float)cnt;
+                    if (pre_slope >= 0.f && !(m > 0.f)) f *= pre_slope;       // every tie holds the window's value: one LeakyReLU'
+                    acc[j] = fmaf(gv[j], f, acc[j]);
                 }
             }
 #pragma unroll
@@ -1111,9 +1353,9 @@ __global__ void __launch_bounds__(256) alpha_ties_c8_kernel(const __half* __rest
     }
 }
 
-int launch_alpha_ties_c8(const __half* A, const float* g, float* alpha_raw, int B, int h, int w, int C, cudaStream_t s) {
+int launch_alpha_ties_c8(const __half* A, const float* g, float* alpha_raw, int B, int h, int w, int C, cudaStream_t s, float pre_slope) {
     BCAD_REQUIRE(C % 8 == 0, "alpha_ties_c8: channel count %d", C);
-    alpha_ties_c8_kernel<<<B, 256, 0, s>>>(A, g, alpha_raw, h, w, C);
+    alpha_ties_c8_kernel<<<B, 256, 0, s>>>(A, g, alpha_raw, h, w, C, pre_slope);
     BCAD_CUDA_CHECK(cudaGetLastError());
     return BCAD_OK;
 }

@@ -89,24 +89,49 @@ struct FcArgs {
 // dz1 fp32 [B][K] -> fp16x3 A tiles [b/128][K/64][(hi|lo)][128][128 B, chunks XOR (row&7)] for the fc1 input-gradient GEMM
 int launch_rows_to_fc_tiles_x3(const float* src, uint8_t* tiles, int B, int K, int m_pad, cudaStream_t s);
 int launch_fc_splitk(const FcArgs& a, cudaStream_t s);
+
+// Grad-CAM weights of the pre-activation target, first-index pooling (profiling name alpha_preact_tcgen05):
+//   alpha_raw[b][k] = sum_q (sum_u dz1[b][u] W1[u][(q, k)]) * (P[b][q][k] > 0 ? 1 : slope)   for C = 64 channels
+struct PreactArgs {
+    const uint8_t* dz_tiles;      // dz1 as launch_dz_rows_to_tiles leaves it: [b/128][units/64][hi|lo][128][128 B] SW128, rows scaled by 2^e
+    const uint8_t* w_tiles;       // the fc1 forward tiles [q][hi (| lo)][unit][128 B] SW128
+    const uint8_t* mask_tiles;    // the fc1 A tiles of the pooled map [b/128][q][hi (| lo)][128][128 B]
+    float* partials;              // [splits][m_pad][64]
+    int units, npix, q_per_split, m_pad;
+    int x3;                       // fp16x3: split operands, sign of the pooled value from hi + lo
+    float slope;                  // LeakyReLU slope of the conv block
+    int nst;                      // (set by the launcher)
+    const int* n_dev = nullptr;
+};
+bool alpha_preact_supported(int units, int C);
+// GEMM + masked epilogue, grid m_tiles x splits (split s covers pooled pixels [s * q_per_split, +q_per_split))
+int launch_alpha_preact(const PreactArgs& a, int m_tiles, int splits, cudaStream_t s);
+// alpha_raw [n][64] = the splits' partials summed in order, times 2^-row_exp[b]
+int launch_alpha_preact_reduce(const float* part, int splits, int m_pad, const int* row_exp, float* alpha_raw, int n, cudaStream_t s);
+// fp32 rows [B][K] -> split fp16 A tiles like launch_rows_to_fc_tiles_x3, each row scaled by 2^row_exp[row] (max |.| in [2^14, 2^15))
+int launch_dz_rows_to_tiles(const float* src, uint8_t* tiles, int* row_exp, int B, int K, int m_pad, cudaStream_t s);
 int launch_fc_reduce(const float* part, int splits, size_t ld_split, const float* bias, float* z, float* h, float alpha,
                      int M, int N, cudaStream_t s);
 
+// inv_slope > 0 (all three tails): A holds post-LeakyReLU values and the target is the pre-activation map, z = a > 0 ? a : a * inv_slope
+// (a separate instantiation: the post-activation kernels are unchanged)
 int launch_cam_c8(const __half* A, const float* alpha_raw, float scale, float* alpha_out, float* cam_lo, float* mm,
-                  int B, int h, int w, int C, int splits, bool x3, cudaStream_t s, const int* n_dev = nullptr);
+                  int B, int h, int w, int C, int splits, bool x3, cudaStream_t s, const int* n_dev = nullptr, float inv_slope = 0.f);
 // fused tail (sm100_tail.cu): cam + min-max + bilinear + min-max, a 2-CTA cluster per image
 bool tail_fused_supported(int h, int w, int H, int W, int C);
 // out_stride: floats between the maps of consecutive images (0 = H * W)
 int launch_tail_fused(const __half* A, const float* alpha_raw, float scale, float* alpha_out, float* out, int B, int h, int w,
-                      int H, int W, int C, bool x3, cudaStream_t s, const int* n_dev = nullptr, size_t out_stride = 0);
+                      int H, int W, int C, bool x3, cudaStream_t s, const int* n_dev = nullptr, size_t out_stride = 0, float inv_slope = 0.f);
 // TF_GROUP target classes in one launch, one read of A: alpha of class k at alpha_raw + k * alpha_ld ([B][C] each), the map of class k
 // of image b at out + b * out_stride + k * H * W; each bit-identical to a launch_tail_fused of that class
 constexpr int TF_GROUP = 2;
 bool tail_fused_classes_supported(int h, int w, int H, int W, int C);
 int launch_tail_fused_classes(const __half* A, const float* alpha_raw, size_t alpha_ld, float scale, float* out, size_t out_stride, int B,
-                              int h, int w, int H, int W, int C, bool x3, cudaStream_t s, const int* n_dev = nullptr);
-// tie-duplicating rule on the fp16x3 path: alpha_raw[b][k] = sum_windows g * (#maxima in the window), A = split C8-planar activations
-int launch_alpha_ties_c8(const __half* A, const float* g_pool, float* alpha_raw, int B, int h, int w, int C, cudaStream_t s);
+                              int h, int w, int H, int W, int C, bool x3, cudaStream_t s, const int* n_dev = nullptr, float inv_slope = 0.f);
+// tie-duplicating rule on the fp16x3 path: alpha_raw[b][k] = sum_windows g * (#maxima in the window), A = split C8-planar activations;
+// pre_slope >= 0 (pre-activation target): each window's term also times LeakyReLU' at its maximum = (max > 0 ? 1 : pre_slope)
+int launch_alpha_ties_c8(const __half* A, const float* g_pool, float* alpha_raw, int B, int h, int w, int C, cudaStream_t s,
+                         float pre_slope = -1.f);
 int launch_c8_to_nhwc(const __half* src, float* dst, int B, int h, int w, int C, bool x3, cudaStream_t s);
 
 }  // namespace bcad

@@ -43,10 +43,12 @@ __device__ __forceinline__ void tf_block_minmax(float& vmin, float& vmax, float*
 
 // CL = CTAs per image (cluster size), NT = threads per CTA, K = target classes (alpha_raw + k * alpha_ld, the H x W map of class k
 // of image b at out + b * out_stride + k * H * W)
-template <bool X3, int CL, int NT, int K>
+// PRE: the pre-activation target, z = a > 0 ? a : a * inv_slope before the channel reduction (the post-activation instantiations are
+// unchanged)
+template <bool X3, int CL, int NT, int K, bool PRE>
 __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(NT, 1024 / NT)
 tail_fused_kernel(const __half* __restrict__ A, const float* __restrict__ alpha_raw, size_t alpha_ld, float scale, float* __restrict__ alpha_out,
-                  float* __restrict__ out, size_t out_stride, int h, int w, int H, int W, int C, const int* __restrict__ n_dev) {
+                  float* __restrict__ out, size_t out_stride, int h, int w, int H, int W, int C, const int* __restrict__ n_dev, float inv_slope) {
     cg::cluster_group cluster = cg::this_cluster();
     const int rank = (int)cluster.block_rank();
     const int b = blockIdx.x / CL;
@@ -119,6 +121,7 @@ tail_fused_kernel(const __half* __restrict__ A, const float* __restrict__ alpha_
                     const float2 g0 = unpack_f16(ql.x), g1 = unpack_f16(ql.y), g2 = unpack_f16(ql.z), g3 = unpack_f16(ql.w);
                     f0.x += g0.x; f0.y += g0.y; f1.x += g1.x; f1.y += g1.y; f2.x += g2.x; f2.y += g2.y; f3.x += g3.x; f3.y += g3.y;
                 }
+                if constexpr (PRE) { f0 = unleaky2(f0, inv_slope); f1 = unleaky2(f1, inv_slope); f2 = unleaky2(f2, inv_slope); f3 = unleaky2(f3, inv_slope); }
 #pragma unroll
                 for (int k = 0; k < K; ++k) {
                     const float* al = s_alpha + k * cpad + c * 8;
@@ -233,29 +236,38 @@ bool tail_fused_classes_supported(int h, int w, int H, int W, int C) {
     return tail_fused_supported(h, w, H, W, C) && tail_fused_smem_k(h, w, H, W, C, TF_GROUP) <= 200 * 1024;
 }
 
-template <bool X3, int CL, int NT, int K>
-static int launch_tf(const __half* A, const float* alpha_raw, size_t alpha_ld, float scale, float* alpha_out, float* out, size_t out_stride,
-                     int B, int h, int w, int H, int W, int C, cudaStream_t s, const int* n_dev) {
+template <bool X3, int CL, int NT, int K, bool PRE>
+static int launch_tf_t(const __half* A, const float* alpha_raw, size_t alpha_ld, float scale, float* alpha_out, float* out, size_t out_stride,
+                       int B, int h, int w, int H, int W, int C, cudaStream_t s, const int* n_dev, float inv_slope) {
     const size_t smem = tail_fused_smem_k(h, w, H, W, C, K);
-    BCAD_CUDA_CHECK(cudaFuncSetAttribute(tail_fused_kernel<X3, CL, NT, K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    tail_fused_kernel<X3, CL, NT, K><<<CL * B, NT, smem, s>>>(A, alpha_raw, alpha_ld, scale, alpha_out, out, out_stride, h, w, H, W, C, n_dev);
+    BCAD_CUDA_CHECK(cudaFuncSetAttribute(tail_fused_kernel<X3, CL, NT, K, PRE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    tail_fused_kernel<X3, CL, NT, K, PRE><<<CL * B, NT, smem, s>>>(A, alpha_raw, alpha_ld, scale, alpha_out, out, out_stride, h, w, H, W, C, n_dev,
+                                                                   inv_slope);
     BCAD_CUDA_CHECK(cudaGetLastError());
     return BCAD_OK;
 }
 
+template <bool X3, int CL, int NT, int K>
+static int launch_tf(const __half* A, const float* alpha_raw, size_t alpha_ld, float scale, float* alpha_out, float* out, size_t out_stride,
+                     int B, int h, int w, int H, int W, int C, cudaStream_t s, const int* n_dev, float inv_slope) {
+    if (inv_slope > 0.f)
+        return launch_tf_t<X3, CL, NT, K, true>(A, alpha_raw, alpha_ld, scale, alpha_out, out, out_stride, B, h, w, H, W, C, s, n_dev, inv_slope);
+    return launch_tf_t<X3, CL, NT, K, false>(A, alpha_raw, alpha_ld, scale, alpha_out, out, out_stride, B, h, w, H, W, C, s, n_dev, 0.f);
+}
+
 int launch_tail_fused(const __half* A, const float* alpha_raw, float scale, float* alpha_out, float* out, int B, int h, int w,
-                      int H, int W, int C, bool x3, cudaStream_t s, const int* n_dev, size_t out_stride) {
+                      int H, int W, int C, bool x3, cudaStream_t s, const int* n_dev, size_t out_stride, float inv_slope) {
     BCAD_REQUIRE(tail_fused_supported(h, w, H, W, C), "tail_fused: map %dx%d -> %dx%d does not fit in shared memory", h, w, H, W);
     const size_t os = out_stride ? out_stride : (size_t)H * W;
-    if (x3) return launch_tf<true, TF_CL, TF_NT, 1>(A, alpha_raw, 0, scale, alpha_out, out, os, B, h, w, H, W, C, s, n_dev);
-    return launch_tf<false, TF_CL, TF_NT, 1>(A, alpha_raw, 0, scale, alpha_out, out, os, B, h, w, H, W, C, s, n_dev);
+    if (x3) return launch_tf<true, TF_CL, TF_NT, 1>(A, alpha_raw, 0, scale, alpha_out, out, os, B, h, w, H, W, C, s, n_dev, inv_slope);
+    return launch_tf<false, TF_CL, TF_NT, 1>(A, alpha_raw, 0, scale, alpha_out, out, os, B, h, w, H, W, C, s, n_dev, inv_slope);
 }
 
 int launch_tail_fused_classes(const __half* A, const float* alpha_raw, size_t alpha_ld, float scale, float* out, size_t out_stride, int B,
-                              int h, int w, int H, int W, int C, bool x3, cudaStream_t s, const int* n_dev) {
+                              int h, int w, int H, int W, int C, bool x3, cudaStream_t s, const int* n_dev, float inv_slope) {
     BCAD_REQUIRE(tail_fused_classes_supported(h, w, H, W, C), "tail_fused_classes: map %dx%d -> %dx%d does not fit in shared memory", h, w, H, W);
-    if (x3) return launch_tf<true, TF2_CL, TF2_NT, TF_GROUP>(A, alpha_raw, alpha_ld, scale, nullptr, out, out_stride, B, h, w, H, W, C, s, n_dev);
-    return launch_tf<false, TF2_CL, TF2_NT, TF_GROUP>(A, alpha_raw, alpha_ld, scale, nullptr, out, out_stride, B, h, w, H, W, C, s, n_dev);
+    if (x3) return launch_tf<true, TF2_CL, TF2_NT, TF_GROUP>(A, alpha_raw, alpha_ld, scale, nullptr, out, out_stride, B, h, w, H, W, C, s, n_dev, inv_slope);
+    return launch_tf<false, TF2_CL, TF2_NT, TF_GROUP>(A, alpha_raw, alpha_ld, scale, nullptr, out, out_stride, B, h, w, H, W, C, s, n_dev, inv_slope);
 }
 
 }  // namespace bcad

@@ -9,6 +9,8 @@
 //   explain: top gradient -> dense backward to dz1 -> alpha = dz1 . S / (h w)  with S[u][k] = sum_pixels W1[u][pixel,k]
 //            (exact for first-index pooling: the un-pooled gradient of a window sums to the pooled gradient, so the
 //             dense gradient map dA never has to exist -- SURVEY P8), cam_c8 -> upsample_norm.
+//   pre-activation target (bcad_set_explain_target): dz1 -> alpha_preact (the fc1 input-gradient GEMM masked by LeakyReLU' of the pooled
+//            map, summed in its epilogue: dA still never exists), tails that undo the activation, z = a > 0 ? a : a / slope.
 #include <math.h>
 #include <stdlib.h>
 #include <string.h>
@@ -47,6 +49,9 @@ struct TensorPath {
     bool x3 = false;                // fp16x3: hi/lo split operands everywhere (fp32-grade)
     uint8_t* d_fc_wT = nullptr;     // tie-duplicating mode: fc1 transposed as W tiles of the input-gradient GEMM [col block][k-block][hi|lo][256][128 B]
     uint8_t* dz_tiles = nullptr;    // dz1 as split A tiles [m_pad/128][units/64][hi|lo][128][128 B]
+    bool preact = false;            // first-index pooling, a pre-activation target is possible (alpha_preact_supported)
+    int* dz_exp = nullptr;          // pre-activation target: dz1 row b enters the GEMM scaled by 2^dz_exp[b]
+    float* pre_part = nullptr;      // pre-activation target: alpha partials [fc_splits][m_pad][64]
     bool p1_valid = true;           // the last forward wrote the pooled first-block map to HBM (the fused kernel only does with keep_all_activations)
     bool wide = false;              // first block has Cin > 1: nhwc_to_c8 + conv_wide (sm100_wide.cu)
     int cin_pad = 0, kc = 0, groups = 0;
@@ -299,6 +304,7 @@ int tensor_path_commit(Model& m) {
             TP_TRY(m.alloc((void**)&t.dz_tiles, (size_t)m_pad * d0.out * 2 * 2));
         }
     }
+    t.preact = m.cfg.pool_ties == BCAD_TIES_FIRST && alpha_preact_supported(d0.out, c1.Cout);
     // ---- workspace
     if (t.p1 == nullptr) {
         t.m_pad = cdiv(mb, 128) * 128;
@@ -315,7 +321,21 @@ int tensor_path_commit(Model& m) {
         BCAD_CUDA_CHECK(cudaMemset(t.fc_a, 0, parts * t.m_pad * npix * 128));     // padding rows: finite zeros
         TP_TRY(m.alloc((void**)&t.fc_part, (size_t)t.fc_splits * t.m_pad * d0.out * 4));
         TP_TRY(m.alloc((void**)&t.alpha_raw, (size_t)TF_GROUP * mb * c1.Cout * 4));      // one [mb][C] slice per class of a tail group
+        if (t.preact) {                                                                   // small: 0.5 + 4.8 MB at max_batch 512
+            TP_TRY(m.alloc((void**)&t.dz_tiles, (size_t)t.m_pad * d0.out * 2 * 2));
+            TP_TRY(m.alloc((void**)&t.dz_exp, (size_t)t.m_pad * sizeof(int)));
+            TP_TRY(m.alloc((void**)&t.pre_part, (size_t)t.fc_splits * t.m_pad * c1.Cout * 4));
+        }
     }
+    return BCAD_OK;
+}
+
+int tensor_preact_supported(const Model& m) {
+    if (m.cfg.pool_ties != BCAD_TIES_FIRST) return BCAD_OK;         // the tie-duplicating flavour forms the dense pooled gradient anyway
+    const int units = m.dense[0].out;
+    BCAD_REQUIRE(alpha_preact_supported(units, m.conv.back().Cout),
+                 "the pre-activation target on the tensor paths needs a first dense layer with a multiple of 64 units (got %d); "
+                 "create the model with BCAD_PREC_FP32 to use the fp32 path for this shape", units);
     return BCAD_OK;
 }
 
@@ -418,6 +438,9 @@ int tensor_forward_chunk(Model& m, const float* x, int n, bool explain, const in
         if (m.cfg.pool_ties != BCAD_TIES_FIRST)              // dz1 stays in dense[0].h for the fp32 tail; no alpha shortcut
             return launch_fused_head(&m, n, t.fc_part, t.fc_splits, (size_t)t.m_pad * d0.out, explain, class_idx, grad_mode,
                                      explain ? d0.h : nullptr, nullptr, 0, nullptr, s);
+        if (m.target == BCAD_TARGET_CONV_PREACT)             // dz1 for the masked input-gradient GEMM instead of the alpha shortcut
+            return launch_fused_head(&m, n, t.fc_part, t.fc_splits, (size_t)t.m_pad * d0.out, explain, class_idx, grad_mode,
+                                     explain ? d0.h : nullptr, nullptr, 0, nullptr, s);
         return launch_fused_head(&m, n, t.fc_part, t.fc_splits, (size_t)t.m_pad * d0.out, explain, class_idx, grad_mode,
                                  nullptr, t.d_S, c1.Cout, t.alpha_raw, s);
     }
@@ -458,7 +481,21 @@ static int tensor_alpha(Model& m, int n, const int32_t* class_idx, int grad_mode
         } else {
             TP_LAUNCH(m, "fc1_dgrad_sgemm", launch_sgemm(D0.h, D0.d_w, m.g_flat, n, D0.in, D0.out, false, 1, s));
         }
-        TP_LAUNCH(m, "alpha_ties_c8", launch_alpha_ties_c8(t.act, m.g_flat, alpha_dst, n, T.Ho, T.Wo, T.Cout, s));
+        TP_LAUNCH(m, "alpha_ties_c8", launch_alpha_ties_c8(t.act, m.g_flat, alpha_dst, n, T.Ho, T.Wo, T.Cout, s,
+                                                           m.target == BCAD_TARGET_CONV_PREACT ? m.cfg.alpha_conv : -1.f));
+    } else if (m.target == BCAD_TARGET_CONV_PREACT) {
+        // pre-activation target: dz1 -> masked input-gradient GEMM on tcgen05 -> alpha_raw (the dense pooled gradient never exists)
+        if (!m.fused_head) TP_TRY(dense_backward(&m, n, class_idx, grad_mode, nullptr, s));
+        else if (rerun_head) TP_TRY(relaunch_fused_head(&m, class_idx, nullptr, s));
+        DenseLayer& D0 = m.dense[0];
+        const float* dz1 = (m.fused_head || m.dense.size() > 1) ? D0.h : m.d_top;
+        TP_LAUNCH(m, "dz1_to_tiles", launch_dz_rows_to_tiles(dz1, t.dz_tiles, t.dz_exp, n, D0.out, t.m_pad, s));
+        PreactArgs a;
+        a.dz_tiles = t.dz_tiles; a.w_tiles = t.d_fc_w; a.mask_tiles = t.fc_a; a.partials = t.pre_part;
+        a.units = D0.out; a.npix = T.Hp * T.Wp; a.q_per_split = t.kb_per_split; a.m_pad = t.m_pad;
+        a.x3 = t.x3 ? 1 : 0; a.slope = m.cfg.alpha_conv; a.nst = 0; a.n_dev = m.n_dev;
+        TP_LAUNCH(m, "alpha_preact_tcgen05", launch_alpha_preact(a, cdiv(n, 128), t.fc_splits, s));
+        TP_LAUNCH(m, "alpha_preact_reduce", launch_alpha_preact_reduce(t.pre_part, t.fc_splits, t.m_pad, t.dz_exp, alpha_dst, n, s));
     } else if (!m.fused_head) {
         // dense backward down to dz1 (left in dense[0].h); no fc1 dgrad GEMM, no dA
         TP_TRY(dense_backward(&m, n, class_idx, grad_mode, nullptr, s));
@@ -475,6 +512,7 @@ int tensor_explain_chunk(Model& m, int n, const int32_t* class_idx, int grad_mod
     TensorPath& t = *m.tp;
     const ConvLayer& T = m.conv.back();
     const float inv_hw = 1.0f / ((float)T.Ho * (float)T.Wo);
+    const float inv_slope = (m.target == BCAD_TARGET_CONV_PREACT) ? 1.0f / m.cfg.alpha_conv : 0.f;    // > 0: the tails undo the activation
     const size_t hm = (size_t)m.heat_h * m.heat_w, slot = (size_t)m.cfg.max_batch * T.Cout;
     // The one-launch cluster tail needs about a CTA pair per SM to pay (one image's pair streams its 2-4 MB map at a single SM
     // pair's bandwidth: 73 us whatever the batch); handles sized for a few images (single requests, the refinement twin) take the
@@ -493,12 +531,13 @@ int tensor_explain_chunk(Model& m, int n, const int32_t* class_idx, int grad_mod
         float* hk = heat + k0 * hm;
         if (g > 1) {
             TP_LAUNCH(m, "tail_fused_classes", launch_tail_fused_classes(t.act, t.alpha_raw, slot, inv_hw, hk, heat_stride, n, T.Ho, T.Wo,
-                                                                         m.heat_h, m.heat_w, T.Cout, t.x3, s, m.n_dev));
+                                                                         m.heat_h, m.heat_w, T.Cout, t.x3, s, m.n_dev, inv_slope));
         } else if (fused) {
             TP_LAUNCH(m, "tail_fused", launch_tail_fused(t.act, t.alpha_raw, inv_hw, m.alpha, hk, n, T.Ho, T.Wo, m.heat_h, m.heat_w, T.Cout, t.x3, s, m.n_dev,
-                                                         heat_stride));
+                                                         heat_stride, inv_slope));
         } else {
-            TP_LAUNCH(m, "cam_c8", launch_cam_c8(t.act, t.alpha_raw, inv_hw, m.alpha, m.cam_lo, m.mm, n, T.Ho, T.Wo, T.Cout, m.cam_splits, t.x3, s, m.n_dev));
+            TP_LAUNCH(m, "cam_c8", launch_cam_c8(t.act, t.alpha_raw, inv_hw, m.alpha, m.cam_lo, m.mm, n, T.Ho, T.Wo, T.Cout, m.cam_splits, t.x3, s, m.n_dev,
+                                                   inv_slope));
             TP_LAUNCH(m, "upsample_norm", launch_upsample_norm(m.cam_lo, m.mm, m.cam_splits, hk, n, T.Ho, T.Wo, m.heat_h, m.heat_w, s, m.n_dev,
                                                                heat_stride));
         }

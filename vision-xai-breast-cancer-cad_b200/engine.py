@@ -189,8 +189,10 @@ class Engine:
 
     def set_explain_target(self, target: str = "conv"):
         """"conv": the last conv block's post-LeakyReLU output (default; explainability.py:64).  "conv_preact": the conv module's own
-        output before the activation -- what pytorch_grad_cam sees when it hooks ``model.convs[-1]`` of ADCNNM.CNNModel (ADCNNM.py:76);
-        fp32 engines only."""
+        output before the activation -- what pytorch_grad_cam sees when it hooks ``model.convs[-1]`` of ADCNNM.CNNModel (ADCNNM.py:76).
+        Every precision runs it: on the tensor paths the channel weights come from a masked fc1 input-gradient GEMM on tcgen05, which
+        with first-index pooling needs a first dense layer of a multiple of 64 units (ValueError otherwise: use an fp32 engine).
+        A handle with ``refine_margin`` passes the target to its refinement twin."""
         _lib.check(self.lib.bcad_set_explain_target(self._h, _lib.TARGET[target]))
         self.explain_target = target
 
@@ -887,6 +889,11 @@ class ShardedEngine:
         """Engine.set_fast_training on every GPU's engine (a model's ``saliency_engine`` has it on where the shape allows)."""
         for e in self.engines:
             e.set_fast_training(on)
+
+    def set_explain_target(self, target: str = "conv"):
+        """Engine.set_explain_target on every GPU's engine (they share one network shape: all accept the target or the first refuses)."""
+        for e in self.engines:
+            e.set_explain_target(target)
 
     def saliency_overlays_classes_host(self, gray_u8: np.ndarray, classes=(0, 1), grad_mode="softmax_ce", standardise=True,
                                        want_saliency=False):
