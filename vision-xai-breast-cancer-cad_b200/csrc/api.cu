@@ -775,6 +775,246 @@ static int run_saliency(Model* m, const float* x, int B, int K, const int32_t* c
     return BCAD_OK;
 }
 
+// -----------------------------------------------------------------------------------------------------
+// host-buffer calls: H2D / compute / D2H in chunks on three streams, double-buffered
+// -----------------------------------------------------------------------------------------------------
+// streams, events and the model-size slot buffers of the pipeline, on first use (caller holds m->mu)
+static int xfer_init(Model* m) {
+    Xfer& X = m->xfer;
+    if (X.inited) return BCAD_OK;
+    const size_t img = (size_t)m->cfg.in_h * m->cfg.in_w * m->cfg.in_c, hm = (size_t)m->cfg.in_h * m->cfg.in_w;
+    int chunk = std::min(m->cfg.max_batch, 128);
+    if (const char* e = getenv("BCAD_HOST_CHUNK")) chunk = std::max(1, std::min(m->cfg.max_batch, atoi(e)));
+    BCAD_CUDA_CHECK(cudaStreamCreateWithFlags(&X.s_in, cudaStreamNonBlocking));
+    BCAD_CUDA_CHECK(cudaStreamCreateWithFlags(&X.s_compute, cudaStreamNonBlocking));
+    BCAD_CUDA_CHECK(cudaStreamCreateWithFlags(&X.s_out, cudaStreamNonBlocking));
+    for (int i = 0; i < 2; ++i) {
+        BCAD_CUDA_CHECK(cudaEventCreateWithFlags(&X.in_done[i], cudaEventDisableTiming));
+        BCAD_CUDA_CHECK(cudaEventCreateWithFlags(&X.compute_done[i], cudaEventDisableTiming));
+        BCAD_CUDA_CHECK(cudaEventCreateWithFlags(&X.out_done[i], cudaEventDisableTiming));
+        BCAD_TRY(m->alloc((void**)&X.x[i], (size_t)chunk * img * sizeof(float)));
+        BCAD_TRY(m->alloc((void**)&X.heat[i], (size_t)chunk * hm * sizeof(float)));
+        BCAD_TRY(m->alloc((void**)&X.cidx[i], (size_t)chunk * sizeof(int32_t)));
+    }
+    X.chunk = chunk;
+    X.inited = true;
+    return BCAD_OK;
+}
+
+// Images per chunk of a host-buffer call (after xfer_init): small enough that the PCIe pipeline fills quickly (the link, ~52 GB/s per
+// direction, is the end-to-end bound), large enough to keep the kernels efficient -- a quarter of the batch, 32 .. cap images.  cap is
+// 64 for float32 images (the link is the bound: at 512 images 3.6-3.7 ms with 64, 3.7-3.8 with 128) and 128 for 8-bit images (compute
+// is the bound: 2.11 ms with 64, 1.73 ms with 128, 1.80 ms with 256).  BCAD_HOST_CHUNK overrides (tuning).
+// Uniform chunks: measured at 512 images, 64-image chunks 3.62 ms, ramped (C/4, C/2, C, ..., C/2, C/4) 3.93 ms.
+static int host_chunk(const Model* m, int B, int cap) {
+    const int chunk = m->xfer.chunk;
+    if (const char* e = getenv("BCAD_HOST_CHUNK")) return std::max(1, std::min(chunk, atoi(e)));
+    return std::min(std::min(chunk, cap), std::max(32, ((B + 3) / 4 + 31) / 32 * 32));
+}
+
+// The checks every host-buffer call makes before any copy.  K = 0: class_idx [B] of the single-class calls; K >= 1: classes [B][K] of
+// the classes calls (NULL: the default targets).  fn names the call in the messages.
+static int check_host(const char* fn, Model* m, const void* image, int B, int grad_mode, const int32_t* classes, int K) {
+    BCAD_REQUIRE(m && image, "%s: null model or image pointer", fn);
+    BCAD_REQUIRE(B >= 1, "batch must be >= 1, got %d", B);
+    if (!m->committed) { set_error("weights not committed: call bcad_commit first"); return BCAD_ERR_STATE; }
+    BCAD_REQUIRE(grad_mode == BCAD_GRAD_LOGIT || grad_mode == BCAD_GRAD_SOFTMAX_CE, "bad grad_mode %d", grad_mode);
+    const int nc = m->cfg.num_classes, kc = K ? K : 1;
+    if (classes != nullptr)
+        for (size_t i = 0; i < (size_t)B * kc; ++i)
+            if (classes[i] < 0 || classes[i] >= nc) {
+                if (K) set_error("classes[%zu][%zu] = %d is outside [0, %d)", i / K, i % K, classes[i], nc);
+                else set_error("class_idx[%zu] = %d is outside [0, %d)", i, classes[i], nc);
+                return BCAD_ERR_INVALID;
+            }
+    return BCAD_OK;
+}
+
+// small outputs (logits, probabilities, classes) go through pinned staging sized for the whole call (caller holds m->host_mu)
+static int stage_small(Model* m, size_t bytes) {
+    Xfer& X = m->xfer;
+    if (X.h_small_bytes < bytes) {
+        if (X.h_small) cudaFreeHost(X.h_small);
+        X.h_small = nullptr;
+        X.h_small_bytes = 0;
+        BCAD_CUDA_CHECK(cudaMallocHost(&X.h_small, bytes));
+        X.h_small_bytes = bytes;
+    }
+    if (X.d_small_bytes < bytes) {
+        std::lock_guard<std::mutex> lock(m->mu);             // grows only when a call is larger than every call before it; the handle
+        X.d_small = nullptr;                                 // owns (and frees at destroy) the smaller ones it replaces: tens of bytes per image
+        X.d_small_bytes = 0;
+        BCAD_TRY(m->alloc(&X.d_small, bytes));
+        X.d_small_bytes = bytes;
+    }
+    return BCAD_OK;
+}
+
+// logits / probabilities / classes of a whole host-buffer call: written on the device per chunk, brought back by one copy behind the
+// last chunk through the pinned staging of stage_small
+struct SmallOutputs {
+    size_t bytes = 0;
+    float *dv_logits = nullptr, *dv_probs = nullptr;
+    int32_t* dv_cls = nullptr;
+};
+
+static int small_outputs(Model* m, int B, SmallOutputs& o) {
+    const int nc = m->cfg.num_classes;
+    o.bytes = ((size_t)(2 * nc) * sizeof(float) + sizeof(int32_t)) * B;
+    BCAD_TRY(stage_small(m, o.bytes));
+    o.dv_logits = reinterpret_cast<float*>(m->xfer.d_small);
+    o.dv_probs = o.dv_logits + (size_t)B * nc;
+    o.dv_cls = reinterpret_cast<int32_t*>(o.dv_probs + (size_t)B * nc);
+    return BCAD_OK;
+}
+
+static void copy_small_outputs(Model* m, int B, float* logits_host, float* probs_host, int32_t* cls_host) {
+    const int nc = m->cfg.num_classes;
+    const float* st_logits = reinterpret_cast<const float*>(m->xfer.h_small);
+    const float* st_probs = st_logits + (size_t)B * nc;
+    const int32_t* st_cls = reinterpret_cast<const int32_t*>(st_probs + (size_t)B * nc);
+    if (logits_host) memcpy(logits_host, st_logits, (size_t)B * nc * sizeof(float));
+    if (probs_host) memcpy(probs_host, st_probs, (size_t)B * nc * sizeof(float));
+    if (cls_host) memcpy(cls_host, st_cls, (size_t)B * sizeof(int32_t));
+}
+
+// The chunk loop of every host-buffer call: per chunk c (slot c & 1, images b0 .. b0 + n) h2d(slot, b0, n) on s_in, compute(slot, b0, n)
+// on s_compute, d2h(slot, b0, n) on s_out, ordered by the slot's events; the steady state runs H2D, compute and D2H of three chunks
+// concurrently.  The small outputs follow the last chunk's D2H.  Returns after both streams have drained.
+template <class H2D, class Compute, class D2H>
+static int host_pipeline(Model* m, int B, int C0, const SmallOutputs& so, H2D h2d, Compute compute, D2H d2h) {
+    Xfer& X = m->xfer;
+    const int nchunks = (B + C0 - 1) / C0;
+    for (int c = 0, b0 = 0; c < nchunks; ++c, b0 += C0) {
+        const int slot = c & 1, n = std::min(C0, B - b0);
+        if (c >= 2) {                                         // slot reuse: its previous D2H (chunk c-2) must have drained
+            BCAD_CUDA_CHECK(cudaStreamWaitEvent(X.s_in, X.compute_done[slot], 0));
+            BCAD_CUDA_CHECK(cudaStreamWaitEvent(X.s_compute, X.out_done[slot], 0));
+        }
+        BCAD_TRY(h2d(slot, b0, n));
+        BCAD_CUDA_CHECK(cudaEventRecord(X.in_done[slot], X.s_in));
+        BCAD_CUDA_CHECK(cudaStreamWaitEvent(X.s_compute, X.in_done[slot], 0));
+        const int rc = compute(slot, b0, n);
+        if (rc != BCAD_OK) { cudaDeviceSynchronize(); return rc; }
+        BCAD_CUDA_CHECK(cudaEventRecord(X.compute_done[slot], X.s_compute));
+        BCAD_CUDA_CHECK(cudaStreamWaitEvent(X.s_out, X.compute_done[slot], 0));
+        BCAD_TRY(d2h(slot, b0, n));
+        if (c + 1 == nchunks) BCAD_CUDA_CHECK(cudaMemcpyAsync(X.h_small, X.d_small, so.bytes, cudaMemcpyDeviceToHost, X.s_out));
+        BCAD_CUDA_CHECK(cudaEventRecord(X.out_done[slot], X.s_out));
+    }
+    BCAD_CUDA_CHECK(cudaStreamSynchronize(X.s_out));
+    BCAD_CUDA_CHECK(cudaStreamSynchronize(X.s_compute));
+    return BCAD_OK;
+}
+
+// The single-class host-buffer calls, one image source: x_host float32 images, x8_host 8-bit pixels (x = u8 / 255 on the device) or
+// gray8_host grey images of the model's size (gray_preprocess; overlay_host gets their RGB overlays).  Chunks run in the handle's Xfer
+// slots, sized for up to 128 images.
+static int predict_explain_host_impl(bcad_model* mm, const float* x_host, const uint8_t* x8_host, int B, const int32_t* class_idx_host,
+                                     int grad_mode, float* logits_host, float* probs_host, int32_t* cls_host, float* heat_host,
+                                     uint8_t* heat_u8_host, const uint8_t* gray8_host = nullptr, int standardise = 0,
+                                     uint8_t* overlay_host = nullptr) {
+    Model* m = reinterpret_cast<Model*>(mm);
+    const void* image = gray8_host ? (const void*)gray8_host : x8_host ? (const void*)x8_host : (const void*)x_host;
+    BCAD_TRY(check_host("predict_explain_host", m, image, B, grad_mode, class_idx_host, 0));
+    DeviceGuard g(m->cfg.device);
+    // one host-buffer call at a time per handle: the three streams, the double-buffered device slots, the events and the pinned
+    // staging are shared (threaded callers -- a Flask app with one model -- queue here; separate handles run concurrently)
+    std::lock_guard<std::mutex> host_lock(m->host_mu);
+    Xfer& X = m->xfer;
+    const int nc = m->cfg.num_classes;
+    const size_t img = (size_t)m->cfg.in_h * m->cfg.in_w * m->cfg.in_c, hm = (size_t)m->cfg.in_h * m->cfg.in_w;
+    {
+        std::lock_guard<std::mutex> lock(m->mu);
+        BCAD_TRY(xfer_init(m));
+        if (heat_u8_host != nullptr && X.heat8[0] == nullptr)
+            for (int i = 0; i < 2; ++i) BCAD_TRY(m->alloc((void**)&X.heat8[i], (size_t)X.chunk * hm));
+        if ((x8_host != nullptr || gray8_host != nullptr) && X.x8[0] == nullptr)
+            for (int i = 0; i < 2; ++i) BCAD_TRY(m->alloc((void**)&X.x8[i], (size_t)X.chunk * img));
+        if (gray8_host != nullptr && X.img01[0] == nullptr)
+            for (int i = 0; i < 2; ++i) {
+                BCAD_TRY(m->alloc((void**)&X.img01[i], (size_t)X.chunk * hm * sizeof(float)));
+                BCAD_TRY(m->alloc((void**)&X.ov8[i], (size_t)X.chunk * hm * 3));
+            }
+    }
+    SmallOutputs so;
+    BCAD_TRY(small_outputs(m, B, so));
+    const bool want_heat = (heat_host != nullptr || heat_u8_host != nullptr || overlay_host != nullptr);
+    BCAD_TRY(host_pipeline(m, B, host_chunk(m, B, (x8_host || gray8_host) ? 128 : 64), so,
+        [&](int slot, int b0, int n) {
+            if (gray8_host) BCAD_CUDA_CHECK(cudaMemcpyAsync(X.x8[slot], gray8_host + (size_t)b0 * hm, (size_t)n * hm, cudaMemcpyHostToDevice, X.s_in));
+            else if (x8_host) BCAD_CUDA_CHECK(cudaMemcpyAsync(X.x8[slot], x8_host + (size_t)b0 * img, (size_t)n * img, cudaMemcpyHostToDevice, X.s_in));
+            else BCAD_CUDA_CHECK(cudaMemcpyAsync(X.x[slot], x_host + (size_t)b0 * img, (size_t)n * img * sizeof(float), cudaMemcpyHostToDevice, X.s_in));
+            if (class_idx_host)
+                BCAD_CUDA_CHECK(cudaMemcpyAsync(X.cidx[slot], class_idx_host + b0, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, X.s_in));
+            return BCAD_OK;
+        },
+        [&](int slot, int b0, int n) {
+            int rc = BCAD_OK;
+            if (gray8_host) rc = launch_gray_preprocess(X.x8[slot], X.img01[slot], X.x[slot], n, (int)hm, m->cfg.in_c, standardise, X.s_compute);
+            else if (x8_host) rc = launch_u8_to_unit(X.x8[slot], X.x[slot], (size_t)n * img, X.s_compute);
+            if (rc == BCAD_OK)
+                rc = run(m, X.x[slot], n, class_idx_host ? X.cidx[slot] : nullptr, grad_mode, want_heat, so.dv_logits + (size_t)b0 * nc,
+                         so.dv_probs + (size_t)b0 * nc, so.dv_cls + b0, X.heat[slot], X.s_compute);
+            if (rc == BCAD_OK && overlay_host != nullptr)     // show_cam_on_image + heatmap_uint8 in one pass (GRADCAM.py:67,70)
+                rc = launch_overlay(X.img01[slot], X.heat[slot], n, m->cfg.in_h, m->cfg.in_w, X.ov8[slot], heat_u8_host ? X.heat8[slot] : nullptr, X.s_compute);
+            else if (rc == BCAD_OK && heat_u8_host != nullptr) rc = launch_heat_to_u8(X.heat[slot], X.heat8[slot], (size_t)n * hm, X.s_compute);
+            return rc;
+        },
+        [&](int slot, int b0, int n) {
+            if (heat_host) BCAD_CUDA_CHECK(cudaMemcpyAsync(heat_host + (size_t)b0 * hm, X.heat[slot], (size_t)n * hm * sizeof(float), cudaMemcpyDeviceToHost, X.s_out));
+            if (heat_u8_host) BCAD_CUDA_CHECK(cudaMemcpyAsync(heat_u8_host + (size_t)b0 * hm, X.heat8[slot], (size_t)n * hm, cudaMemcpyDeviceToHost, X.s_out));
+            if (overlay_host) BCAD_CUDA_CHECK(cudaMemcpyAsync(overlay_host + (size_t)b0 * hm * 3, X.ov8[slot], (size_t)n * hm * 3, cudaMemcpyDeviceToHost, X.s_out));
+            return BCAD_OK;
+        }));
+    copy_small_outputs(m, B, logits_host, probs_host, cls_host);
+    return BCAD_OK;
+}
+
+// Staging bound of the host-buffer classes calls (bcad_gradcam_overlays_classes_host, bcad_saliency_overlays_classes_host): both slots'
+// 8-bit images, classes and maps stay within this many bytes of the handle's memory (the chunk shrinks to fit; a single image larger
+// than half of it still runs, one image per chunk).  Grad-CAM, 512 x 512 images with K = 2: 4.25 MB per image and slot, chunks of up
+// to 60 images.
+static const size_t kClassesStagingBytes = (size_t)512 << 20;
+
+static size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
+
+// The checks of the classes calls on top of check_host, all made before any copy.  fn names the call in the messages.
+static int check_classes_host(const char* fn, Model* m, const uint8_t* gray_u8_host, int B, int img_h, int img_w, int K,
+                              const int32_t* classes_host_or_null, int grad_mode, int standardise, bool any_output) {
+    BCAD_REQUIRE(any_output, "%s: the output pointers are all null", fn);
+    BCAD_REQUIRE(img_h >= 1 && img_w >= 1 && img_h <= 16384 && img_w <= 16384, "%s: bad image size %dx%d", fn, img_h, img_w);
+    BCAD_REQUIRE(K >= 1 && K <= BCAD_MAX_EXPLAIN_CLASSES, "%s: K=%d out of range 1..%d", fn, K, BCAD_MAX_EXPLAIN_CLASSES);
+    BCAD_REQUIRE(standardise == 0 || standardise == 1, "%s: standardise must be 0 or 1", fn);
+    BCAD_TRY(check_host(fn, m, gray_u8_host, B, grad_mode, classes_host_or_null, K));
+    BCAD_REQUIRE(classes_host_or_null || K <= m->cfg.num_classes, "%s: classes=NULL explains classes 0..K-1, but K=%d > num_classes=%d",
+                 fn, K, m->cfg.num_classes);
+    return BCAD_OK;
+}
+
+// Chunk size of a classes call and the arena holding both slots of per_img_slot bytes per image (caller holds m->host_mu): host_chunk
+// with the 8-bit cap, shrunk to the staging bound.  Slot i starts at arena + i * C0 * per_img_slot.
+static int classes_staging(Model* m, int B, size_t per_img_slot, int& C0, uint8_t*& arena) {
+    Xfer& X = m->xfer;
+    std::lock_guard<std::mutex> lock(m->mu);
+    BCAD_TRY(xfer_init(m));
+    C0 = (int)std::max<size_t>(1, std::min<size_t>((size_t)host_chunk(m, B, 128), kClassesStagingBytes / (2 * per_img_slot)));
+    const size_t need = 2 * (size_t)C0 * per_img_slot;
+    if (X.cls_arena_bytes < need) {
+        if (X.cls_arena != nullptr) {                     // replaced, not kept until destroy: it can be hundreds of MB
+            BCAD_CUDA_CHECK(cudaFree(X.cls_arena));       // (synchronises the device: no earlier call still reads it)
+            m->allocs.erase(std::find(m->allocs.begin(), m->allocs.end(), X.cls_arena));
+            m->ws_bytes -= X.cls_arena_bytes;
+            X.cls_arena = nullptr;
+            X.cls_arena_bytes = 0;
+        }
+        BCAD_TRY(m->alloc(&X.cls_arena, need));
+        X.cls_arena_bytes = need;
+    }
+    arena = reinterpret_cast<uint8_t*>(X.cls_arena);
+    return BCAD_OK;
+}
+
 }  // namespace bcad
 
 extern "C" {
@@ -919,180 +1159,8 @@ int bcad_get_tensor(bcad_model* mm, int kind, int index, int B, float* dst, void
 }
 
 // -----------------------------------------------------------------------------------------------------
-// host-buffer end-to-end call: H2D / compute / D2H in chunks on three streams, double-buffered
+// host-buffer calls: chunked over three streams by host_pipeline
 // -----------------------------------------------------------------------------------------------------
-// streams, events and the model-size slot buffers of the pipeline, on first use (caller holds m->mu)
-static int xfer_init(Model* m) {
-    Xfer& X = m->xfer;
-    if (X.inited) return BCAD_OK;
-    const size_t img = (size_t)m->cfg.in_h * m->cfg.in_w * m->cfg.in_c, hm = (size_t)m->cfg.in_h * m->cfg.in_w;
-    int chunk = std::min(m->cfg.max_batch, 128);
-    if (const char* e = getenv("BCAD_HOST_CHUNK")) chunk = std::max(1, std::min(m->cfg.max_batch, atoi(e)));
-    BCAD_CUDA_CHECK(cudaStreamCreateWithFlags(&X.s_in, cudaStreamNonBlocking));
-    BCAD_CUDA_CHECK(cudaStreamCreateWithFlags(&X.s_compute, cudaStreamNonBlocking));
-    BCAD_CUDA_CHECK(cudaStreamCreateWithFlags(&X.s_out, cudaStreamNonBlocking));
-    for (int i = 0; i < 2; ++i) {
-        BCAD_CUDA_CHECK(cudaEventCreateWithFlags(&X.in_done[i], cudaEventDisableTiming));
-        BCAD_CUDA_CHECK(cudaEventCreateWithFlags(&X.compute_done[i], cudaEventDisableTiming));
-        BCAD_CUDA_CHECK(cudaEventCreateWithFlags(&X.out_done[i], cudaEventDisableTiming));
-        BCAD_TRY(m->alloc((void**)&X.x[i], (size_t)chunk * img * sizeof(float)));
-        BCAD_TRY(m->alloc((void**)&X.heat[i], (size_t)chunk * hm * sizeof(float)));
-        BCAD_TRY(m->alloc((void**)&X.cidx[i], (size_t)chunk * sizeof(int32_t)));
-    }
-    X.chunk = chunk;
-    X.inited = true;
-    return BCAD_OK;
-}
-
-// small outputs (logits, probabilities, classes) go through pinned staging sized for the whole call (caller holds m->host_mu)
-static int stage_small(Model* m, size_t bytes) {
-    Xfer& X = m->xfer;
-    if (X.h_small_bytes < bytes) {
-        if (X.h_small) cudaFreeHost(X.h_small);
-        X.h_small = nullptr;
-        X.h_small_bytes = 0;
-        BCAD_CUDA_CHECK(cudaMallocHost(&X.h_small, bytes));
-        X.h_small_bytes = bytes;
-    }
-    if (X.d_small_bytes < bytes) {
-        std::lock_guard<std::mutex> lock(m->mu);             // grows only when a call is larger than every call before it; the handle
-        X.d_small = nullptr;                                 // owns (and frees at destroy) the smaller ones it replaces: tens of bytes per image
-        X.d_small_bytes = 0;
-        BCAD_TRY(m->alloc(&X.d_small, bytes));
-        X.d_small_bytes = bytes;
-    }
-    return BCAD_OK;
-}
-
-static int predict_explain_host_impl(bcad_model* mm, const float* x_host, const uint8_t* x8_host, int B, const int32_t* class_idx_host,
-                                     int grad_mode, float* logits_host, float* probs_host, int32_t* cls_host, float* heat_host,
-                                     uint8_t* heat_u8_host, const uint8_t* gray8_host = nullptr, int standardise = 0,
-                                     uint8_t* overlay_host = nullptr) {
-    Model* m = reinterpret_cast<Model*>(mm);
-    BCAD_REQUIRE(m && (x_host || x8_host || gray8_host), "predict_explain_host: null argument");
-    BCAD_REQUIRE(B >= 1, "batch must be >= 1, got %d", B);
-    if (!m->committed) { set_error("weights not committed: call bcad_commit first"); return BCAD_ERR_STATE; }
-    BCAD_REQUIRE(grad_mode == BCAD_GRAD_LOGIT || grad_mode == BCAD_GRAD_SOFTMAX_CE, "bad grad_mode %d", grad_mode);
-    if (class_idx_host != nullptr)
-        for (int b = 0; b < B; ++b)
-            BCAD_REQUIRE(class_idx_host[b] >= 0 && class_idx_host[b] < m->cfg.num_classes, "class_idx[%d] = %d is outside [0, %d)", b,
-                         class_idx_host[b], m->cfg.num_classes);
-    DeviceGuard g(m->cfg.device);
-    // one host-buffer call at a time per handle: the three streams, the double-buffered device slots, the events and the pinned
-    // staging are shared (threaded callers -- a Flask app with one model -- queue here; separate handles run concurrently)
-    std::lock_guard<std::mutex> host_lock(m->host_mu);
-    Xfer& X = m->xfer;
-    const int nc = m->cfg.num_classes;
-    const size_t img = (size_t)m->cfg.in_h * m->cfg.in_w * m->cfg.in_c, hm = (size_t)m->cfg.in_h * m->cfg.in_w;
-    // transfer/compute chunk: small enough that the PCIe pipeline fills quickly (the link, ~52 GB/s per direction, is the
-    // end-to-end bound), large enough to keep the kernels efficient.  BCAD_HOST_CHUNK overrides (tuning).
-    // Buffers are sized for 128 images; a call uses about a quarter of its batch per chunk (32..128 images: measured at 512
-    // images, float32 in/out 3.6-3.7 ms with 64, 3.7-3.8 with 128; 8-bit in/out 2.11 ms with 64, 1.73 ms with 128, 1.80 ms with 256).
-    {
-        std::lock_guard<std::mutex> lock(m->mu);
-        BCAD_TRY(xfer_init(m));
-        if (heat_u8_host != nullptr && X.heat8[0] == nullptr)
-            for (int i = 0; i < 2; ++i) BCAD_TRY(m->alloc((void**)&X.heat8[i], (size_t)X.chunk * hm));
-        if ((x8_host != nullptr || gray8_host != nullptr) && X.x8[0] == nullptr)
-            for (int i = 0; i < 2; ++i) BCAD_TRY(m->alloc((void**)&X.x8[i], (size_t)X.chunk * img));
-        if (gray8_host != nullptr && X.img01[0] == nullptr)
-            for (int i = 0; i < 2; ++i) {
-                BCAD_TRY(m->alloc((void**)&X.img01[i], (size_t)X.chunk * hm * sizeof(float)));
-                BCAD_TRY(m->alloc((void**)&X.ov8[i], (size_t)X.chunk * hm * 3));
-            }
-    }
-    const size_t per_img = (size_t)(2 * nc) * sizeof(float) + sizeof(int32_t);
-    BCAD_TRY(stage_small(m, per_img * B));
-    float* st_logits = reinterpret_cast<float*>(X.h_small);
-    float* st_probs = st_logits + (size_t)B * nc;
-    int32_t* st_cls = reinterpret_cast<int32_t*>(st_probs + (size_t)B * nc);
-    float* dv_logits = reinterpret_cast<float*>(X.d_small);
-    float* dv_probs = dv_logits + (size_t)B * nc;
-    int32_t* dv_cls = reinterpret_cast<int32_t*>(dv_probs + (size_t)B * nc);
-    // chunk schedule: ramp up and down (C/4, C/2, C, ..., C, C/2, C/4) so the un-overlapped head (first H2D + compute) and
-    // tail (last D2H) of the pipeline are short; the steady state runs H2D, compute and D2H of three chunks concurrently
-    std::vector<int> sizes;
-    {
-        int C0 = X.chunk;
-        // float32 images: the link is the bound and 64-image chunks fill the pipeline sooner; 8-bit images: compute is the bound
-        // and 128-image chunks run the kernels more efficiently
-        if (getenv("BCAD_HOST_CHUNK") == nullptr)
-            C0 = std::min(std::min(X.chunk, (x8_host || gray8_host) ? 128 : 64), std::max(32, ((B + 3) / 4 + 31) / 32 * 32));
-        int left = B;
-        std::vector<int> head, tail;
-        // measured on the bench workload (512 images): uniform 64-image chunks 3.62 ms, ramped 3.93 ms -- the small
-        // chunks cost more in per-chunk launch/sync overhead than they save; the ramp stays available for tuning
-        const char* ramp = getenv("BCAD_HOST_RAMP");
-        if (ramp && atoi(ramp) == 1 && B >= 4 * C0 && C0 >= 8) {
-            head = {C0 / 4, C0 / 2};
-            tail = {C0 / 2, C0 / 4};
-        } else if (ramp && atoi(ramp) == 2 && B >= 4 * C0 && C0 >= 8) {
-            head = {C0 / 2};
-            tail = {C0 / 2};
-        }
-        // tuning: an explicit schedule, e.g. "64,192,192,64" (must sum to B; buffers via BCAD_HOST_CHUNK).  Measured at 512 images,
-        // 8-bit in/out: 4 x 128 1.64 ms, 64,192,192,64 1.58 ms, 8 x 64 1.99 ms -- ramps buy 4 %, not worth 2x the staging memory
-        if (const char* e = getenv("BCAD_HOST_SIZES")) {
-            std::vector<int> v;
-            int sum = 0;
-            for (const char* q = e; *q;) {
-                const int k = atoi(q);
-                if (k < 1 || k > X.chunk) { v.clear(); break; }
-                v.push_back(k);
-                sum += k;
-                while (*q && *q != ',') ++q;
-                if (*q == ',') ++q;
-            }
-            if (!v.empty() && sum == B) { sizes = v; left = 0; head.clear(); tail.clear(); }
-        }
-        for (int v : head) { sizes.push_back(v); left -= v; }
-        int tail_sum = 0;
-        for (int v : tail) tail_sum += v;
-        while (left - tail_sum > 0) { const int v = std::min(C0, left - tail_sum); sizes.push_back(v); left -= v; }
-        for (int v : tail) { sizes.push_back(v); left -= v; }
-    }
-    int b0 = 0;
-    for (int c = 0; c < (int)sizes.size(); b0 += sizes[c], ++c) {
-        const int slot = c & 1, n = sizes[c];
-        // slot reuse: its previous D2H (chunk c-2) must have drained before we overwrite its buffers
-        if (c >= 2) {
-            BCAD_CUDA_CHECK(cudaStreamWaitEvent(X.s_in, X.compute_done[slot], 0));
-            BCAD_CUDA_CHECK(cudaStreamWaitEvent(X.s_compute, X.out_done[slot], 0));
-        }
-        if (gray8_host) BCAD_CUDA_CHECK(cudaMemcpyAsync(X.x8[slot], gray8_host + (size_t)b0 * hm, (size_t)n * hm, cudaMemcpyHostToDevice, X.s_in));
-        else if (x8_host) BCAD_CUDA_CHECK(cudaMemcpyAsync(X.x8[slot], x8_host + (size_t)b0 * img, (size_t)n * img, cudaMemcpyHostToDevice, X.s_in));
-        else BCAD_CUDA_CHECK(cudaMemcpyAsync(X.x[slot], x_host + (size_t)b0 * img, (size_t)n * img * sizeof(float), cudaMemcpyHostToDevice, X.s_in));
-        if (class_idx_host)
-            BCAD_CUDA_CHECK(cudaMemcpyAsync(X.cidx[slot], class_idx_host + b0, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, X.s_in));
-        BCAD_CUDA_CHECK(cudaEventRecord(X.in_done[slot], X.s_in));
-        BCAD_CUDA_CHECK(cudaStreamWaitEvent(X.s_compute, X.in_done[slot], 0));
-        const bool want_heat = (heat_host != nullptr || heat_u8_host != nullptr || overlay_host != nullptr);
-        int rc = BCAD_OK;
-        if (gray8_host) rc = launch_gray_preprocess(X.x8[slot], X.img01[slot], X.x[slot], n, (int)hm, m->cfg.in_c, standardise, X.s_compute);
-        else if (x8_host) rc = launch_u8_to_unit(X.x8[slot], X.x[slot], (size_t)n * img, X.s_compute);
-        if (rc == BCAD_OK) rc = run(m, X.x[slot], n, class_idx_host ? X.cidx[slot] : nullptr, grad_mode, want_heat, dv_logits + (size_t)b0 * nc,
-                     dv_probs + (size_t)b0 * nc, dv_cls + b0, X.heat[slot], X.s_compute);
-        if (rc == BCAD_OK && overlay_host != nullptr)             // show_cam_on_image + heatmap_uint8 in one pass (GRADCAM.py:67,70)
-            rc = launch_overlay(X.img01[slot], X.heat[slot], n, m->cfg.in_h, m->cfg.in_w, X.ov8[slot], heat_u8_host ? X.heat8[slot] : nullptr, X.s_compute);
-        else if (rc == BCAD_OK && heat_u8_host != nullptr) rc = launch_heat_to_u8(X.heat[slot], X.heat8[slot], (size_t)n * hm, X.s_compute);
-        if (rc != BCAD_OK) { cudaDeviceSynchronize(); return rc; }
-        BCAD_CUDA_CHECK(cudaEventRecord(X.compute_done[slot], X.s_compute));
-        BCAD_CUDA_CHECK(cudaStreamWaitEvent(X.s_out, X.compute_done[slot], 0));
-        if (heat_host) BCAD_CUDA_CHECK(cudaMemcpyAsync(heat_host + (size_t)b0 * hm, X.heat[slot], (size_t)n * hm * sizeof(float), cudaMemcpyDeviceToHost, X.s_out));
-        if (heat_u8_host) BCAD_CUDA_CHECK(cudaMemcpyAsync(heat_u8_host + (size_t)b0 * hm, X.heat8[slot], (size_t)n * hm, cudaMemcpyDeviceToHost, X.s_out));
-        if (overlay_host) BCAD_CUDA_CHECK(cudaMemcpyAsync(overlay_host + (size_t)b0 * hm * 3, X.ov8[slot], (size_t)n * hm * 3, cudaMemcpyDeviceToHost, X.s_out));
-        if (c + 1 == (int)sizes.size())                       // the small outputs of the whole call, once, behind the last chunk
-            BCAD_CUDA_CHECK(cudaMemcpyAsync(X.h_small, X.d_small, per_img * B, cudaMemcpyDeviceToHost, X.s_out));
-        BCAD_CUDA_CHECK(cudaEventRecord(X.out_done[slot], X.s_out));
-    }
-    BCAD_CUDA_CHECK(cudaStreamSynchronize(X.s_out));
-    BCAD_CUDA_CHECK(cudaStreamSynchronize(X.s_compute));
-    if (logits_host) memcpy(logits_host, st_logits, (size_t)B * nc * sizeof(float));
-    if (probs_host) memcpy(probs_host, st_probs, (size_t)B * nc * sizeof(float));
-    if (cls_host) memcpy(cls_host, st_cls, (size_t)B * sizeof(int32_t));
-    return BCAD_OK;
-}
-
 int bcad_predict_explain_host(bcad_model* mm, const float* x_host, int B, const int32_t* class_idx_host, int grad_mode,
                               float* logits_host, float* probs_host, int32_t* cls_host, float* heat_host) {
     return predict_explain_host_impl(mm, x_host, nullptr, B, class_idx_host, grad_mode, logits_host, probs_host, cls_host, heat_host, nullptr);
@@ -1119,119 +1187,6 @@ int bcad_gradcam_overlays_host(bcad_model* mm, const uint8_t* gray_u8_host, int 
     return predict_explain_host_impl(mm, nullptr, nullptr, B, class_idx_host, grad_mode, logits_host, probs_host, cls_host, nullptr,
                                      heat_u8_host, gray_u8_host, standardise, overlay_rgb_host);
 }
-
-// Staging bound of the host-buffer classes calls (bcad_gradcam_overlays_classes_host, bcad_saliency_overlays_classes_host): both slots'
-// 8-bit images, classes and maps stay within this many bytes of the handle's memory (the chunk shrinks to fit; a single image larger
-// than half of it still runs, one image per chunk).  Grad-CAM, 512 x 512 images with K = 2: 4.25 MB per image and slot, chunks of up
-// to 60 images.
-static const size_t kClassesStagingBytes = (size_t)512 << 20;
-
-static size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
-
-// The checks shared by the classes calls, all made before any copy.  fn names the call in the messages.
-static int check_classes_host(const char* fn, Model* m, const uint8_t* gray_u8_host, int B, int img_h, int img_w, int K,
-                              const int32_t* classes_host_or_null, int grad_mode, int standardise, bool any_output) {
-    BCAD_REQUIRE(m && gray_u8_host, "%s: null model or image pointer", fn);
-    BCAD_REQUIRE(any_output, "%s: the output pointers are all null", fn);
-    BCAD_REQUIRE(B >= 1, "batch must be >= 1, got %d", B);
-    BCAD_REQUIRE(img_h >= 1 && img_w >= 1 && img_h <= 16384 && img_w <= 16384, "%s: bad image size %dx%d", fn, img_h, img_w);
-    BCAD_REQUIRE(K >= 1 && K <= BCAD_MAX_EXPLAIN_CLASSES, "%s: K=%d out of range 1..%d", fn, K, BCAD_MAX_EXPLAIN_CLASSES);
-    BCAD_REQUIRE(standardise == 0 || standardise == 1, "%s: standardise must be 0 or 1", fn);
-    BCAD_REQUIRE(grad_mode == BCAD_GRAD_LOGIT || grad_mode == BCAD_GRAD_SOFTMAX_CE, "bad grad_mode %d", grad_mode);
-    const int nc = m->cfg.num_classes;
-    BCAD_REQUIRE(classes_host_or_null || K <= nc, "%s: classes=NULL explains classes 0..K-1, but K=%d > num_classes=%d", fn, K, nc);
-    if (classes_host_or_null != nullptr)
-        for (size_t i = 0; i < (size_t)B * K; ++i)
-            BCAD_REQUIRE(classes_host_or_null[i] >= 0 && classes_host_or_null[i] < nc, "classes[%zu][%zu] = %d is outside [0, %d)", i / K, i % K,
-                         classes_host_or_null[i], nc);
-    if (!m->committed) { set_error("weights not committed: call bcad_commit first"); return BCAD_ERR_STATE; }
-    return BCAD_OK;
-}
-
-// Chunk size of a classes call and the arena holding both slots of per_img_slot bytes per image (caller holds m->host_mu): the chunk of
-// bcad_gradcam_overlays_host (a quarter of the batch, 32..128 images), shrunk to the staging bound.  Slot i starts at
-// arena + i * C0 * per_img_slot.
-static int classes_staging(Model* m, int B, size_t per_img_slot, int& C0, uint8_t*& arena) {
-    Xfer& X = m->xfer;
-    std::lock_guard<std::mutex> lock(m->mu);
-    BCAD_TRY(xfer_init(m));
-    C0 = std::min(std::min(X.chunk, 128), std::max(32, ((B + 3) / 4 + 31) / 32 * 32));
-    if (const char* e = getenv("BCAD_HOST_CHUNK")) C0 = std::max(1, std::min(X.chunk, atoi(e)));
-    C0 = (int)std::max<size_t>(1, std::min<size_t>((size_t)C0, kClassesStagingBytes / (2 * per_img_slot)));
-    const size_t need = 2 * (size_t)C0 * per_img_slot;
-    if (X.cls_arena_bytes < need) {
-        if (X.cls_arena != nullptr) {                     // replaced, not kept until destroy: it can be hundreds of MB
-            BCAD_CUDA_CHECK(cudaFree(X.cls_arena));       // (synchronises the device: no earlier call still reads it)
-            m->allocs.erase(std::find(m->allocs.begin(), m->allocs.end(), X.cls_arena));
-            m->ws_bytes -= X.cls_arena_bytes;
-            X.cls_arena = nullptr;
-            X.cls_arena_bytes = 0;
-        }
-        BCAD_TRY(m->alloc(&X.cls_arena, need));
-        X.cls_arena_bytes = need;
-    }
-    arena = reinterpret_cast<uint8_t*>(X.cls_arena);
-    return BCAD_OK;
-}
-
-// logits / probabilities / classes of a whole classes call: written on the device per chunk, brought back by one copy behind the last
-// chunk through the pinned staging of stage_small
-struct SmallOutputs {
-    size_t bytes = 0;
-    float *dv_logits = nullptr, *dv_probs = nullptr;
-    int32_t* dv_cls = nullptr;
-};
-
-static int small_outputs(Model* m, int B, SmallOutputs& o) {
-    const int nc = m->cfg.num_classes;
-    o.bytes = ((size_t)(2 * nc) * sizeof(float) + sizeof(int32_t)) * B;
-    BCAD_TRY(stage_small(m, o.bytes));
-    o.dv_logits = reinterpret_cast<float*>(m->xfer.d_small);
-    o.dv_probs = o.dv_logits + (size_t)B * nc;
-    o.dv_cls = reinterpret_cast<int32_t*>(o.dv_probs + (size_t)B * nc);
-    return BCAD_OK;
-}
-
-static void copy_small_outputs(Model* m, int B, float* logits_host, float* probs_host, int32_t* cls_host) {
-    const int nc = m->cfg.num_classes;
-    const float* st_logits = reinterpret_cast<const float*>(m->xfer.h_small);
-    const float* st_probs = st_logits + (size_t)B * nc;
-    const int32_t* st_cls = reinterpret_cast<const int32_t*>(st_probs + (size_t)B * nc);
-    if (logits_host) memcpy(logits_host, st_logits, (size_t)B * nc * sizeof(float));
-    if (probs_host) memcpy(probs_host, st_probs, (size_t)B * nc * sizeof(float));
-    if (cls_host) memcpy(cls_host, st_cls, (size_t)B * sizeof(int32_t));
-}
-
-// The chunk loop of the classes calls: per chunk c (slot c & 1, images b0 .. b0 + n) h2d(slot, b0, n) on s_in, compute(slot, b0, n) on
-// s_compute, d2h(slot, b0, n) on s_out, ordered by the slot's events; the small outputs follow the last chunk's D2H.  Returns after
-// both streams have drained.
-extern "C++" {
-template <class H2D, class Compute, class D2H>
-static int classes_pipeline(Model* m, int B, int C0, const SmallOutputs& so, H2D h2d, Compute compute, D2H d2h) {
-    Xfer& X = m->xfer;
-    const int nchunks = (B + C0 - 1) / C0;
-    for (int c = 0, b0 = 0; c < nchunks; ++c, b0 += C0) {
-        const int slot = c & 1, n = std::min(C0, B - b0);
-        if (c >= 2) {                                         // slot reuse, as in predict_explain_host_impl
-            BCAD_CUDA_CHECK(cudaStreamWaitEvent(X.s_in, X.compute_done[slot], 0));
-            BCAD_CUDA_CHECK(cudaStreamWaitEvent(X.s_compute, X.out_done[slot], 0));
-        }
-        BCAD_TRY(h2d(slot, b0, n));
-        BCAD_CUDA_CHECK(cudaEventRecord(X.in_done[slot], X.s_in));
-        BCAD_CUDA_CHECK(cudaStreamWaitEvent(X.s_compute, X.in_done[slot], 0));
-        const int rc = compute(slot, b0, n);
-        if (rc != BCAD_OK) { cudaDeviceSynchronize(); return rc; }
-        BCAD_CUDA_CHECK(cudaEventRecord(X.compute_done[slot], X.s_compute));
-        BCAD_CUDA_CHECK(cudaStreamWaitEvent(X.s_out, X.compute_done[slot], 0));
-        BCAD_TRY(d2h(slot, b0, n));
-        if (c + 1 == nchunks) BCAD_CUDA_CHECK(cudaMemcpyAsync(X.h_small, X.d_small, so.bytes, cudaMemcpyDeviceToHost, X.s_out));
-        BCAD_CUDA_CHECK(cudaEventRecord(X.out_done[slot], X.s_out));
-    }
-    BCAD_CUDA_CHECK(cudaStreamSynchronize(X.s_out));
-    BCAD_CUDA_CHECK(cudaStreamSynchronize(X.s_compute));
-    return BCAD_OK;
-}
-}  // extern "C++"
 
 int bcad_gradcam_overlays_classes_host(bcad_model* mm, const uint8_t* gray_u8_host, int B, int img_h, int img_w, int K,
                                        const int32_t* classes_host_or_null, int grad_mode, int standardise, float* logits_host,
@@ -1264,7 +1219,7 @@ int bcad_gradcam_overlays_classes_host(bcad_model* mm, const uint8_t* gray_u8_ho
     }
     SmallOutputs so;
     BCAD_TRY(small_outputs(m, B, so));
-    BCAD_TRY(classes_pipeline(m, B, C0, so,
+    BCAD_TRY(host_pipeline(m, B, C0, so,
         [&](int slot, int b0, int n) {
             BCAD_CUDA_CHECK(cudaMemcpyAsync(d_img[slot], gray_u8_host + (size_t)b0 * hw, (size_t)n * hw, cudaMemcpyHostToDevice, X.s_in));
             if (classes_host_or_null)
@@ -1330,7 +1285,7 @@ int bcad_saliency_overlays_classes_host(bcad_model* mm, const uint8_t* gray_u8_h
     }
     SmallOutputs so;
     BCAD_TRY(small_outputs(m, B, so));
-    BCAD_TRY(classes_pipeline(m, B, C0, so,
+    BCAD_TRY(host_pipeline(m, B, C0, so,
         [&](int slot, int b0, int n) {
             BCAD_CUDA_CHECK(cudaMemcpyAsync(d_img[slot], gray_u8_host + (size_t)b0 * hw, (size_t)n * hw, cudaMemcpyHostToDevice, X.s_in));
             if (classes_host_or_null)

@@ -66,6 +66,58 @@ def _f32c(a) -> np.ndarray:
     return np.ascontiguousarray(np.asarray(a), dtype=np.float32)
 
 
+def _stream_of(device):
+    return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
+
+
+def _gray_batch(gray_u8) -> np.ndarray:
+    """uint8 grey images [B,H,W] or [H,W] -> a C-contiguous uint8 [B,H,W] array."""
+    g = np.ascontiguousarray(gray_u8)
+    if g.dtype != np.uint8:
+        raise ValueError("gray_u8 must be uint8 (0-255 grey levels)")
+    if g.ndim == 2:
+        g = g[None]
+    if g.ndim != 3:
+        raise ValueError(f"gray_u8 must be [B,H,W] or [H,W], got shape {g.shape}")
+    return g
+
+
+def _out_array(out, shape, dtype, name):
+    a = out if out is not None else np.empty(shape, dtype)
+    if a.dtype != dtype or a.shape != shape or not a.flags["C_CONTIGUOUS"]:
+        raise ValueError(f"{name} must be a C-contiguous {np.dtype(dtype).name} array of shape {shape}")
+    return a
+
+
+def _host_class_idx(class_idx, B, nc):
+    """class_idx of the single-class host calls (None, one class or one per image) -> C-contiguous int32 [B] array or None."""
+    if class_idx is None:
+        return None
+    ci = np.ascontiguousarray(np.broadcast_to(np.asarray(class_idx, dtype=np.int32).reshape(-1), (B,)))
+    if ci.min() < 0 or ci.max() >= nc:
+        raise ValueError("class_idx out of range")
+    return ci
+
+
+def _host_class_rows(classes, B, nc):
+    """classes of the host multi-class calls -> (K, C-contiguous int32 [B,K] array or None = column k is class k)."""
+    if classes is None:
+        K, ci = nc, None
+    else:
+        ci = np.asarray(classes, dtype=np.int32)
+        if ci.ndim == 1:
+            ci = np.broadcast_to(ci[None], (B, ci.shape[0]))
+        if ci.ndim != 2 or ci.shape[0] != B:
+            raise ValueError(f"classes must be a length-K sequence or a [{B},K] array, got shape {ci.shape}")
+        K = ci.shape[1]
+        if K >= 1 and (int(ci.min()) < 0 or int(ci.max()) >= nc):
+            raise ValueError("classes out of range")
+        ci = np.ascontiguousarray(ci)
+    if not 1 <= K <= _lib.MAX_EXPLAIN_CLASSES:
+        raise ValueError(f"{K} target classes per image; 1..{_lib.MAX_EXPLAIN_CLASSES} are supported")
+    return K, ci
+
+
 class Engine:
     """One libbcad handle on one GPU."""
 
@@ -167,7 +219,7 @@ class Engine:
 
     # ------------------------------------------------------------------ helpers
     def _stream(self):
-        return C.c_void_p(torch.cuda.current_stream(self.tdev).cuda_stream)
+        return _stream_of(self.tdev)
 
     def _as_device_input(self, x) -> torch.Tensor:
         h, w, c = self.spec.input_shape
@@ -482,19 +534,9 @@ class Engine:
         if x.shape[1:] != (h, w, c):
             raise ValueError(f"input shape {x.shape} does not match [B,{h},{w},{c}]")
         B, nc = x.shape[0], self.spec.num_classes
-        logits = np.empty((B, nc), np.float32)
-        probs = np.empty((B, nc), np.float32)
-        cls = np.empty((B,), np.int32)
-        heat = None
-        if want_heat:
-            heat = heat_out if heat_out is not None else np.empty((B, h, w), np.uint8 if u8 else np.float32)
-            if heat.dtype != (np.uint8 if u8 else np.float32) or not heat.flags["C_CONTIGUOUS"]:
-                raise ValueError("heat_out must be a C-contiguous array of heat_dtype")
-        ci = None
-        if class_idx is not None:
-            ci = np.ascontiguousarray(np.broadcast_to(np.asarray(class_idx, dtype=np.int32).reshape(-1), (B,)))
-            if ci.min() < 0 or ci.max() >= nc:
-                raise ValueError("class_idx out of range")
+        logits, probs, cls = np.empty((B, nc), np.float32), np.empty((B, nc), np.float32), np.empty((B,), np.int32)
+        heat = _out_array(heat_out, (B, h, w), np.uint8 if u8 else np.float32, "heat_out") if want_heat else None
+        ci = _host_class_idx(class_idx, B, nc)
         if x8:
             hf, h8 = (None, heat) if u8 else (heat, None)
             _lib.check(self.lib.bcad_predict_explain_host_u8in(self._h, _ptr(x), B, _ptr(ci), _lib.GRAD_MODE[grad_mode], _ptr(logits),
@@ -504,150 +546,74 @@ class Engine:
         _lib.check(fn(self._h, _ptr(x), B, _ptr(ci), _lib.GRAD_MODE[grad_mode], _ptr(logits), _ptr(probs), _ptr(cls), _ptr(heat)))
         return cls, probs, logits, heat
 
+    def gradcam_overlays_host(self, gray_u8: np.ndarray, class_idx=None, grad_mode: str = "logit", standardise: bool = True,
+                              overlay_out: Optional[np.ndarray] = None, heat_out: Optional[np.ndarray] = None,
+                              want_overlay: bool = True, want_heat: bool = True):
+        """The GRADCAM.py call surface for a batch, end to end through one C-ABI call (bcad_gradcam_overlays_host): uint8 grey
+        images [B,H,W] (model input size) -> (cls int32 [B], probs [B,nc], logits [B,nc], overlay uint8 RGB [B,H,W,3] =
+        show_cam_on_image, heatmap_uint8 [B,H,W]).  ``standardise``: the CNN input is the per-image standardised img/255 (the
+        reference's CNN-input normalisation, app.py:179-182), else img/255 itself.  Pinned host arrays make the copies asynchronous."""
+        self.cache_tag = None
+        h, w, _ = self.spec.input_shape
+        g = _gray_batch(gray_u8)
+        if g.shape[1:] != (h, w):
+            raise ValueError(f"image shape {g.shape} does not match [B,{h},{w}]")
+        B, nc = g.shape[0], self.spec.num_classes
+        logits, probs, cls = np.empty((B, nc), np.float32), np.empty((B, nc), np.float32), np.empty((B,), np.int32)
+        ov = _out_array(overlay_out, (B, h, w, 3), np.uint8, "overlay_out") if want_overlay else None
+        hu = _out_array(heat_out, (B, h, w), np.uint8, "heat_out") if want_heat else None
+        ci = _host_class_idx(class_idx, B, nc)
+        _lib.check(self.lib.bcad_gradcam_overlays_host(self._h, _ptr(g), B, _ptr(ci), _lib.GRAD_MODE[grad_mode], 1 if standardise else 0,
+                                                       _ptr(logits), _ptr(probs), _ptr(cls), _ptr(ov), _ptr(hu)))
+        return cls, probs, logits, ov, hu
 
-def _gradcam_overlays_host(self, gray_u8: np.ndarray, class_idx=None, grad_mode: str = "logit", standardise: bool = True,
-                           overlay_out: Optional[np.ndarray] = None, heat_out: Optional[np.ndarray] = None,
-                           want_overlay: bool = True, want_heat: bool = True):
-    """The GRADCAM.py call surface for a batch, end to end through one C-ABI call (bcad_gradcam_overlays_host): uint8 grey
-    images [B,H,W] (model input size) -> (cls int32 [B], probs [B,nc], logits [B,nc], overlay uint8 RGB [B,H,W,3] =
-    show_cam_on_image, heatmap_uint8 [B,H,W]).  ``standardise``: the CNN input is the per-image standardised img/255 (the
-    reference's CNN-input normalisation, app.py:179-182), else img/255 itself.  Pinned host arrays make the copies asynchronous."""
-    self.cache_tag = None
-    h, w, c = self.spec.input_shape
-    g = np.ascontiguousarray(gray_u8)
-    if g.dtype != np.uint8:
-        raise ValueError("gray_u8 must be uint8 (0-255 grey levels)")
-    if g.ndim == 2:
-        g = g[None]
-    if g.shape[1:] != (h, w):
-        raise ValueError(f"image shape {g.shape} does not match [B,{h},{w}]")
-    B, nc = g.shape[0], self.spec.num_classes
-    logits, probs, cls = np.empty((B, nc), np.float32), np.empty((B, nc), np.float32), np.empty((B,), np.int32)
-    ov = hu = None
-    if want_overlay:
-        ov = overlay_out if overlay_out is not None else np.empty((B, h, w, 3), np.uint8)
-    if want_heat:
-        hu = heat_out if heat_out is not None else np.empty((B, h, w), np.uint8)
-    for a, shp in ((ov, (B, h, w, 3)), (hu, (B, h, w))):
-        if a is not None and (a.dtype != np.uint8 or a.shape != shp or not a.flags["C_CONTIGUOUS"]):
-            raise ValueError("output arrays must be C-contiguous uint8 of the documented shape")
-    ci = None
-    if class_idx is not None:
-        ci = np.ascontiguousarray(np.broadcast_to(np.asarray(class_idx, dtype=np.int32).reshape(-1), (B,)))
-        if ci.min() < 0 or ci.max() >= nc:
-            raise ValueError("class_idx out of range")
-    _lib.check(self.lib.bcad_gradcam_overlays_host(self._h, _ptr(g), B, _ptr(ci), _lib.GRAD_MODE[grad_mode], 1 if standardise else 0,
-                                                   _ptr(logits), _ptr(probs), _ptr(cls), _ptr(ov), _ptr(hu)))
-    return cls, probs, logits, ov, hu
+    def gradcam_overlays_classes_host(self, gray_u8: np.ndarray, classes=(0, 1), grad_mode: str = "logit", standardise: bool = True,
+                                      overlay_out: Optional[np.ndarray] = None, heat_out: Optional[np.ndarray] = None,
+                                      want_overlay: bool = True, want_heat: bool = True):
+        """The deployed dual-class call (app.py:649-657 -> GRADCAM.py:31-81) for a batch, end to end through one C-ABI call
+        (bcad_gradcam_overlays_classes_host): uint8 grey images [B,h,w] of ANY size -> (cls int32 [B], probs [B,nc], logits [B,nc],
+        overlay uint8 RGB [B,K,h,w,3] = show_cam_on_image, heatmap_uint8 [B,K,h,w]).  The CNN sees cv2.resize(img / 255, model size)
+        (standardised per image when ``standardise``); the maps have the size of the image.  ``classes``: a length-K sequence shared by
+        the batch, a [B,K] array or None (every class); K <= 8.  Pinned host arrays make the copies asynchronous."""
+        self.cache_tag = None
+        g = _gray_batch(gray_u8)
+        B, h, w = g.shape
+        nc = self.spec.num_classes
+        K, ci = _host_class_rows(classes, B, nc)
+        logits, probs, cls = np.empty((B, nc), np.float32), np.empty((B, nc), np.float32), np.empty((B,), np.int32)
+        ov = _out_array(overlay_out, (B, K, h, w, 3), np.uint8, "overlay_out") if want_overlay else None
+        hu = _out_array(heat_out, (B, K, h, w), np.uint8, "heat_out") if want_heat else None
+        _lib.check(self.lib.bcad_gradcam_overlays_classes_host(self._h, _ptr(g), B, h, w, K, _ptr(ci), _lib.GRAD_MODE[grad_mode],
+                                                               1 if standardise else 0, _ptr(logits), _ptr(probs), _ptr(cls), _ptr(ov),
+                                                               _ptr(hu)))
+        return cls, probs, logits, ov, hu
 
-
-Engine.gradcam_overlays_host = _gradcam_overlays_host
-
-
-def _host_class_rows(classes, B, nc):
-    """classes of the host multi-class calls -> (K, C-contiguous int32 [B,K] array or None = column k is class k)."""
-    if classes is None:
-        K, ci = nc, None
-    else:
-        ci = np.asarray(classes, dtype=np.int32)
-        if ci.ndim == 1:
-            ci = np.broadcast_to(ci[None], (B, ci.shape[0]))
-        if ci.ndim != 2 or ci.shape[0] != B:
-            raise ValueError(f"classes must be a length-K sequence or a [{B},K] array, got shape {ci.shape}")
-        K = ci.shape[1]
-        if K >= 1 and (int(ci.min()) < 0 or int(ci.max()) >= nc):
-            raise ValueError("classes out of range")
-        ci = np.ascontiguousarray(ci)
-    if not 1 <= K <= _lib.MAX_EXPLAIN_CLASSES:
-        raise ValueError(f"{K} target classes per image; 1..{_lib.MAX_EXPLAIN_CLASSES} are supported")
-    return K, ci
-
-
-def _gradcam_overlays_classes_host(self, gray_u8: np.ndarray, classes=(0, 1), grad_mode: str = "logit", standardise: bool = True,
-                                   overlay_out: Optional[np.ndarray] = None, heat_out: Optional[np.ndarray] = None,
-                                   want_overlay: bool = True, want_heat: bool = True):
-    """The deployed dual-class call (app.py:649-657 -> GRADCAM.py:31-81) for a batch, end to end through one C-ABI call
-    (bcad_gradcam_overlays_classes_host): uint8 grey images [B,h,w] of ANY size -> (cls int32 [B], probs [B,nc], logits [B,nc],
-    overlay uint8 RGB [B,K,h,w,3] = show_cam_on_image, heatmap_uint8 [B,K,h,w]).  The CNN sees cv2.resize(img / 255, model size)
-    (standardised per image when ``standardise``); the maps have the size of the image.  ``classes``: a length-K sequence shared by
-    the batch, a [B,K] array or None (every class); K <= 8.  Pinned host arrays make the copies asynchronous."""
-    self.cache_tag = None
-    g = np.ascontiguousarray(gray_u8)
-    if g.dtype != np.uint8:
-        raise ValueError("gray_u8 must be uint8 (0-255 grey levels)")
-    if g.ndim == 2:
-        g = g[None]
-    if g.ndim != 3:
-        raise ValueError(f"gray_u8 must be [B,H,W] or [H,W], got shape {g.shape}")
-    B, h, w = g.shape
-    nc = self.spec.num_classes
-    K, ci = _host_class_rows(classes, B, nc)
-    logits, probs, cls = np.empty((B, nc), np.float32), np.empty((B, nc), np.float32), np.empty((B,), np.int32)
-    ov = hu = None
-    if want_overlay:
-        ov = overlay_out if overlay_out is not None else np.empty((B, K, h, w, 3), np.uint8)
-    if want_heat:
-        hu = heat_out if heat_out is not None else np.empty((B, K, h, w), np.uint8)
-    for a, shp in ((ov, (B, K, h, w, 3)), (hu, (B, K, h, w))):
-        if a is not None and (a.dtype != np.uint8 or a.shape != shp or not a.flags["C_CONTIGUOUS"]):
-            raise ValueError(f"output arrays must be C-contiguous uint8 of shape {shp}")
-    _lib.check(self.lib.bcad_gradcam_overlays_classes_host(self._h, _ptr(g), B, h, w, K, _ptr(ci), _lib.GRAD_MODE[grad_mode],
-                                                           1 if standardise else 0, _ptr(logits), _ptr(probs), _ptr(cls), _ptr(ov),
-                                                           _ptr(hu)))
-    return cls, probs, logits, ov, hu
-
-
-Engine.gradcam_overlays_classes_host = _gradcam_overlays_classes_host
-
-
-def _gray_batch(gray_u8) -> np.ndarray:
-    """uint8 grey images [B,H,W] or [H,W] -> a C-contiguous uint8 [B,H,W] array."""
-    g = np.ascontiguousarray(gray_u8)
-    if g.dtype != np.uint8:
-        raise ValueError("gray_u8 must be uint8 (0-255 grey levels)")
-    if g.ndim == 2:
-        g = g[None]
-    if g.ndim != 3:
-        raise ValueError(f"gray_u8 must be [B,H,W] or [H,W], got shape {g.shape}")
-    return g
-
-
-def _out_array(out, shape, dtype, name):
-    a = out if out is not None else np.empty(shape, dtype)
-    if a.dtype != dtype or a.shape != shape or not a.flags["C_CONTIGUOUS"]:
-        raise ValueError(f"{name} must be a C-contiguous {np.dtype(dtype).name} array of shape {shape}")
-    return a
-
-
-def _saliency_overlays_classes_host(self, gray_u8: np.ndarray, classes=(0, 1), grad_mode: str = "softmax_ce", standardise: bool = True,
-                                    overlay_out: Optional[np.ndarray] = None, heat_out: Optional[np.ndarray] = None,
-                                    saliency_out: Optional[np.ndarray] = None, want_overlay: bool = True, want_heat: bool = True,
-                                    want_saliency: bool = False):
-    """The dual-class input-gradient saliency overlays (explainability.py:81-108) for a batch, end to end through one C-ABI call
-    (bcad_saliency_overlays_classes_host): uint8 grey images [B,h,w] of ANY size -> (cls int32 [B], probs [B,nc], logits [B,nc],
-    overlays uint8 BGR [B,K,h,w,3], heat-maps uint8 BGR [B,K,h,w,3], saliency fp32 [B,K,H,W] at the model's size or None).  The CNN
-    sees the input ``gradcam_overlays_classes_host`` builds (cv2.resize(img / 255, model size), standardised per image when
-    ``standardise``); each map is coloured with JET, resized to the image's size as cv2.resize does on 8-bit BGR, and blended 50/50 with
-    the grey image.  ``classes`` as in ``gradcam_overlays_classes_host``; ``grad_mode`` defaults to the reference's softmax
-    cross-entropy gradient.  fp32 engines with ``keep_all_activations`` (a model's ``saliency_engine``).  The saliency maps are copied
-    back only when ``want_saliency`` or ``saliency_out`` is given.  Pinned host arrays make the copies asynchronous."""
-    self.cache_tag = None
-    g = _gray_batch(gray_u8)
-    B, h, w = g.shape
-    H, W, _ = self.spec.input_shape
-    nc = self.spec.num_classes
-    K, ci = _host_class_rows(classes, B, nc)
-    logits, probs, cls = np.empty((B, nc), np.float32), np.empty((B, nc), np.float32), np.empty((B,), np.int32)
-    ov = _out_array(overlay_out, (B, K, h, w, 3), np.uint8, "overlay_out") if want_overlay else None
-    hm = _out_array(heat_out, (B, K, h, w, 3), np.uint8, "heat_out") if want_heat else None
-    sal = _out_array(saliency_out, (B, K, H, W), np.float32, "saliency_out") if (want_saliency or saliency_out is not None) else None
-    _lib.check(self.lib.bcad_saliency_overlays_classes_host(self._h, _ptr(g), B, h, w, K, _ptr(ci), _lib.GRAD_MODE[grad_mode],
-                                                            1 if standardise else 0, _ptr(logits), _ptr(probs), _ptr(cls), _ptr(sal),
-                                                            _ptr(ov), _ptr(hm)))
-    return cls, probs, logits, ov, hm, sal
-
-
-Engine.saliency_overlays_classes_host = _saliency_overlays_classes_host
+    def saliency_overlays_classes_host(self, gray_u8: np.ndarray, classes=(0, 1), grad_mode: str = "softmax_ce", standardise: bool = True,
+                                       overlay_out: Optional[np.ndarray] = None, heat_out: Optional[np.ndarray] = None,
+                                       saliency_out: Optional[np.ndarray] = None, want_overlay: bool = True, want_heat: bool = True,
+                                       want_saliency: bool = False):
+        """The dual-class input-gradient saliency overlays (explainability.py:81-108) for a batch, end to end through one C-ABI call
+        (bcad_saliency_overlays_classes_host): uint8 grey images [B,h,w] of ANY size -> (cls int32 [B], probs [B,nc], logits [B,nc],
+        overlays uint8 BGR [B,K,h,w,3], heat-maps uint8 BGR [B,K,h,w,3], saliency fp32 [B,K,H,W] at the model's size or None).  The CNN
+        sees the input ``gradcam_overlays_classes_host`` builds (cv2.resize(img / 255, model size), standardised per image when
+        ``standardise``); each map is coloured with JET, resized to the image's size as cv2.resize does on 8-bit BGR, and blended 50/50 with
+        the grey image.  ``classes`` as in ``gradcam_overlays_classes_host``; ``grad_mode`` defaults to the reference's softmax
+        cross-entropy gradient.  fp32 engines with ``keep_all_activations`` (a model's ``saliency_engine``).  The saliency maps are copied
+        back only when ``want_saliency`` or ``saliency_out`` is given.  Pinned host arrays make the copies asynchronous."""
+        self.cache_tag = None
+        g = _gray_batch(gray_u8)
+        B, h, w = g.shape
+        H, W, _ = self.spec.input_shape
+        nc = self.spec.num_classes
+        K, ci = _host_class_rows(classes, B, nc)
+        logits, probs, cls = np.empty((B, nc), np.float32), np.empty((B, nc), np.float32), np.empty((B,), np.int32)
+        ov = _out_array(overlay_out, (B, K, h, w, 3), np.uint8, "overlay_out") if want_overlay else None
+        hm = _out_array(heat_out, (B, K, h, w, 3), np.uint8, "heat_out") if want_heat else None
+        sal = _out_array(saliency_out, (B, K, H, W), np.float32, "saliency_out") if (want_saliency or saliency_out is not None) else None
+        _lib.check(self.lib.bcad_saliency_overlays_classes_host(self._h, _ptr(g), B, h, w, K, _ptr(ci), _lib.GRAD_MODE[grad_mode],
+                                                                1 if standardise else 0, _ptr(logits), _ptr(probs), _ptr(cls), _ptr(sal),
+                                                                _ptr(ov), _ptr(hm)))
+        return cls, probs, logits, ov, hm, sal
 
 
 def gradcam_tail(A: torch.Tensor, dA: torch.Tensor, out_hw: Tuple[int, int]) -> torch.Tensor:
@@ -663,7 +629,7 @@ def gradcam_tail(A: torch.Tensor, dA: torch.Tensor, out_hw: Tuple[int, int]) -> 
     out = torch.empty((B, H, W), device=A.device, dtype=torch.float32)
     with torch.cuda.device(A.device):
         _lib.check(lib.bcad_gradcam_tail(_ptr(A), _ptr(dA), B, K, h, w, H, W, 0 if A.dtype == torch.float32 else 1,
-                                         _ptr(out), C.c_void_p(torch.cuda.current_stream(A.device).cuda_stream)))
+                                         _ptr(out), _stream_of(A.device)))
     return out
 
 
@@ -678,7 +644,7 @@ def gray_preprocess(gray_u8: torch.Tensor, channels: int = 1, standardise: bool 
     x = torch.empty((B, H, W, channels), device=g.device, dtype=torch.float32)
     with torch.cuda.device(g.device):
         _lib.check(lib.bcad_gray_preprocess(_ptr(g), B, H, W, int(channels), 1 if standardise else 0, _ptr(img01), _ptr(x),
-                                            C.c_void_p(torch.cuda.current_stream(g.device).cuda_stream)))
+                                            _stream_of(g.device)))
     return img01, x
 
 
@@ -694,7 +660,7 @@ def gray_resize_preprocess(gray_u8: torch.Tensor, out_hw: Tuple[int, int], chann
     x = torch.empty((B, H, W, channels), device=g.device, dtype=torch.float32)
     with torch.cuda.device(g.device):
         _lib.check(lib.bcad_gray_resize_preprocess(_ptr(g), B, h, w, H, W, int(channels), 1 if standardise else 0, _ptr(x),
-                                                   C.c_void_p(torch.cuda.current_stream(g.device).cuda_stream)))
+                                                   _stream_of(g.device)))
     return x
 
 
@@ -713,7 +679,7 @@ def overlay_classes(gray_u8: torch.Tensor, cams: torch.Tensor, want_overlay=True
     hu = torch.empty((B, K, H, W), device=cam.device, dtype=torch.uint8) if want_heat_u8 else None
     with torch.cuda.device(cam.device):
         _lib.check(lib.bcad_overlay_classes(_ptr(g), _ptr(cam), B, K, H, W, _ptr(ov), _ptr(hu),
-                                            C.c_void_p(torch.cuda.current_stream(cam.device).cuda_stream)))
+                                            _stream_of(cam.device)))
     return ov, hu
 
 
@@ -727,7 +693,7 @@ def overlay(img01: torch.Tensor, cam: torch.Tensor, want_overlay=True, want_heat
     hu = torch.empty((B, H, W), device=cam.device, dtype=torch.uint8) if want_heat_u8 else None
     with torch.cuda.device(cam.device):
         _lib.check(lib.bcad_overlay(_ptr(img01), _ptr(cam), B, H, W, _ptr(ov), _ptr(hu),
-                                    C.c_void_p(torch.cuda.current_stream(cam.device).cuda_stream)))
+                                    _stream_of(cam.device)))
     return ov, hu
 
 
@@ -750,7 +716,7 @@ def saliency_overlay(base_u8, saliency: torch.Tensor):
     heat = torch.empty((B, K, H, W, 3), device=sal.device, dtype=torch.uint8)
     with torch.cuda.device(sal.device):
         _lib.check(lib.bcad_saliency_overlay(_ptr(base), int(base.shape[3]), _ptr(sal), B, K, H, W, _ptr(ov), _ptr(heat),
-                                             C.c_void_p(torch.cuda.current_stream(sal.device).cuda_stream)))
+                                             _stream_of(sal.device)))
     return ov, heat
 
 
@@ -772,7 +738,7 @@ def saliency_overlay_resized(gray_u8: torch.Tensor, saliency: torch.Tensor, want
     heat = torch.empty((B, K, h, w, 3), device=sal.device, dtype=torch.uint8) if want_heat else None
     with torch.cuda.device(sal.device):
         _lib.check(lib.bcad_saliency_overlay_resized(_ptr(g), _ptr(sal), B, K, H, W, h, w, _ptr(ov), _ptr(heat),
-                                                     C.c_void_p(torch.cuda.current_stream(sal.device).cuda_stream)))
+                                                     _stream_of(sal.device)))
     return ov, heat
 
 
@@ -805,84 +771,68 @@ class ShardedEngine:
         for e in self.engines:
             e.set_weights(*a, **k)
 
-    def _outputs(self, B, heat_dtype):
-        h, w, _ = self.spec.input_shape
-        nc = self.spec.num_classes
-        key = (B, np.dtype(heat_dtype).str)
+    def _pinned(self, key, specs):
+        """The driver's pinned output arrays for ``key``, one per (shape, torch dtype) of ``specs``.  One set is kept: a call with
+        another key replaces it."""
         if self._out is None or self._out[0] != key:
-            tdt = torch.uint8 if np.dtype(heat_dtype) == np.uint8 else torch.float32
-            bufs = (torch.empty((B,), dtype=torch.int32).pin_memory(), torch.empty((B, nc), dtype=torch.float32).pin_memory(),
-                    torch.empty((B, nc), dtype=torch.float32).pin_memory(), torch.empty((B, h, w), dtype=tdt).pin_memory())
-            self._out = (key, bufs)
+            self._out = (key, tuple(torch.empty(shape, dtype=dt).pin_memory() for shape, dt in specs))
         return tuple(t.numpy() for t in self._out[1])
 
-    def predict_explain_host(self, x: np.ndarray, class_idx=None, grad_mode="logit", heat_dtype=np.float32):
-        """-> (cls, probs, logits, heat) host arrays over the whole batch.  The arrays are the driver's pinned buffers: they are
-        overwritten by the next call with the same batch size (copy what must outlive it)."""
-        B = x.shape[0]
-        cls, probs, logits, heat = self._outputs(B, heat_dtype)
+    def _fan_out(self, B, work):
+        """work(engine, start, stop) on one host thread per engine over shard_bounds(B), empty shards skipped; raises the first error
+        once every thread has joined."""
         errs = []
-        ci_all = None if class_idx is None else np.ascontiguousarray(np.broadcast_to(np.asarray(class_idx, np.int32).reshape(-1), (B,)))
 
-        def work(e, s, t):
+        def run(e, s, t):
             try:
-                if t <= s:
-                    return
-                c, p, l, hm = e.predict_explain_host(x[s:t], None if ci_all is None else ci_all[s:t], grad_mode, heat_out=heat[s:t],
-                                                     heat_dtype=heat_dtype)
-                cls[s:t], probs[s:t], logits[s:t] = c, p, l
+                work(e, s, t)
             except Exception as ex:  # surfaced after join
                 errs.append(ex)
 
-        ths = [threading.Thread(target=work, args=(e, s, t))
-               for e, (s, t) in zip(self.engines, shard_bounds(B, len(self.engines)))]
+        ths = [threading.Thread(target=run, args=(e, s, t))
+               for e, (s, t) in zip(self.engines, shard_bounds(B, len(self.engines))) if t > s]
         for t in ths:
             t.start()
         for t in ths:
             t.join()
         if errs:
             raise errs[0]
+
+    def predict_explain_host(self, x: np.ndarray, class_idx=None, grad_mode="logit", heat_dtype=np.float32):
+        """-> (cls, probs, logits, heat) host arrays over the whole batch.  The arrays are the driver's pinned buffers: they are
+        overwritten by the next call with the same batch size (copy what must outlive it)."""
+        B = x.shape[0]
+        h, w, _ = self.spec.input_shape
+        nc = self.spec.num_classes
+        heat_t = torch.uint8 if np.dtype(heat_dtype) == np.uint8 else torch.float32
+        cls, probs, logits, heat = self._pinned((B, np.dtype(heat_dtype).str), [((B,), torch.int32), ((B, nc), torch.float32),
+                                                                                ((B, nc), torch.float32), ((B, h, w), heat_t)])
+        ci = _host_class_idx(class_idx, B, nc)
+
+        def work(e, s, t):
+            cls[s:t], probs[s:t], logits[s:t], _ = e.predict_explain_host(x[s:t], None if ci is None else ci[s:t], grad_mode,
+                                                                          heat_out=heat[s:t], heat_dtype=heat_dtype)
+
+        self._fan_out(B, work)
         return cls, probs, logits, heat
 
     def gradcam_overlays_classes_host(self, gray_u8: np.ndarray, classes=(0, 1), grad_mode="logit", standardise=True):
         """Engine.gradcam_overlays_classes_host over the GPUs of the box: contiguous split, one host thread per GPU
         -> (cls, probs, logits, overlays [B,K,h,w,3], heatmap_uint8 [B,K,h,w]).  The arrays are the driver's pinned buffers: they are
         overwritten by the next call of the same shape (copy what must outlive it)."""
-        g = np.ascontiguousarray(gray_u8)
-        if g.dtype != np.uint8 or g.ndim not in (2, 3):
-            raise ValueError("gray_u8 must be uint8 [B,H,W] or [H,W]")
-        if g.ndim == 2:
-            g = g[None]
+        g = _gray_batch(gray_u8)
         B, h, w = g.shape
         nc = self.spec.num_classes
         K, ci = _host_class_rows(classes, B, nc)
-        key = ("classes", B, K, h, w)
-        if self._out is None or self._out[0] != key:
-            bufs = (torch.empty((B,), dtype=torch.int32).pin_memory(), torch.empty((B, nc), dtype=torch.float32).pin_memory(),
-                    torch.empty((B, nc), dtype=torch.float32).pin_memory(), torch.empty((B, K, h, w, 3), dtype=torch.uint8).pin_memory(),
-                    torch.empty((B, K, h, w), dtype=torch.uint8).pin_memory())
-            self._out = (key, bufs)
-        cls, probs, logits, ov, hu = (t.numpy() for t in self._out[1])
-        errs = []
+        cls, probs, logits, ov, hu = self._pinned(("classes", B, K, h, w), [((B,), torch.int32), ((B, nc), torch.float32),
+                                                                             ((B, nc), torch.float32), ((B, K, h, w, 3), torch.uint8),
+                                                                             ((B, K, h, w), torch.uint8)])
 
         def work(e, s, t):
-            try:
-                if t <= s:
-                    return
-                c, p, l, _, _ = e.gradcam_overlays_classes_host(g[s:t], None if ci is None else ci[s:t], grad_mode, standardise,
-                                                                overlay_out=ov[s:t], heat_out=hu[s:t])
-                cls[s:t], probs[s:t], logits[s:t] = c, p, l
-            except Exception as ex:  # surfaced after join
-                errs.append(ex)
+            cls[s:t], probs[s:t], logits[s:t], _, _ = e.gradcam_overlays_classes_host(g[s:t], None if ci is None else ci[s:t], grad_mode,
+                                                                                      standardise, overlay_out=ov[s:t], heat_out=hu[s:t])
 
-        ths = [threading.Thread(target=work, args=(e, s, t))
-               for e, (s, t) in zip(self.engines, shard_bounds(B, len(self.engines)))]
-        for t in ths:
-            t.start()
-        for t in ths:
-            t.join()
-        if errs:
-            raise errs[0]
+        self._fan_out(B, work)
         return cls, probs, logits, ov, hu
 
     def set_fast_training(self, on: bool = True):
@@ -906,37 +856,17 @@ class ShardedEngine:
         H, W, _ = self.spec.input_shape
         nc = self.spec.num_classes
         K, ci = _host_class_rows(classes, B, nc)
-        key = ("saliency", B, K, h, w, bool(want_saliency))
-        if self._out is None or self._out[0] != key:
-            bufs = (torch.empty((B,), dtype=torch.int32).pin_memory(), torch.empty((B, nc), dtype=torch.float32).pin_memory(),
-                    torch.empty((B, nc), dtype=torch.float32).pin_memory(), torch.empty((B, K, h, w, 3), dtype=torch.uint8).pin_memory(),
-                    torch.empty((B, K, h, w, 3), dtype=torch.uint8).pin_memory())
-            if want_saliency:
-                bufs += (torch.empty((B, K, H, W), dtype=torch.float32).pin_memory(),)
-            self._out = (key, bufs)
-        cls, probs, logits, ov, hm, *rest = (t.numpy() for t in self._out[1])
+        specs = [((B,), torch.int32), ((B, nc), torch.float32), ((B, nc), torch.float32), ((B, K, h, w, 3), torch.uint8),
+                 ((B, K, h, w, 3), torch.uint8)] + ([((B, K, H, W), torch.float32)] if want_saliency else [])
+        cls, probs, logits, ov, hm, *rest = self._pinned(("saliency", B, K, h, w, bool(want_saliency)), specs)
         sal = rest[0] if want_saliency else None
-        errs = []
 
         def work(e, s, t):
-            try:
-                if t <= s:
-                    return
-                c, p, l, _, _, _ = e.saliency_overlays_classes_host(g[s:t], None if ci is None else ci[s:t], grad_mode, standardise,
-                                                                    overlay_out=ov[s:t], heat_out=hm[s:t],
-                                                                    saliency_out=None if sal is None else sal[s:t])
-                cls[s:t], probs[s:t], logits[s:t] = c, p, l
-            except Exception as ex:  # surfaced after join
-                errs.append(ex)
+            cls[s:t], probs[s:t], logits[s:t], _, _, _ = e.saliency_overlays_classes_host(
+                g[s:t], None if ci is None else ci[s:t], grad_mode, standardise, overlay_out=ov[s:t], heat_out=hm[s:t],
+                saliency_out=None if sal is None else sal[s:t])
 
-        ths = [threading.Thread(target=work, args=(e, s, t))
-               for e, (s, t) in zip(self.engines, shard_bounds(B, len(self.engines)))]
-        for t in ths:
-            t.start()
-        for t in ths:
-            t.join()
-        if errs:
-            raise errs[0]
+        self._fan_out(B, work)
         return cls, probs, logits, ov, hm, sal
 
     def close(self):
